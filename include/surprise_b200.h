@@ -308,6 +308,39 @@ int sb2_slope_one_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* 
                               const double* user_mean, double* est, uint8_t* impossible, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * CoClustering.  sb2_coclustering_fit replaces CoClustering.fit's epoch loop and compute_averages
+ * (prediction_algorithms/co_clustering.pyx:68-155, :157-237): n_epochs x (averages, user pass, item pass),
+ * then the final averages.  Bit-identical to the reference: ratings are truncated to C ints like its
+ * `cdef int r`; the cluster averages are exact integer sums / counts (global_mean for an empty cluster); every
+ * errors[c] is an ordered fp64 sum in ur[u] (ir[i]) list order; argmin takes the first minimum.
+ * u_ptr / ui_idx / u_r: the ur CSR; i_ptr / iu_idx / i_r: the ir CSR (nnz entries each).
+ * user_mean / item_mean: np.mean of each ur[u] / ir[i] list (computed by the caller, untruncated).
+ * cltr_u[n_users], cltr_i[n_items] (int32, in/out): the rng.randint draw on entry, the final clusters on exit.
+ * avg_cltr_u[n_cltr_u], avg_cltr_i[n_cltr_i], avg_cocltr[n_cltr_u x n_cltr_i] (row-major): outputs.
+ * SB2_ERR_INVALID for n_cltr_u < 1 or n_cltr_i < 1, an initial cluster out of range, or a rating outside the C
+ * int range (the reference raises OverflowError).  The _dev form enqueues the whole fit and synchronises
+ * `stream` once at the end to read that status.
+ * sb2_coclustering_predict_dev replaces CoClustering.estimate (co_clustering.pyx, after compute_averages):
+ * u[k] < 0 or i[k] < 0 (unknown) gives global_mean -- an estimate, not PredictionImpossible.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_coclustering_fit_dev(int64_t n_users, int64_t n_items, int64_t nnz, const int64_t* u_ptr,
+                             const int32_t* ui_idx, const double* u_r, const int64_t* i_ptr, const int32_t* iu_idx,
+                             const double* i_r, const double* user_mean, const double* item_mean,
+                             double global_mean, int n_cltr_u, int n_cltr_i, int n_epochs, int32_t* cltr_u,
+                             int32_t* cltr_i, double* avg_cltr_u, double* avg_cltr_i, double* avg_cocltr,
+                             void* stream);
+int sb2_coclustering_fit(int64_t n_users, int64_t n_items, const int64_t* u_ptr, const int32_t* ui_idx,
+                         const double* u_r, const int64_t* i_ptr, const int32_t* iu_idx, const double* i_r,
+                         const double* user_mean, const double* item_mean, double global_mean, int n_cltr_u,
+                         int n_cltr_i, int n_epochs, int32_t* cltr_u, int32_t* cltr_i, double* avg_cltr_u,
+                         double* avg_cltr_i, double* avg_cocltr);
+int sb2_coclustering_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i, int64_t n_users,
+                                 int64_t n_items, int n_cltr_i, const int32_t* cltr_u, const int32_t* cltr_i,
+                                 const double* user_mean, const double* item_mean, const double* avg_cltr_u,
+                                 const double* avg_cltr_i, const double* avg_cocltr, double global_mean,
+                                 double* est, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * AlgoBase.get_neighbors (algo_base.py:303-334) on the device-resident similarity matrix: for each
  * requested row x = rows[b], the k other ids with the largest sim[x, .], in the order of the reference's
  * stable descending sort (ties by ascending id).  out: n_rows x k int32, padded with -1 when fewer than

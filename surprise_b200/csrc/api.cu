@@ -75,6 +75,15 @@ int slope_one_fit_dev(int64_t n_items, int64_t n_users, const int64_t* u_ptr, co
 int slope_one_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i, int64_t n_items, const int64_t* freq,
                           const double* dev, const int64_t* u_ptr, const int32_t* i_idx, const double* user_mean,
                           double* est, uint8_t* impossible, cudaStream_t st);
+int coclustering_fit_dev(int64_t n_users, int64_t n_items, int64_t nnz, const int64_t* u_ptr, const int32_t* ui_idx,
+                         const double* u_r, const int64_t* i_ptr, const int32_t* iu_idx, const double* i_r,
+                         const double* user_mean, const double* item_mean, double mu, int n_cu, int n_ci, int n_epochs,
+                         int32_t* cltr_u, int32_t* cltr_i, double* avg_u, double* avg_i, double* avg_co,
+                         cudaStream_t st);
+int coclustering_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i, int64_t n_users, int64_t n_items,
+                             int n_ci, const int32_t* cltr_u, const int32_t* cltr_i, const double* user_mean,
+                             const double* item_mean, const double* avg_u, const double* avg_i, const double* avg_co,
+                             double mu, double* est, cudaStream_t st);
 int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32_t* u, const int32_t* i,
                         const double* r, const sb2_sgd_params* prm, int with_yj, const int64_t* u_ptr,
                         const int32_t* ui_idx, int rank, int world, cudaStream_t st, sb2_svd_plan** out);
@@ -688,6 +697,66 @@ int sb2_slope_one_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* 
     SB2_TRY(ensure_device());
     return slope_one_predict_dev(n_pairs, u, i, n_items, freq, dev, u_ptr, i_idx, user_mean, est, impossible,
                                  (cudaStream_t)stream);
+}
+
+// ---- CoClustering ------------------------------------------------------------------------------
+int sb2_coclustering_fit_dev(int64_t n_users, int64_t n_items, int64_t nnz, const int64_t* u_ptr, const int32_t* ui_idx,
+                             const double* u_r, const int64_t* i_ptr, const int32_t* iu_idx, const double* i_r,
+                             const double* user_mean, const double* item_mean, double global_mean, int n_cltr_u,
+                             int n_cltr_i, int n_epochs, int32_t* cltr_u, int32_t* cltr_i, double* avg_cltr_u,
+                             double* avg_cltr_i, double* avg_cocltr, void* stream) {
+    SB2_TRY(ensure_device());
+    return coclustering_fit_dev(n_users, n_items, nnz, u_ptr, ui_idx, u_r, i_ptr, iu_idx, i_r, user_mean, item_mean,
+                                global_mean, n_cltr_u, n_cltr_i, n_epochs, cltr_u, cltr_i, avg_cltr_u, avg_cltr_i,
+                                avg_cocltr, (cudaStream_t)stream);
+}
+
+int sb2_coclustering_fit(int64_t n_users, int64_t n_items, const int64_t* u_ptr, const int32_t* ui_idx, const double* u_r,
+                         const int64_t* i_ptr, const int32_t* iu_idx, const double* i_r, const double* user_mean,
+                         const double* item_mean, double global_mean, int n_cltr_u, int n_cltr_i, int n_epochs,
+                         int32_t* cltr_u, int32_t* cltr_i, double* avg_cltr_u, double* avg_cltr_i, double* avg_cocltr) {
+    SB2_TRY(ensure_device());
+    if (n_cltr_u < 1 || n_cltr_i < 1 || n_users < 0 || n_items < 0) {
+        set_error("coclustering: n_cltr_u and n_cltr_i must be >= 1 (got %d, %d)", n_cltr_u, n_cltr_i);
+        return SB2_ERR_INVALID;
+    }
+    cudaStream_t st = nullptr;
+    const int64_t nnz = u_ptr[n_users];
+    const size_t cells = (size_t)n_cltr_u * (size_t)n_cltr_i;
+    DevBuf d_up, d_ui, d_ur, d_ip, d_iu, d_ir, d_um, d_im, d_cu, d_ci, d_au, d_ai, d_ac;
+    SB2_TRY(upload(d_up, u_ptr, (size_t)n_users + 1, st));
+    SB2_TRY(upload(d_ui, ui_idx, (size_t)nnz, st));
+    SB2_TRY(upload(d_ur, u_r, (size_t)nnz, st));
+    SB2_TRY(upload(d_ip, i_ptr, (size_t)n_items + 1, st));
+    SB2_TRY(upload(d_iu, iu_idx, (size_t)nnz, st));
+    SB2_TRY(upload(d_ir, i_r, (size_t)nnz, st));
+    SB2_TRY(upload(d_um, user_mean, (size_t)n_users, st));
+    SB2_TRY(upload(d_im, item_mean, (size_t)n_items, st));
+    SB2_TRY(upload(d_cu, cltr_u, (size_t)n_users, st));
+    SB2_TRY(upload(d_ci, cltr_i, (size_t)n_items, st));
+    SB2_TRY(d_au.alloc((size_t)n_cltr_u * 8, st));
+    SB2_TRY(d_ai.alloc((size_t)n_cltr_i * 8, st));
+    SB2_TRY(d_ac.alloc(cells * 8, st));
+    SB2_TRY(coclustering_fit_dev(n_users, n_items, nnz, d_up.as<int64_t>(), d_ui.as<int32_t>(), d_ur.as<double>(),
+                                 d_ip.as<int64_t>(), d_iu.as<int32_t>(), d_ir.as<double>(), d_um.as<double>(),
+                                 d_im.as<double>(), global_mean, n_cltr_u, n_cltr_i, n_epochs, d_cu.as<int32_t>(),
+                                 d_ci.as<int32_t>(), d_au.as<double>(), d_ai.as<double>(), d_ac.as<double>(), st));
+    SB2_TRY(download(cltr_u, d_cu.p, (size_t)n_users, st));
+    SB2_TRY(download(cltr_i, d_ci.p, (size_t)n_items, st));
+    SB2_TRY(download(avg_cltr_u, d_au.p, (size_t)n_cltr_u, st));
+    SB2_TRY(download(avg_cltr_i, d_ai.p, (size_t)n_cltr_i, st));
+    SB2_TRY(download(avg_cocltr, d_ac.p, cells, st));
+    SB2_CUDA(cudaStreamSynchronize(st));
+    return SB2_OK;
+}
+
+int sb2_coclustering_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i, int64_t n_users, int64_t n_items,
+                                 int n_cltr_i, const int32_t* cltr_u, const int32_t* cltr_i, const double* user_mean,
+                                 const double* item_mean, const double* avg_cltr_u, const double* avg_cltr_i,
+                                 const double* avg_cocltr, double global_mean, double* est, void* stream) {
+    SB2_TRY(ensure_device());
+    return coclustering_predict_dev(n_pairs, u, i, n_users, n_items, n_cltr_i, cltr_u, cltr_i, user_mean, item_mean,
+                                    avg_cltr_u, avg_cltr_i, avg_cocltr, global_mean, est, (cudaStream_t)stream);
 }
 
 int sb2_get_neighbors_dev(int64_t n_x, const double* sim, int64_t sim_ld, int64_t n_rows, const int32_t* rows, int k,

@@ -19,6 +19,18 @@ def _func(m):
     return getattr(m, "__func__", m)
 
 
+def list_means(ptr, val):
+    """np.mean of every list of a flattened yr CSR (``np.mean([r for (_, r) in ur[u]])`` for all u), as a float64
+    array.  Quarter-step ratings take an exact fast path: every partial sum is exact, so any summation order gives
+    np.mean's bits; other ratings run np.mean list by list."""
+    n = len(ptr) - 1
+    cnt = np.diff(ptr)
+    if len(val) and np.array_equal(val * 4, np.rint(val * 4)) and np.abs(val).max() < 2 ** 20 and cnt.min() > 0:
+        sums = np.bincount(np.repeat(np.arange(n), cnt), weights=val, minlength=n)
+        return sums / cnt
+    return np.array([np.mean(val[ptr[k]:ptr[k + 1]].tolist()) for k in range(n)], dtype=np.float64)
+
+
 class AlgoBase(object):
     # set by device-backed subclasses to the estimate() their _estimate_batch is equivalent to
     _batch_estimate_of = None

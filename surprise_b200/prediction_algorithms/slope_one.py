@@ -8,7 +8,7 @@ materialised to numpy lazily.  test() sends all known pairs to the warp-per-pair
 import numpy as np
 
 from .. import _native as nat
-from .algo_base import AlgoBase
+from .algo_base import AlgoBase, list_means
 from .predictions import PredictionImpossible
 
 
@@ -34,13 +34,7 @@ class SlopeOne(AlgoBase):
                                                   nat.ptr(self._ur_dev[2]), len(val), nat.ptr(self._freq_dev),
                                                   nat.ptr(self._dev_dev), nat.stream()))
         # mean ratings of all users (slope_one.pyx:76-77): np.mean over each ur[u] list
-        cnt = np.diff(ptr)
-        if len(val) and np.array_equal(val * 4, np.rint(val * 4)) and np.abs(val).max() < 2 ** 20 and cnt.min() > 0:
-            # quarter-step ratings: every partial sum is exact, so any summation order gives np.mean's bits
-            sums = np.bincount(np.repeat(np.arange(ts.n_users), cnt), weights=val, minlength=ts.n_users)
-            self.user_mean = list(sums / cnt)
-        else:
-            self.user_mean = [np.mean(val[ptr[u]:ptr[u + 1]].tolist()) for u in range(ts.n_users)]
+        self.user_mean = list(list_means(ptr, val))
         self._mean_dev = nat.to_dev(np.asarray(self.user_mean, dtype=np.float64), np.float64)
         return self
 
