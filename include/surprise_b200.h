@@ -350,6 +350,34 @@ int sb2_get_neighbors_dev(int64_t n_x, const double* sim, int64_t sim_ld, int64_
                           int k, int32_t* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Top-N recommendations (AlgoBase.get_top_n / top_n_inner): the FAQ's get_top_n over
+ * algo.test(trainset.build_anti_testset()), on the device.
+ * sb2_mf_score_block_dev: scores[b * ld + i] = the estimate sb2_mf_predict_dev returns for the pair
+ * (rows[b], i), bit for bit, for every b < n_rows and every item i < n_items (SVD, SVD++ with yj / u_ptr /
+ * ui_idx, NMF, and BaselineOnly with f = 0, pu = qi = NULL).  rows[b] must be known users (0 <= rows[b] <
+ * n_users); biased as in sb2_mf_predict_dev.  Three launches per call (factor repacks, then the scorer).
+ * sb2_top_n_select_dev: for each row b, the candidates are the items rows[b] did not rate (ur CSR u_ptr /
+ * ui_idx).  Each gets the value AlgoBase.test gives it: scores[b * ld + i], replaced by default_est where
+ * impossible[b * ld + i] == 1 (impossible may be NULL: no impossible pairs), minus offset, then
+ * min(high, .) and max(low, .).  Output: the first n candidates in (value desc, item asc) order -- Python's
+ * stable sort(reverse=True) of the anti-testset -- with -0.0 equal to +0.0 and NaN after every number:
+ * items_out[b * n + j] (int32 inner ids) and est_out[b * n + j] (the values), padded with -1 / NaN;
+ * count_out[b] = the number emitted.  One launch per call; one pass over each row for n <= 2048 and one
+ * more per further 2048 entries.  SB2_ERR_INVALID for n < 1; SB2_ERR_ZERO_DIVISION where a candidate has
+ * impossible == 2 (the reference raises ZeroDivisionError; the call then synchronises `stream` to read
+ * that status); SB2_ERR_UNSUPPORTED when the rated-item bitmap (n_items bits) does not fit in shared memory
+ * (about 1.4 M items).
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_mf_score_block_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, int f, int biased,
+                           double global_mean, const double* pu, const double* qi, const double* bu,
+                           const double* bi, const double* yj, const int64_t* u_ptr, const int32_t* ui_idx,
+                           double* scores, int64_t ld, void* stream);
+int sb2_top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                         const uint8_t* impossible, double default_est, double offset, double low, double high,
+                         const int64_t* u_ptr, const int32_t* ui_idx, int n, int32_t* items_out,
+                         double* est_out, int32_t* count_out, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Row shard of a SYMMETRIC multi-rank similarity build (SURVEY.md 8e "cyclic upper-triangular tile sharding").
  * Same arguments as sb2_sim_build_dev, but only sim[i][j] with row_begin <= i < row_end and j >= row_begin is
  * computed (tiles at or above the block diagonal; the shard's own diagonal square is mirrored like the

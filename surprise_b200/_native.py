@@ -100,6 +100,10 @@ SIGNATURES = {
                                     _vp, _vp, _vp, _vp]),
     "sb2_coclustering_predict_dev": (_int, [_i64, _vp, _vp, _i64, _i64, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                             _dbl, _vp, _vp]),
+    "sb2_mf_score_block_dev": (_int, [_i64, _vp, _i64, _int, _int, _dbl, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                      _i64, _vp]),
+    "sb2_top_n_select_dev": (_int, [_i64, _vp, _i64, _vp, _i64, _vp, _dbl, _dbl, _dbl, _dbl, _vp, _vp, _int, _vp,
+                                    _vp, _vp, _vp]),
 }
 
 _lib = None

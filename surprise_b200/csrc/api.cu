@@ -84,6 +84,13 @@ int coclustering_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i
                              int n_ci, const int32_t* cltr_u, const int32_t* cltr_i, const double* user_mean,
                              const double* item_mean, const double* avg_u, const double* avg_i, const double* avg_co,
                              double mu, double* est, cudaStream_t st);
+int mf_score_block_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, int f, int biased, double mu,
+                       const double* pu, const double* qi, const double* bu, const double* bi, const double* yj,
+                       const int64_t* u_ptr, const int32_t* ui_idx, double* scores, int64_t ld, cudaStream_t st);
+int top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                     const uint8_t* impossible, double default_est, double offset, double low, double high,
+                     const int64_t* u_ptr, const int32_t* ui_idx, int n, int32_t* items_out, double* est_out,
+                     int32_t* count_out, cudaStream_t st);
 int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32_t* u, const int32_t* i,
                         const double* r, const sb2_sgd_params* prm, int with_yj, const int64_t* u_ptr,
                         const int32_t* ui_idx, int rank, int world, cudaStream_t st, sb2_svd_plan** out);
@@ -763,6 +770,24 @@ int sb2_get_neighbors_dev(int64_t n_x, const double* sim, int64_t sim_ld, int64_
                           int32_t* out, void* stream) {
     SB2_TRY(ensure_device());
     return get_neighbors_dev(n_x, sim, sim_ld, n_rows, rows, k, out, (cudaStream_t)stream);
+}
+
+// ---- top-N -------------------------------------------------------------------------------------
+int sb2_mf_score_block_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, int f, int biased, double global_mean,
+                           const double* pu, const double* qi, const double* bu, const double* bi, const double* yj,
+                           const int64_t* u_ptr, const int32_t* ui_idx, double* scores, int64_t ld, void* stream) {
+    SB2_TRY(ensure_device());
+    return mf_score_block_dev(n_rows, rows, n_items, f, biased, global_mean, pu, qi, bu, bi, yj, u_ptr, ui_idx, scores,
+                              ld, (cudaStream_t)stream);
+}
+
+int sb2_top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                         const uint8_t* impossible, double default_est, double offset, double low, double high,
+                         const int64_t* u_ptr, const int32_t* ui_idx, int n, int32_t* items_out, double* est_out,
+                         int32_t* count_out, void* stream) {
+    SB2_TRY(ensure_device());
+    return top_n_select_dev(n_rows, rows, n_items, scores, ld, impossible, default_est, offset, low, high, u_ptr,
+                            ui_idx, n, items_out, est_out, count_out, (cudaStream_t)stream);
 }
 
 int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,

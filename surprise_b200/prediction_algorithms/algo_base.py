@@ -31,6 +31,26 @@ def list_means(ptr, val):
     return np.array([np.mean(val[ptr[k]:ptr[k + 1]].tolist()) for k in range(n)], dtype=np.float64)
 
 
+# scores of one user block of top_n_inner: near the B200's 126 MB L2
+_TOP_N_BLOCK_BYTES = 96 << 20
+# rows sb2_mf_score_block_dev accepts per call (65535 blocks of 16 rows); tiny catalogues would otherwise exceed it
+_TOP_N_MAX_SCORER_ROWS = 65535 * 16
+
+
+def _check_top_n(n):
+    if isinstance(n, bool) or not isinstance(n, (int, np.integer)) or n < 1:
+        raise ValueError("n must be an int >= 1 (got %r)" % (n,))
+    return min(int(n), 2 ** 31 - 1)
+
+
+def rank_top_n(est, items):
+    """Order of the entries (est[k], items[k]) in the top-N ranking: est descending with -0.0 == 0.0 and NaN last,
+    ties by ascending item -- a stable sort(reverse=True) of a list in ascending item order."""
+    est = np.asarray(est, dtype=np.float64)
+    nan = np.isnan(est)
+    return np.lexsort((np.asarray(items), -np.where(nan, 0.0, est), nan))
+
+
 class AlgoBase(object):
     # set by device-backed subclasses to the estimate() their _estimate_batch is equivalent to
     _batch_estimate_of = None
@@ -135,6 +155,125 @@ class AlgoBase(object):
             for pred in out:
                 print(pred)
         return out
+
+    # -- top-N recommendations -------------------------------------------------------------------------
+    def get_top_n(self, n=10, uids=None):
+        """The n best items each user has not rated, as the reference FAQ computes them:
+
+            get_top_n(algo.test(trainset.build_anti_testset()), n)
+
+        i.e. {raw uid: [(raw iid, est), ...]} with every est the bits ``test()`` gives the pair, sorted by est
+        descending, ties in ascending inner item id (Python's stable sort(reverse=True) of the anti-testset).  -0.0
+        ranks equal to 0.0; NaN (diverged factors, where the FAQ's order is undefined) ranks after every number.
+        Users who rated every item get no entry.  ``uids`` (raw ids) restricts the output to those users, keys in
+        the given order; an unknown uid raises ValueError.  Device-batched algorithms score and rank on the GPU
+        (see ``top_n_inner``); any other algorithm goes through ``test()`` on the requested users' anti-testset."""
+        n = _check_top_n(n)
+        ts = self.trainset
+        if uids is None:
+            users = np.arange(ts.n_users, dtype=np.int32)
+            raw_u = [ts.to_raw_uid(u) for u in range(ts.n_users)]
+        else:
+            raw_u = list(uids)
+            users = np.array([ts.to_inner_uid(x) for x in raw_u], dtype=np.int32)
+        items, est, count = self.top_n_inner(n, users)
+        raw_i = np.empty(ts.n_items, dtype=object)
+        raw_i[:] = [ts.to_raw_iid(i) for i in range(ts.n_items)]
+        out = {}
+        for k in np.flatnonzero(count).tolist():
+            c = int(count[k])
+            out[raw_u[k]] = list(zip(raw_i[items[k, :c]].tolist(), est[k, :c].tolist()))
+        return out
+
+    def top_n_inner(self, n=10, users=None, _block_rows=None, _events=None):
+        """``get_top_n`` on inner ids: (items int32 [U, w], est float64 [U, w], count int32 [U]) for the users
+        ``users`` (inner ids, default all), w = min(n, n_items).  Row k holds the count[k] best items of users[k],
+        padded with -1 / NaN.  ``_block_rows`` overrides the number of users scored per device block (the output
+        does not depend on it).  ``_events``, a list, receives three recorded CUDA events per block (before the
+        scoring, between scoring and selection, after the selection) for timing."""
+        n = _check_top_n(n)
+        ts = self.trainset
+        if users is None:
+            users = np.arange(ts.n_users, dtype=np.int32)
+        else:
+            users = np.asarray(users).reshape(-1)
+            if users.size and (users.dtype.kind not in "iu" or users.min() < 0 or users.max() >= ts.n_users):
+                raise ValueError("users must be inner user ids in [0, %d)" % ts.n_users)
+            users = users.astype(np.int32)
+        width = min(n, ts.n_items)
+        if not self._batched():
+            return self._top_n_by_test(width, users)
+        from .. import _native as nat
+        torch = nat.torch_cuda()
+        n_u, n_i = len(users), ts.n_items
+        items = nat.empty_dev((max(n_u, 1), width), np.int32)
+        est = nat.empty_dev((max(n_u, 1), width), np.float64)
+        count = nat.empty_dev((max(n_u, 1),), np.int32)
+        ptr, idx, _ = ts.user_csr()
+        d_up, d_ui = nat.to_dev(ptr, np.int64), nat.to_dev(idx, np.int32)
+        d_users = nat.to_dev(users, np.int32)
+        scorer = self._top_n_scorer()
+        rows = int(_block_rows) if _block_rows else max(1, _TOP_N_BLOCK_BYTES // (8 * n_i))
+        rows = min(rows, max(n_u, 1), _TOP_N_MAX_SCORER_ROWS)
+        low, high = ts.rating_scale
+        scores = nat.empty_dev((rows * n_i,), np.float64) if scorer is not None else None
+        lib, stream = nat.lib(), nat.stream()
+        for b0 in range(0, n_u, rows):
+            d_rows = d_users[b0:b0 + rows]
+            nr = len(d_rows)
+            imp = None
+            ev = None
+            if _events is not None:
+                ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+                _events.append(ev)
+                ev[0].record()
+            if scorer is not None:
+                nat.check(lib.sb2_mf_score_block_dev(nr, nat.ptr(d_rows), n_i, scorer["f"], scorer["biased"],
+                                                     float(ts.global_mean), nat.ptr(scorer["pu"]),
+                                                     nat.ptr(scorer["qi"]), nat.ptr(scorer["bu"]),
+                                                     nat.ptr(scorer["bi"]), nat.ptr(scorer.get("yj")),
+                                                     nat.ptr(scorer.get("up")), nat.ptr(scorer.get("ui")),
+                                                     nat.ptr(scores), n_i, stream))
+                sc = scores
+            else:
+                d_u = d_rows.repeat_interleave(n_i)
+                d_i = torch.arange(n_i, dtype=torch.int32, device=d_rows.device).repeat(nr)
+                sc, imp = self._estimate_dev(d_u, d_i)
+            if ev:
+                ev[1].record()
+            nat.check(lib.sb2_top_n_select_dev(nr, nat.ptr(d_rows), n_i, nat.ptr(sc), n_i, nat.ptr(imp),
+                                               float(self.default_prediction()), float(ts.offset), float(low),
+                                               float(high), nat.ptr(d_up), nat.ptr(d_ui), width,
+                                               nat.ptr(items[b0:]), nat.ptr(est[b0:]), nat.ptr(count[b0:]), stream))
+            if ev:
+                ev[2].record()
+        return items.cpu().numpy()[:n_u], est.cpu().numpy()[:n_u], count.cpu().numpy()[:n_u]
+
+    def _top_n_scorer(self):
+        """Device arrays for sb2_mf_score_block_dev (dict: f, biased, pu, qi, bu, bi[, yj, up, ui]), or None when
+        the algorithm is scored pair by pair through ``_estimate_dev``."""
+        return None
+
+    def _top_n_by_test(self, width, users):
+        """top_n_inner through ``test()``: for algorithms whose estimate() is not the device batch."""
+        ts = self.trainset
+        ptr, idx, _ = ts.user_csr()
+        fill = ts.global_mean
+        items = np.full((len(users), width), -1, dtype=np.int32)
+        est = np.full((len(users), width), np.nan)
+        count = np.zeros(len(users), dtype=np.int32)
+        all_i = np.arange(ts.n_items)
+        for k, u in enumerate(users.tolist()):
+            cand = np.setdiff1d(all_i, idx[ptr[u]:ptr[u + 1]])
+            if not len(cand):
+                continue
+            ru = ts.to_raw_uid(u)
+            preds = self.test([(ru, ts.to_raw_iid(i), fill) for i in cand.tolist()])
+            e = np.array([p.est for p in preds], dtype=np.float64)
+            order = rank_top_n(e, cand)[:width]
+            c = len(order)
+            items[k, :c], est[k, :c], count[k] = cand[order], e[order], c
+        return items, est, count
 
     # -- shared fit-time helpers ----------------------------------------------------------------------
     def compute_baselines(self):

@@ -35,18 +35,30 @@ class BaselineOnly(AlgoBase):
         state["_bias_dev"] = None
         return state
 
-    def _estimate_batch(self, iu, ii):
-        n = len(iu)
+    def _biases_dev(self):
         if getattr(self, "_bias_dev", None) is None:
             self._bias_dev = (nat.to_dev(self.bu, np.float64), nat.to_dev(self.bi, np.float64))
-        d_bu, d_bi = self._bias_dev
+        return self._bias_dev
+
+    def _estimate_dev(self, d_u, d_i):
+        """(est, impossible) device tensors for the device pairs (d_u, d_i)."""
+        n = len(d_u)
+        d_bu, d_bi = self._biases_dev()
         est = nat.empty_dev((max(n, 1),), np.float64)
         imp = nat.empty_dev((max(n, 1),), np.uint8)
-        d_u, d_i = nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32)
         nat.check(nat.lib().sb2_mf_predict_dev(n, nat.ptr(d_u), nat.ptr(d_i), 0, 1, float(self.trainset.global_mean), None,
                                                None, nat.ptr(d_bu), nat.ptr(d_bi), None, None, None, nat.ptr(est),
                                                nat.ptr(imp), nat.stream()))
+        return est, imp
+
+    def _estimate_batch(self, iu, ii):
+        n = len(iu)
+        est, _ = self._estimate_dev(nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32))
         return est.cpu().numpy()[:n], [{"was_impossible": False} for _ in range(n)]
+
+    def _top_n_scorer(self):
+        d_bu, d_bi = self._biases_dev()
+        return dict(f=0, biased=1, pu=None, qi=None, bu=d_bu, bi=d_bi)
 
     def estimate(self, u, i):
         as_inner = lambda v: int(v) if isinstance(v, (int, np.integer)) else -1

@@ -76,16 +76,21 @@ class CoClustering(AlgoBase):
                          nat.to_dev(self.avg_cocltr, np.float64))
         return self._dev
 
-    def _estimate_batch(self, iu, ii):
-        n = len(iu)
+    def _estimate_dev(self, d_u, d_i):
+        """(est, None) for the device pairs (d_u, d_i): CoClustering has no impossible pairs."""
+        n = len(d_u)
         ts = self.trainset
         cu, ci, um, im, au, ai, ac = self._device_state()
         est = nat.empty_dev((max(n, 1),), np.float64)
-        d_u, d_i = nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32)
         nat.check(nat.lib().sb2_coclustering_predict_dev(n, nat.ptr(d_u), nat.ptr(d_i), ts.n_users, ts.n_items,
                                                          int(self.n_cltr_i), nat.ptr(cu), nat.ptr(ci), nat.ptr(um),
                                                          nat.ptr(im), nat.ptr(au), nat.ptr(ai), nat.ptr(ac),
                                                          float(ts.global_mean), nat.ptr(est), nat.stream()))
+        return est, None
+
+    def _estimate_batch(self, iu, ii):
+        n = len(iu)
+        est, _ = self._estimate_dev(nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32))
         return est.cpu().numpy()[:n], [{"was_impossible": False} for _ in range(n)]
 
     def estimate(self, u, i):

@@ -73,15 +73,15 @@ class SymmetricAlgo(AlgoBase):
         state["_yr_dev"] = None
         return state
 
-    def _knn_batch(self, iu, ii, mode, bx=None, by=None):
-        x, y = self.switch(iu, ii)
-        n = len(x)
+    def _knn_dev(self, d_u, d_i, mode, bx=None, by=None):
+        """(est, actual_k, impossible) device tensors for the device pairs (d_u, d_i)."""
+        d_x, d_y = self.switch(d_u, d_i)
+        n = len(d_x)
         ptr, idx, val = self._yr_device()
         sim = self._sim_device()
         est = nat.empty_dev((max(n, 1),), np.float64)
         ak = nat.empty_dev((max(n, 1),), np.int32)
         imp = nat.empty_dev((max(n, 1),), np.uint8)
-        d_x, d_y = nat.to_dev(x, np.int32), nat.to_dev(y, np.int32)
         d_bx = nat.to_dev(bx, np.float64) if bx is not None else None
         d_by = nat.to_dev(by, np.float64) if by is not None else None
         rc = nat.lib().sb2_knn_predict_dev(n, nat.ptr(d_x), nat.ptr(d_y), self.n_x, nat.ptr(sim), self.n_x,
@@ -89,7 +89,17 @@ class SymmetricAlgo(AlgoBase):
                                            mode, float(self.trainset.global_mean), nat.ptr(d_bx), nat.ptr(d_by),
                                            nat.ptr(est), nat.ptr(ak), nat.ptr(imp), nat.stream())
         nat.check(rc)
+        return est, ak, imp
+
+    def _knn_batch(self, iu, ii, mode, bx=None, by=None):
+        n = len(iu)
+        est, ak, imp = self._knn_dev(nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32), mode, bx, by)
         return est.cpu().numpy()[:n], ak.cpu().numpy()[:n], imp.cpu().numpy()[:n]
+
+    def _estimate_dev(self, d_u, d_i):
+        """(est, impossible) device tensors for the device pairs (d_u, d_i)."""
+        est, _, imp = self._knn_dev(d_u, d_i, *self._knn_args())
+        return est, imp
 
 
 def _as_inner(v):
@@ -108,6 +118,9 @@ class KNNBasic(SymmetricAlgo):
         SymmetricAlgo.fit(self, trainset)
         self._sim_dev = self.compute_similarities_device()
         return self
+
+    def _knn_args(self):
+        return (0,)
 
     def _estimate_batch(self, iu, ii):
         est, ak, imp = self._knn_batch(iu, ii, 0)
@@ -148,9 +161,11 @@ class KNNBaseline(SymmetricAlgo):
         self._sim_dev = self.compute_similarities_device()
         return self
 
+    def _knn_args(self):
+        return (1 if self.sim_options["user_based"] else 2), self.bx, self.by
+
     def _estimate_batch(self, iu, ii):
-        mode = 1 if self.sim_options["user_based"] else 2
-        est, ak, _ = self._knn_batch(iu, ii, mode, self.bx, self.by)
+        est, ak, _ = self._knn_batch(iu, ii, *self._knn_args())
         details = [({"actual_k": int(ak[k]), "was_impossible": False} if ak[k] >= 0 else {"was_impossible": False})
                    for k in range(len(est))]
         return est, details
@@ -203,8 +218,11 @@ class _MeanCenteredKNN(SymmetricAlgo):
         self.k = k
         self.min_k = min_k
 
+    def _knn_args(self):
+        return self._mode, self.means, getattr(self, "sigmas", None)
+
     def _estimate_batch(self, iu, ii):
-        est, ak, imp = self._knn_batch(iu, ii, self._mode, self.means, getattr(self, "sigmas", None))
+        est, ak, imp = self._knn_batch(iu, ii, *self._knn_args())
         details = [({"was_impossible": True, "reason": "User and/or item is unkown."} if imp[k]
                     else {"actual_k": int(ak[k]), "was_impossible": False}) for k in range(len(est))]
         return est, details

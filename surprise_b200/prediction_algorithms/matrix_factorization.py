@@ -31,13 +31,10 @@ class _FactorModel(AlgoBase):
         u, i, r = trainset.coo()
         return nat.to_dev(u, np.int32), nat.to_dev(i, np.int32), nat.to_dev(r, np.float64), len(r)
 
-    def _predict_batch(self, iu, ii, biased):
-        ts = self.trainset
-        n = len(iu)
-        f = self.pu.shape[1]
-        d_u, d_i = nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32)
+    def _device_factors(self):
         dev = getattr(self, "_dev_cache", None)
         if dev is None:
+            ts = self.trainset
             dev = dict(pu=nat.to_dev(self.pu, np.float64), qi=nat.to_dev(self.qi, np.float64),
                        bu=nat.to_dev(self.bu, np.float64), bi=nat.to_dev(self.bi, np.float64))
             if self._has_yj:
@@ -45,18 +42,35 @@ class _FactorModel(AlgoBase):
                 dev.update(yj=nat.to_dev(self.yj, np.float64), up=nat.to_dev(ptr, np.int64),
                            ui=nat.to_dev(idx, np.int32))
             self._dev_cache = dev
+        return dev
+
+    def _predict_dev(self, d_u, d_i, biased):
+        """(est, impossible) device tensors for the device pairs (d_u, d_i) (sb2_mf_predict_dev)."""
+        n = len(d_u)
+        dev = self._device_factors()
         est = nat.empty_dev((max(n, 1),), np.float64)
         imp = nat.empty_dev((max(n, 1),), np.uint8)
-        rc = nat.lib().sb2_mf_predict_dev(n, nat.ptr(d_u), nat.ptr(d_i), f, int(bool(biased)),
-                                          float(ts.global_mean), nat.ptr(dev["pu"]), nat.ptr(dev["qi"]),
+        rc = nat.lib().sb2_mf_predict_dev(n, nat.ptr(d_u), nat.ptr(d_i), self.pu.shape[1], int(bool(biased)),
+                                          float(self.trainset.global_mean), nat.ptr(dev["pu"]), nat.ptr(dev["qi"]),
                                           nat.ptr(dev["bu"]), nat.ptr(dev["bi"]), nat.ptr(dev.get("yj")),
                                           nat.ptr(dev.get("up")), nat.ptr(dev.get("ui")), nat.ptr(est), nat.ptr(imp),
                                           nat.stream())
         nat.check(rc)
+        return est, imp
+
+    def _predict_batch(self, iu, ii, biased):
+        n = len(iu)
+        est, imp = self._predict_dev(nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32), biased)
         est, imp = est.cpu().numpy()[:n], imp.cpu().numpy()[:n]
         details = [({"was_impossible": True, "reason": "User and item are unkown."} if imp[k]
                     else {"was_impossible": False}) for k in range(n)]
         return est, details
+
+    def _estimate_dev(self, d_u, d_i):
+        return self._predict_dev(d_u, d_i, self._est_biased())
+
+    def _top_n_scorer(self):
+        return dict(self._device_factors(), f=int(self.pu.shape[1]), biased=int(bool(self._est_biased())))
 
     def __setattr__(self, name, value):
         # the reference's estimate() reads pu / qi / bu / bi / yj live: assigning any of them after fit (warm starts,
@@ -162,6 +176,9 @@ class SVD(_FactorModel):
         self.bu, self.bi = d_bu.cpu().numpy(), d_bi.cpu().numpy()
         self._dev_cache = None
 
+    def _est_biased(self):
+        return self.biased
+
     def _estimate_batch(self, iu, ii):
         return self._predict_batch(iu, ii, self.biased)
 
@@ -224,6 +241,9 @@ class SVDpp(_FactorModel):
         self.bu, self.bi = d_bu.cpu().numpy(), d_bi.cpu().numpy()
         self._dev_cache = None
 
+    def _est_biased(self):
+        return True
+
     def _estimate_batch(self, iu, ii):
         return self._predict_batch(iu, ii, True)
 
@@ -274,6 +294,9 @@ class NMF(_FactorModel):
         self.pu, self.qi = d_pu.cpu().numpy(), d_qi.cpu().numpy()
         self.bu, self.bi = d_bu.cpu().numpy(), d_bi.cpu().numpy()
         self._dev_cache = None
+
+    def _est_biased(self):
+        return self.biased
 
     def _estimate_batch(self, iu, ii):
         return self._predict_batch(iu, ii, self.biased)

@@ -67,15 +67,20 @@ class SlopeOne(AlgoBase):
             self._mean_dev = nat.to_dev(np.asarray(self.user_mean, dtype=np.float64), np.float64)
         return self._freq_dev, self._dev_dev, self._ur_dev, self._mean_dev
 
-    def _estimate_batch(self, iu, ii):
-        n = len(iu)
+    def _estimate_dev(self, d_u, d_i):
+        """(est, impossible) device tensors for the device pairs (d_u, d_i)."""
+        n = len(d_u)
         freq, dev, ur, mean = self._device_state()
         est = nat.empty_dev((max(n, 1),), np.float64)
         imp = nat.empty_dev((max(n, 1),), np.uint8)
-        d_u, d_i = nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32)
         nat.check(nat.lib().sb2_slope_one_predict_dev(n, nat.ptr(d_u), nat.ptr(d_i), self.trainset.n_items,
                                                       nat.ptr(freq), nat.ptr(dev), nat.ptr(ur[0]), nat.ptr(ur[1]),
                                                       nat.ptr(mean), nat.ptr(est), nat.ptr(imp), nat.stream()))
+        return est, imp
+
+    def _estimate_batch(self, iu, ii):
+        n = len(iu)
+        est, imp = self._estimate_dev(nat.to_dev(iu, np.int32), nat.to_dev(ii, np.int32))
         est, imp = est.cpu().numpy()[:n], imp.cpu().numpy()[:n]
         details = [{"was_impossible": True, "reason": "User and/or item is unkown."} if imp[k]
                    else {"was_impossible": False} for k in range(n)]
