@@ -378,6 +378,28 @@ int sb2_top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, c
                          double* est_out, int32_t* count_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Per-user counts behind accuracy.fcp and accuracy.precision_recall_at_k (DESIGN.md section 3.7).  All
+ * arrays are DEVICE arrays.  The n predictions are grouped into n_seg segments (users): segment s holds
+ * entries [seg_ptr[s], seg_ptr[s + 1]) of r (true ratings) and est (estimates), in prediction order;
+ * seg_ptr (int64, n_seg + 1 entries) must start at 0, not decrease and end at n, else SB2_ERR_INVALID.
+ * Compares are fp64 (NaN compares false, -0.0 == +0.0).  i and j run over one segment, i == j included.
+ * sb2_fcp_counts_dev: counts[2 s] = #{(i, j) : est_i > est_j and r_i > r_j},
+ *   counts[2 s + 1] = #{(i, j) : est_i >= est_j and r_i < r_j}.
+ * sb2_precision_at_k_counts_dev: with m = the segment's length, rank_j = #{i : est_i > est_j} +
+ *   #{i < j : est_i == est_j} (Python's stable sort(reverse=True)) and top = {j : rank_j < k_eff[s]}
+ *   (k_eff int64 per segment; k_eff >= m: every entry, k_eff <= 0: none):
+ *   counts[3 s] = #{j : r_j >= threshold}, counts[3 s + 1] = #{j in top : est_j >= threshold},
+ *   counts[3 s + 2] = #{j in top : r_j >= threshold and est_j >= threshold}.
+ * counts: int64, zeroed by the call.  One launch per call; the call synchronises `stream` to check the
+ * offsets, so the counts are ready when it returns.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_fcp_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r, const double* est,
+                       int64_t* counts, void* stream);
+int sb2_precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r,
+                                  const double* est, const int64_t* k_eff, double threshold, int64_t* counts,
+                                  void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Row shard of a SYMMETRIC multi-rank similarity build (SURVEY.md 8e "cyclic upper-triangular tile sharding").
  * Same arguments as sb2_sim_build_dev, but only sim[i][j] with row_begin <= i < row_end and j >= row_begin is
  * computed (tiles at or above the block diagonal; the shard's own diagonal square is mirrored like the

@@ -1,7 +1,17 @@
-"""rmse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143)."""
+"""rmse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), and the FAQ's
+precision_recall_at_k.
+
+fcp and precision_recall_at_k reduce to integer counts per user.  Where a CUDA device is usable and every r_ui and est
+is a real number that float64 holds exactly, the counts come from the device (csrc/rank_metrics.cu, DESIGN.md section
+3.7); otherwise from the Python loops below, which are the metrics' definition (and what the tests compare against).
+The arithmetic on the counts runs on the host either way, so both routes return the same values.
+"""
 from collections import defaultdict
+from operator import index, itemgetter
 
 import numpy as np
+
+__all__ = ["rmse", "mae", "fcp", "precision_recall_at_k"]
 
 
 def _need(predictions):
@@ -28,6 +38,64 @@ def mae(predictions, verbose=True):
 
 def fcp(predictions, verbose=True):
     _need(predictions)
+    nc, nd = _fcp_counts(predictions)
+    c_mean = np.mean(list(nc.values())) if nc else 0
+    d_mean = np.mean(list(nd.values())) if nd else 0
+    try:
+        out = c_mean / (c_mean + d_mean)
+    except ZeroDivisionError:
+        raise ValueError("cannot compute fcp on this list of prediction. Does every user have at least two "
+                         "predictions?")
+    if verbose:
+        print("FCP:  {0:1.4f}".format(out))
+    return out
+
+
+def precision_recall_at_k(predictions, k=10, threshold=3.5):
+    """Precision and recall at k per user, as the Surprise FAQ's recipe computes them: each user's predictions sorted
+    by est descending (a stable sort), the first k of them recommended where est >= threshold, relevant where
+    r_ui >= threshold.  Returns (precisions, recalls), two dicts keyed by uid in first-appearance order.
+
+    precisions[uid] = n_rel_and_rec_k / n_rec_k and recalls[uid] = n_rel_and_rec_k / n_rel, each the int 0 where its
+    denominator is 0 (the current FAQ; releases before it gave 1).  k follows list slicing: None means all, a negative
+    k counts from the end, and a k that is not an index raises TypeError (only when there is at least one user).
+
+    The counts come from the device when it is usable and threshold and every r_ui and est is a float, a bool, an int
+    with |x| <= 2**53 or a numpy float64, bool or integer scalar.  A user with a NaN est (for which the stable sort has
+    no defined order) gets the recipe itself, on the host; so does a user with numpy scalars when threshold is a Python
+    number, because which of the recipe's sums become numpy integers then depends on which entries are in the top k.
+    With a numpy threshold every compare is a numpy bool, so every non-empty sum is a numpy integer."""
+    if _device_usable() and _exact_reals([threshold]):
+        predictions = predictions if isinstance(predictions, (list, tuple)) else list(predictions)
+        cols = _exact_columns(predictions)
+        if cols is not None:
+            return _precision_recall_dev(*cols, k, threshold)
+    user_est_true = defaultdict(list)
+    for uid, _, true_r, est, _ in predictions:
+        user_est_true[uid].append((est, true_r))
+    precisions = dict()
+    recalls = dict()
+    for uid, user_ratings in user_est_true.items():
+        precisions[uid], recalls[uid] = _precision_recall_user(user_ratings, k, threshold)
+    return precisions, recalls
+
+
+def _precision_recall_user(user_ratings, k, threshold):
+    user_ratings.sort(key=lambda x: x[0], reverse=True)
+    n_rel = sum((true_r >= threshold) for (_, true_r) in user_ratings)
+    n_rec_k = sum((est >= threshold) for (est, _) in user_ratings[:k])
+    n_rel_and_rec_k = sum(((true_r >= threshold) and (est >= threshold)) for (est, true_r) in user_ratings[:k])
+    return (n_rel_and_rec_k / n_rec_k if n_rec_k != 0 else 0,
+            n_rel_and_rec_k / n_rel if n_rel != 0 else 0)
+
+
+def _fcp_counts(predictions):
+    """nc, nd: {uid: count} in first-appearance order."""
+    if _device_usable():
+        predictions = predictions if isinstance(predictions, (list, tuple)) else list(predictions)
+        cols = _exact_columns(predictions)
+        if cols is not None:
+            return _fcp_counts_dev(*cols)
     per_user = defaultdict(list)
     for u0, _, r0, est, _ in predictions:
         per_user[u0].append((est, r0))
@@ -41,13 +109,118 @@ def fcp(predictions, verbose=True):
                 if esi >= esj and ri < rj:
                     d += 1
         nc[u0], nd[u0] = c, d
-    c_mean = np.mean(list(nc.values())) if nc else 0
-    d_mean = np.mean(list(nd.values())) if nd else 0
-    try:
-        out = c_mean / (c_mean + d_mean)
-    except ZeroDivisionError:
-        raise ValueError("cannot compute fcp on this list of prediction. Does every user have at least two "
-                         "predictions?")
-    if verbose:
-        print("FCP:  {0:1.4f}".format(out))
-    return out
+    return nc, nd
+
+
+# -- device route ----------------------------------------------------------------------------------------------------
+_EXACT_INT = 2 ** 53
+
+
+def _device_usable():
+    """A CUDA device the library's sm_100a kernels run on (compute capability 10.0)."""
+    import torch
+    return torch.cuda.is_available() and torch.cuda.get_device_capability() == (10, 0)
+
+
+def _exact_reals(values):
+    """True when every value is a float, a bool, an int with |x| <= 2**53, or a numpy float64, bool or integer scalar
+    with |x| <= 2**53: float64 holds these exactly, and Python and numpy compare them with each other exactly.  (numpy
+    compares a float32 with a Python float in float32, so float32 and other float widths are left out.)"""
+    for t in set(map(type, values)):
+        if t is float or t is bool or t is np.float64 or t is np.bool_:
+            continue
+        if not (t is int or issubclass(t, np.integer)):
+            return False
+        if not all(-_EXACT_INT <= int(x) <= _EXACT_INT for x in values if type(x) is t):
+            return False
+    return True
+
+
+def _exact_columns(predictions):
+    """(keys, code, r_ui, est, has_numpy), or None when the Python route must run.  The columns are read as
+    `for uid, _, r_ui, est, _ in predictions` reads them (an item that does not unpack raises the same exception);
+    keys are the distinct uids as defaultdict(list) keeps them (first appearance, equal uids merged into the first), code
+    the position of each prediction's uid in keys."""
+    if not predictions:
+        return None
+    kinds = set(map(type, predictions))
+    if all(t is list or (issubclass(t, tuple) and t.__iter__ is tuple.__iter__ and t.__getitem__ is tuple.__getitem__)
+           for t in kinds) and set(map(len, predictions)) == {5}:
+        uid, r_ui, est = (list(map(itemgetter(c), predictions)) for c in (0, 2, 3))
+    else:
+        uid, r_ui, est = map(list, zip(*[(u, r, e) for u, _, r, e, _ in predictions]))
+    if not (_exact_reals(r_ui) and _exact_reals(est)):
+        return None
+    has_numpy = any(issubclass(t, np.generic) for t in set(map(type, r_ui)) | set(map(type, est)))
+    codes = {}
+    setd = codes.setdefault
+    code = np.array([setd(u, len(codes)) for u in uid], dtype=np.int64)
+    return list(codes), code, r_ui, est, has_numpy
+
+
+def _segments(code, n_seg, r_ui, est):
+    """Device segment CSR: seg_ptr (int64) and r, est (float64) grouped by code, prediction order kept in a group."""
+    from . import _native as nat
+    torch = nat.torch_cuda()
+    d_code = nat.to_dev(code, np.int64)
+    order = torch.sort(d_code, stable=True).indices
+    seg_ptr = torch.zeros(n_seg + 1, dtype=torch.int64, device=d_code.device)
+    seg_ptr[1:] = torch.cumsum(torch.bincount(d_code, minlength=n_seg), 0)
+    r = nat.to_dev(np.array(r_ui, dtype=np.float64), np.float64)[order]
+    e = nat.to_dev(np.array(est, dtype=np.float64), np.float64)[order]
+    return seg_ptr, r, e
+
+
+def _fcp_counts_dev(keys, code, r_ui, est, has_numpy):
+    from . import _native as nat
+    seg_ptr, r, e = _segments(code, len(keys), r_ui, est)
+    counts = nat.empty_dev((len(keys), 2), np.int64)
+    nat.check(nat.lib().sb2_fcp_counts_dev(len(keys), len(code), nat.ptr(seg_ptr), nat.ptr(r), nat.ptr(e),
+                                           nat.ptr(counts), nat.stream()))
+    nc, nd = counts.cpu().numpy().T.tolist()
+    return dict(zip(keys, nc)), dict(zip(keys, nd))
+
+
+def _precision_recall_dev(keys, code, r_ui, est, has_numpy, k, threshold):
+    from . import _native as nat
+    [][:k]                                      # a k that is not an index raises here, as the recipe's slice does
+    n_seg = len(keys)
+    m = np.bincount(code, minlength=n_seg)
+    if k is None:
+        k_eff = m
+    else:
+        kk = max(min(index(k), 1 << 62), -(1 << 62))
+        k_eff = np.minimum(m, kk) if kk >= 0 else np.maximum(m + kk, 0)
+    seg_ptr, r, e = _segments(code, n_seg, r_ui, est)
+    d_k_eff = nat.to_dev(k_eff, np.int64)
+    counts = nat.empty_dev((n_seg, 3), np.int64)
+    nat.check(nat.lib().sb2_precision_at_k_counts_dev(n_seg, len(code), nat.ptr(seg_ptr), nat.ptr(r), nat.ptr(e),
+                                                      nat.ptr(d_k_eff), float(threshold), nat.ptr(counts),
+                                                      nat.stream()))
+    n_rel, n_rec_k, n_rel_and_rec_k = counts.cpu().numpy().T.tolist()
+    numpy_threshold = isinstance(threshold, np.generic)
+    if numpy_threshold:
+        # the recipe's sums over numpy bools: a numpy integer, or the int 0 when the top k is empty
+        num = type(sum([threshold >= threshold]))
+        top = k_eff.tolist()
+        n_rel = [num(a) for a in n_rel]
+        n_rec_k = [num(b) if t else 0 for b, t in zip(n_rec_k, top)]
+        n_rel_and_rec_k = [num(c) if t else 0 for c, t in zip(n_rel_and_rec_k, top)]
+    precisions = dict()
+    recalls = dict()
+    for uid, a, b, c in zip(keys, n_rel, n_rec_k, n_rel_and_rec_k):
+        precisions[uid] = c / b if b != 0 else 0
+        recalls[uid] = c / a if a != 0 else 0
+    # users the recipe itself must run for: a NaN est, or numpy scalars compared with a Python threshold
+    on_host_rows = np.isnan(np.array(est, dtype=np.float64))
+    if has_numpy and not numpy_threshold:
+        on_host_rows |= np.fromiter((isinstance(x, np.generic) or isinstance(y, np.generic)
+                                     for x, y in zip(r_ui, est)), dtype=bool, count=len(code))
+    if on_host_rows.any():
+        rows = np.nonzero(np.isin(code, np.unique(code[on_host_rows])))[0]
+        user_est_true = defaultdict(list)
+        for j in rows.tolist():
+            user_est_true[int(code[j])].append((est[j], r_ui[j]))
+        for u, user_ratings in user_est_true.items():
+            precisions[keys[u]], recalls[keys[u]] = _precision_recall_user(user_ratings, k, threshold)
+    return precisions, recalls

@@ -91,6 +91,10 @@ int top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const
                      const uint8_t* impossible, double default_est, double offset, double low, double high,
                      const int64_t* u_ptr, const int32_t* ui_idx, int n, int32_t* items_out, double* est_out,
                      int32_t* count_out, cudaStream_t st);
+int fcp_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r, const double* est,
+                   int64_t* counts, cudaStream_t st);
+int precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r, const double* est,
+                              const int64_t* k_eff, double threshold, int64_t* counts, cudaStream_t st);
 int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32_t* u, const int32_t* i,
                         const double* r, const sb2_sgd_params* prm, int with_yj, const int64_t* u_ptr,
                         const int32_t* ui_idx, int rank, int world, cudaStream_t st, sb2_svd_plan** out);
@@ -788,6 +792,19 @@ int sb2_top_n_select_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, c
     SB2_TRY(ensure_device());
     return top_n_select_dev(n_rows, rows, n_items, scores, ld, impossible, default_est, offset, low, high, u_ptr,
                             ui_idx, n, items_out, est_out, count_out, (cudaStream_t)stream);
+}
+
+int sb2_fcp_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r, const double* est,
+                       int64_t* counts, void* stream) {
+    SB2_TRY(ensure_device());
+    return fcp_counts_dev(n_seg, n, seg_ptr, r, est, counts, (cudaStream_t)stream);
+}
+
+int sb2_precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r,
+                                  const double* est, const int64_t* k_eff, double threshold, int64_t* counts,
+                                  void* stream) {
+    SB2_TRY(ensure_device());
+    return precision_at_k_counts_dev(n_seg, n, seg_ptr, r, est, k_eff, threshold, counts, (cudaStream_t)stream);
 }
 
 int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,
