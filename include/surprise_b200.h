@@ -161,6 +161,12 @@ void sb2_svd_plan_destroy(sb2_svd_plan* plan);
 /* algorithmic bytes per rating update of the plan's kernel (DESIGN.md: 2*(2f+2)*4 + 12 for SVD) */
 int64_t sb2_svd_plan_bytes_per_update(const sb2_svd_plan* plan);
 int sb2_svd_plan_grid(const sb2_svd_plan* plan, int* n_blocks, int* n_sub);
+/* Read-only layout of a plan (any pointer may be NULL): B blocks (CTAs), cluster size C (1 = no clusters), G lanes per
+ * rating, CH 128-bit chunks per lane (0: 32 lanes stride the row), W lane-groups per CTA, whether the user / item
+ * rows of a block are staged in shared memory, dependency-driven cells, dynamic shared memory per CTA, records of a
+ * cell staged in shared memory, and the largest cell.  A plan with C > 1 always has stage_i == 1. */
+int sb2_svd_plan_layout(const sb2_svd_plan* plan, int* n_blocks, int* cluster, int* lanes, int* chunks, int* n_sub,
+                        int* stage_u, int* stage_i, int* dep_mode, int64_t* smem_bytes, int* rec_cap, int* max_cell);
 /* Synchronises `stream` and reports whether the persistent kernel ran to completion: every wait of a CTA for a
  * neighbour CTA / rank is bounded (~6 s); if a partner was never scheduled (SMs held by another persistent kernel,
  * a dead peer rank) the launch drains and this returns SB2_ERR_CUDA instead of the GPU hanging.  The host forms

@@ -63,6 +63,7 @@ SIGNATURES = {
     "sb2_svd_plan_destroy": (None, [_vp]),
     "sb2_svd_plan_bytes_per_update": (_i64, [_vp]),
     "sb2_svd_plan_grid": (_int, [_vp, _vp, _vp]),
+    "sb2_svd_plan_layout": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb2_svd_plan_status": (_int, [_vp, _vp]),
     "sb2_svd_ring_create_dev": (_int, [_i64, _i64, _i64, _vp, _vp, _vp, _vp, _int, _vp, _vp, _int, _int, _vp, _vp]),
     "sb2_svd_ring_ipc_handle": (_int, [_vp, _vp]),

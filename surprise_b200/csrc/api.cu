@@ -104,6 +104,8 @@ int svd_plan_read_dev(sb2_svd_plan* p, double* pu, double* qi, double* bu, doubl
 void svd_plan_destroy(sb2_svd_plan* p);
 int64_t svd_plan_bytes_per_update(const sb2_svd_plan* p);
 void svd_plan_grid(const sb2_svd_plan* p, int* b, int* w);
+void svd_plan_layout(const sb2_svd_plan* p, int* b, int* c, int* g, int* ch, int* w, int* stage_u, int* stage_i,
+                     int* dep_mode, int64_t* smem, int* rec_cap, int* max_cell);
 int svd_plan_status(sb2_svd_plan* p, cudaStream_t st);
 int svd_ring_epoch_dev(sb2_svd_plan* p, int phase, float* xch, cudaStream_t st);
 int svd_ring_run_local(sb2_svd_plan** plans, int n, int n_epochs, cudaStream_t st);
@@ -543,6 +545,16 @@ int sb2_svd_plan_profile(const sb2_svd_plan* plan, int64_t* cycles_host) {
 }
 int sb2_svd_plan_grid(const sb2_svd_plan* plan, int* n_blocks, int* n_sub) {
     svd_plan_grid(plan, n_blocks, n_sub);
+    return SB2_OK;
+}
+int sb2_svd_plan_layout(const sb2_svd_plan* plan, int* n_blocks, int* cluster, int* lanes, int* chunks, int* n_sub,
+                        int* stage_u, int* stage_i, int* dep_mode, int64_t* smem_bytes, int* rec_cap, int* max_cell) {
+    if (!plan) {
+        set_error("svd_plan_layout: null plan");
+        return SB2_ERR_INVALID;
+    }
+    svd_plan_layout(plan, n_blocks, cluster, lanes, chunks, n_sub, stage_u, stage_i, dep_mode, smem_bytes, rec_cap,
+                    max_cell);
     return SB2_OK;
 }
 

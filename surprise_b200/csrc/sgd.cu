@@ -1529,17 +1529,13 @@ int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32
         }
     }
     // largest cluster size (16 is the non-portable maximum, 7 such clusters are co-resident on a B200) that
-    // leaves at least two clusters, fits two item buffers in shared memory and passes the occupancy query
+    // leaves at least two clusters, fits two item buffers in shared memory and passes the occupancy query.
+    // Clusters hand item blocks through shared memory only, so the two buffers must fit at the B the plan finally
+    // runs with: capping B at the co-resident clusters makes the item blocks larger (27 000 items, f = 100:
+    // B 144 -> 112, 188 -> 242 rows), and a cluster size whose buffers no longer fit there is rejected.
     int c_first = 16;
     if (const char* e = getenv("SB2_DSGD_CLUSTER")) c_first = atoi(e);
-    bool clustered = false;
-    for (int Cc = 16; Cc >= 2 && !clustered; Cc >>= 1) {
-        if (Cc > c_first || b_lim < 2 * Cc) continue;
-        int Bc = b_lim / Cc * Cc;
-        p->B = Bc; p->C = Cc;
-        plan_smem(Bc, Cc, &p->stage_i, &p->stage_u, &smem_used, &p->ibuf);
-        if (!p->stage_i) continue;
-        p->smem = smem_used + 256 * 32 + 64;
+    auto max_active_clusters = [&](int Bc, int Cc) {
         dsgd_kernel_t kern = dsgd_kernel(p);
         int max_clusters = 0;
         cudaLaunchConfig_t cfg;
@@ -1552,8 +1548,25 @@ int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32
             cudaGetLastError();
             max_clusters = 0;
         }
+        return max_clusters;
+    };
+    bool clustered = false;
+    for (int Cc = 16; Cc >= 2 && !clustered; Cc >>= 1) {
+        if (Cc > c_first || b_lim < 2 * Cc) continue;
+        int Bc = b_lim / Cc * Cc;
+        p->B = Bc; p->C = Cc;
+        plan_smem(Bc, Cc, &p->stage_i, &p->stage_u, &smem_used, &p->ibuf);
+        if (!p->stage_i) continue;
+        const int max_clusters = max_active_clusters(Bc, Cc);
         if (max_clusters < 2) continue;
-        if (Bc / Cc > max_clusters) Bc = max_clusters * Cc;
+        if (Bc / Cc > max_clusters) {
+            Bc = max_clusters * Cc;
+            p->B = Bc;
+            plan_smem(Bc, Cc, &p->stage_i, &p->stage_u, &smem_used, &p->ibuf);
+            if (!p->stage_i) continue;
+            // the staging variant may have changed with B: its kernel must fit as many clusters
+            if (max_active_clusters(Bc, Cc) < Bc / Cc) continue;
+        }
         B = Bc;
         C = Cc;
         clustered = true;
@@ -1575,6 +1588,11 @@ int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32
     auto fail = [&](int rc) { plan_free(p); return rc; };
     if (P > 1 && !p->stage_i) {
         set_error("svd ring: item blocks of %d rows x %d factors do not fit in shared memory", max_il, f);
+        return fail(SB2_ERR_UNSUPPORTED);
+    }
+    if (C > 1 && !p->stage_i) {   // the DSMEM hop copies the item buffer: a cluster without one has nothing to copy
+        set_error("svd_plan: clusters of %d CTAs need two item buffers of %d rows x %d factors in shared memory", C,
+                  max_il, f);
         return fail(SB2_ERR_UNSUPPORTED);
     }
 #define PLAN_CUDA(expr)                                                                        \
@@ -1776,6 +1794,12 @@ int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32
     p->rec_cap = rec_cap;
     p->max_cell = status_h[1];
     p->smem = smem_used + (size_t)rec_cap * rec_bytes + 64;
+    int smem_optin = 0;
+    PLAN_CUDA(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, p->device));
+    if (p->smem > (size_t)smem_optin) {
+        set_error("svd_plan: %zu bytes of shared memory per CTA exceed the device's %d", p->smem, smem_optin);
+        return fail(SB2_ERR_UNSUPPORTED);
+    }
     *out = p;
     return SB2_OK;
 }
@@ -2141,6 +2165,20 @@ int64_t svd_plan_bytes_per_update(const sb2_svd_plan* p) {
 void svd_plan_grid(const sb2_svd_plan* p, int* b, int* w) {
     if (b) *b = p->B;
     if (w) *w = p->W;
+}
+void svd_plan_layout(const sb2_svd_plan* p, int* b, int* c, int* g, int* ch, int* w, int* stage_u, int* stage_i,
+                     int* dep_mode, int64_t* smem, int* rec_cap, int* max_cell) {
+    if (b) *b = p->B;
+    if (c) *c = p->C;
+    if (g) *g = p->G;
+    if (ch) *ch = p->CH;
+    if (w) *w = p->W;
+    if (stage_u) *stage_u = p->stage_u ? 1 : 0;
+    if (stage_i) *stage_i = p->stage_i ? 1 : 0;
+    if (dep_mode) *dep_mode = p->dep_mode ? 1 : 0;
+    if (smem) *smem = (int64_t)p->smem;
+    if (rec_cap) *rec_cap = p->rec_cap;
+    if (max_cell) *max_cell = p->max_cell;
 }
 void svd_plan_dims(const sb2_svd_plan* p, int64_t* n_users, int64_t* n_items, int* f, int* with_yj) {
     *n_users = p->n_users; *n_items = p->n_items; *f = p->prm.n_factors; *with_yj = p->with_yj ? 1 : 0;

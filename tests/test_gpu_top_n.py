@@ -269,25 +269,12 @@ def reference_top_n(algo, ts, users, n):
     return out_i, out_e
 
 
-def assigned_svd(ts, f, seed=0):
-    """An SVD whose factors and biases are drawn, not trained (top-N only reads them)."""
-    algo = sb.SVD(n_factors=f)
-    sb.AlgoBase.fit(algo, ts)
-    rng = np.random.RandomState(seed)
-    algo.pu, algo.qi = rng.normal(0, .3, (ts.n_users, f)), rng.normal(0, .3, (ts.n_items, f))
-    algo.bu, algo.bi = rng.normal(0, .3, ts.n_users), rng.normal(0, .3, ts.n_items)
-    return algo
-
-
 @pytest.mark.parametrize("shape", ["ml-1m", "ml-20m"])
 def test_scale(shape):
     d = synth.shaped(shape, seed=0)
     u, i, r = d["train"]
     ts = sb.Trainset.from_coo(u, i, r, d["n_users"], d["n_items"], (0.5, 5.0) if shape == "ml-20m" else (1, 5))
-    if shape == "ml-1m":
-        algo = sb.SVD(n_factors=100, n_epochs=2, random_state=0).fit(ts)
-    else:
-        algo = assigned_svd(ts, 100)
+    algo = sb.SVD(n_factors=100, n_epochs=2, random_state=0).fit(ts)
     cnt = np.diff(ts.user_csr()[0])
     if shape == "ml-1m":
         users = np.arange(ts.n_users, dtype=np.int32)
