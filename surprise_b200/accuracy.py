@@ -1,4 +1,4 @@
-"""rmse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), and the FAQ's
+"""rmse / mse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), and the FAQ's
 precision_recall_at_k.
 
 fcp and precision_recall_at_k reduce to integer counts per user.  Where a CUDA device is usable and every r_ui and est
@@ -11,7 +11,7 @@ from operator import index, itemgetter
 
 import numpy as np
 
-__all__ = ["rmse", "mae", "fcp", "precision_recall_at_k"]
+__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k"]
 
 
 def _need(predictions):
@@ -20,11 +20,17 @@ def _need(predictions):
 
 
 def rmse(predictions, verbose=True):
-    _need(predictions)
-    mse = np.mean([float((true_r - est) ** 2) for (_, _, true_r, est, _) in predictions])
-    out = np.sqrt(mse)
+    out = np.sqrt(mse(predictions, verbose=False))
     if verbose:
         print("RMSE: {0:1.4f}".format(out))
+    return out
+
+
+def mse(predictions, verbose=True):
+    _need(predictions)
+    out = np.mean([float((true_r - est) ** 2) for (_, _, true_r, est, _) in predictions])
+    if verbose:
+        print("MSE: {0:1.4f}".format(out))
     return out
 
 
@@ -38,7 +44,10 @@ def mae(predictions, verbose=True):
 
 def fcp(predictions, verbose=True):
     _need(predictions)
-    nc, nd = _fcp_counts(predictions)
+    return _fcp_of_counts(*_fcp_counts(predictions), verbose)
+
+
+def _fcp_of_counts(nc, nd, verbose):
     c_mean = np.mean(list(nc.values())) if nc else 0
     d_mean = np.mean(list(nd.values())) if nd else 0
     try:
@@ -224,3 +233,31 @@ def _precision_recall_dev(keys, code, r_ui, est, has_numpy, k, threshold):
         for u, user_ratings in user_est_true.items():
             precisions[keys[u]], recalls[keys[u]] = _precision_recall_user(user_ratings, k, threshold)
     return precisions, recalls
+
+
+# -- measures of predictions held in arrays (model_selection's array route) ------------------------------------------
+ARRAY_MEASURES = ("rmse", "mse", "mae", "fcp")
+
+
+def _of_arrays(measure, r_ui, est, users):
+    """``measure(predictions, verbose=False)`` with the same bits, for predictions given as float64 arrays r_ui and est
+    (measure one of ARRAY_MEASURES).  ``users()`` returns (code, n_users): each prediction's user numbered in first
+    appearance order, equal uids merged, as fcp groups them; it is only called for fcp.
+
+    The squares are Python's ``d ** 2``, which calls libm's pow as the tuple route does: ``d * d`` and np.square
+    round differently from glibc's pow for some d.  The sums are np.mean's pairwise sum over the same sequence."""
+    if not len(r_ui):
+        _need(())
+    d = r_ui - est
+    if measure == "mae":
+        return np.mean(np.abs(d))
+    if measure in ("mse", "rmse"):
+        out = np.mean([x ** 2 for x in d.tolist()])
+        return out if measure == "mse" else np.sqrt(out)
+    code, n_users = users()
+    if _device_usable():
+        nc, nd = _fcp_counts_dev(range(n_users), code, r_ui, est, False)
+    else:
+        n = len(code)
+        nc, nd = _fcp_counts(list(zip(code.tolist(), [None] * n, r_ui.tolist(), est.tolist(), [None] * n)))
+    return _fcp_of_counts(nc, nd, False)

@@ -110,6 +110,12 @@ class ShuffleSplit(object):
         return self.n_splits
 
 
+def get_cv(cv):
+    """The splitter cross_validate and the searches use: 5-fold KFold for None, KFold(n_splits=cv) for an int, cv
+    itself otherwise."""
+    return KFold(n_splits=5) if cv is None else (KFold(n_splits=cv) if isinstance(cv, int) else cv)
+
+
 def train_test_split(data, test_size=.2, train_size=None, random_state=None, shuffle=True):
     """split.py:543-583: one ShuffleSplit draw."""
     ss = ShuffleSplit(n_splits=1, test_size=test_size, train_size=train_size, random_state=random_state,

@@ -123,6 +123,22 @@ class AlgoBase(object):
     def default_prediction(self):
         return self.trainset.global_mean
 
+    def _final_estimates(self, est, code):
+        """The values test() gives a batch of raw estimates: ``default_prediction()`` where ``code`` is 1 (impossible),
+        ZeroDivisionError if any code is 2 (KNNBasic with min_k <= 0 and no positive neighbour), then minus the offset
+        and clipped to the rating scale as predict() clips one estimate.  ``code`` may be None (nothing impossible)."""
+        est = np.array(est, dtype=np.float64)
+        if code is not None:
+            code = np.asarray(code)
+            if (code == 2).any():
+                raise ZeroDivisionError("division by zero")
+            imp = code == 1
+            if imp.any():
+                est[imp] = self.default_prediction()
+        est -= self.trainset.offset
+        low, high = self.trainset.rating_scale
+        return np.maximum(low, np.minimum(high, est))      # est = min(high, est); est = max(low, est)
+
     def _batched(self):
         cls = type(self)
         return cls._batch_estimate_of is not None and _func(cls.estimate) is _func(cls._batch_estimate_of)
@@ -142,13 +158,8 @@ class AlgoBase(object):
         iids = [row[1] for row in rows]
         iu, ii = ts.to_inner_uids(uids), ts.to_inner_iids(iids)
         est, details = self._estimate_batch(iu, ii)
-        est = np.asarray(est, dtype=np.float64).copy()
-        imp = np.fromiter((bool(d.get("was_impossible")) for d in details), dtype=bool, count=n)
-        if imp.any():
-            est[imp] = self.default_prediction()
-        est -= off
-        low, high = ts.rating_scale
-        est = np.maximum(low, np.minimum(high, est))      # est = min(high, est); est = max(low, est)
+        imp = np.fromiter((bool(d.get("was_impossible")) for d in details), dtype=np.uint8, count=n)
+        est = self._final_estimates(est, imp)
         r_ui = (np.fromiter((row[2] for row in rows), dtype=np.float64, count=n) - off).tolist()
         out = [Prediction(uid, iid, r, e, d) for uid, iid, r, e, d in zip(uids, iids, r_ui, est.tolist(), details)]
         if verbose:
