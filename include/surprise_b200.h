@@ -406,6 +406,23 @@ int sb2_precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_p
                                   void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Hits of top-N lists against held-out relevant items (AlgoBase.top_n_measures; the definition is
+ * accuracy.top_n_measures, DESIGN.md section 3.9).  All arrays are DEVICE arrays.  items (int32, row b at
+ * items + b * ld) and count (int32 per row) are a block of sb2_top_n_select_dev's output; w <= ld is the
+ * cutoff.  Row b's relevant items are rel_idx[rel_ptr[b], rel_ptr[b + 1]) (rel_ptr int64, n_rows + 1
+ * entries, offsets into rel_idx of rel_len entries), distinct inner item ids in strictly ascending order.
+ * With H_b = {p < min(count[b], w) : items[b * ld + p] in row b's list}:
+ *   hits[b] = |H_b|, rr[b] = the sum of inv[p] over H_b, dcg[b] = the sum of disc[p] over H_b,
+ * each sum taken in ascending p from +0.0 with one fp64 add per term (no FMA).  inv and disc (fp64, at least w
+ * entries) are the host's tables, so no logarithm is evaluated on the device.  SB2_ERR_INVALID for a null
+ * pointer, w < 0, ld < w, or offsets outside [0, rel_len], decreasing, or a list not strictly ascending (checked
+ * inside the kernel).  One launch per call; the call synchronises `stream` to read that check.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_top_n_hits_dev(int64_t n_rows, const int32_t* items, int64_t ld, const int32_t* count, int w,
+                       const int64_t* rel_ptr, const int32_t* rel_idx, int64_t rel_len, const double* inv,
+                       const double* disc, int32_t* hits, double* rr, double* dcg, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Row shard of a SYMMETRIC multi-rank similarity build (SURVEY.md 8e "cyclic upper-triangular tile sharding").
  * Same arguments as sb2_sim_build_dev, but only sim[i][j] with row_begin <= i < row_end and j >= row_begin is
  * computed (tiles at or above the block diagonal; the shard's own diagonal square is mirrored like the

@@ -1,17 +1,19 @@
-"""rmse / mse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), and the FAQ's
-precision_recall_at_k.
+"""rmse / mse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), the FAQ's
+precision_recall_at_k, and top_n_measures: hit rate, ARHR, precision@N, recall@N and nDCG@N of get_top_n output against
+held-out ratings.
 
 fcp and precision_recall_at_k reduce to integer counts per user.  Where a CUDA device is usable and every r_ui and est
 is a real number that float64 holds exactly, the counts come from the device (csrc/rank_metrics.cu, DESIGN.md section
 3.7); otherwise from the Python loops below, which are the metrics' definition (and what the tests compare against).
 The arithmetic on the counts runs on the host either way, so both routes return the same values.
 """
+import re
 from collections import defaultdict
 from operator import index, itemgetter
 
 import numpy as np
 
-__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k"]
+__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k", "top_n_measures"]
 
 
 def _need(predictions):
@@ -119,6 +121,94 @@ def _fcp_counts(predictions):
                     d += 1
         nc[u0], nd[u0] = c, d
     return nc, nd
+
+
+def top_n_measures(top_n, testset, n, threshold=None, offset=0, verbose=True):
+    """Top-N measures of ``top_n`` (get_top_n output, ``{raw uid: [(raw iid, est), ...]}``) against the held-out rows
+    ``(raw uid, raw iid, r_ui)`` of ``testset``, as a dict of floats with keys hr, arhr, precision, recall, ndcg.
+
+    This plain-Python function is what the measures mean: AlgoBase.top_n_measures computes them on the device and the
+    tests compare it against this function.
+
+    * A row is relevant when ``threshold`` is None or ``r_ui - offset >= threshold`` (``r_ui - offset`` is the value
+      ``test()`` reports: a float64 subtraction, then a Python compare).
+    * The evaluated users U* are the uids with at least one relevant row, in first-appearance order, equal uids merged
+      as dict keys merge them.  No such user raises ValueError.
+    * R_u is the set of u's relevant raw iids (duplicates collapse; items the trainset does not know count).  L_u is
+      the first n raw iids of ``top_n.get(u, [])``, and H_u the positions p (0-based, ascending) with L_u[p] in R_u.
+      A user absent from ``top_n`` (unknown to the trainset, or who rated every item) has no hits but is evaluated.
+    * With the host tables inv[p] = 1.0 / (p + 1), disc[p] = 1.0 / np.log2(p + 2) and idcg[m] the left-to-right sum of
+      disc[:m]: hits_u = |H_u|, rr_u and dcg_u the left-to-right sums from 0.0 of inv[p] and disc[p] over H_u,
+      prec_u = hits_u / n, rec_u = hits_u / |R_u|, ndcg_u = dcg_u / idcg[min(|R_u|, n)].
+    * hr = sum(hits_u) / sum(|R_u|), arhr = float(np.sum(rr)) / sum(|R_u|); precision, recall and ndcg are
+      float(np.mean(...)) of the per-user values in U* order.
+
+    With one held-out rating per user (LeaveOneOut) and threshold None, hr is the leave-one-out hit rate and arhr the
+    average reciprocal hit rank.  ``n`` must be an int >= 1."""
+    from .prediction_algorithms.algo_base import _check_top_n
+    n = _check_top_n(n)
+    relevant = {}
+    for uid, iid, r_ui in testset:
+        if threshold is None or float(r_ui) - offset >= threshold:
+            relevant.setdefault(uid, set()).add(iid)
+    if not relevant:
+        raise ValueError("top-N measures need at least one relevant rating in the testset")
+    lists = [[iid for iid, _ in top_n.get(u, [])][:n] for u in relevant]
+    inv, disc, idcg = _rank_tables(min(n, max(max(map(len, lists)), max(map(len, relevant.values())))))
+    inv, disc = inv.tolist(), disc.tolist()
+    hits, rr, dcg = [], [], []
+    for r_u, l_u in zip(relevant.values(), lists):
+        h, a, d = 0, 0.0, 0.0
+        for p, iid in enumerate(l_u):
+            if iid in r_u:
+                h += 1
+                a += inv[p]
+                d += disc[p]
+        hits.append(h)
+        rr.append(a)
+        dcg.append(d)
+    return _top_n_of_counts(hits, rr, dcg, [len(r_u) for r_u in relevant.values()], n, idcg, verbose)
+
+
+def _rank_tables(m):
+    """inv[p] = 1.0 / (p + 1) and disc[p] = 1.0 / np.log2(p + 2) for p < m (float64 arrays; an entry does not depend
+    on m), and idcg[k] = the left-to-right sum of disc[:k] for k <= m."""
+    p = np.arange(m, dtype=np.float64)
+    inv, disc = 1.0 / (p + 1), 1.0 / np.log2(p + 2)
+    idcg = [0.0]
+    for d in disc.tolist():
+        idcg.append(idcg[-1] + d)
+    return inv, disc, np.array(idcg)
+
+
+_TOP_N_LABELS = {"hr": "HR", "arhr": "ARHR", "precision": "Precision", "recall": "Recall", "ndcg": "nDCG"}
+
+
+def _top_n_of_counts(hits, rr, dcg, n_rel, n, idcg, verbose):
+    """top_n_measures' result from the per-user hits, rr, dcg and |R_u| in U* order (both routes end here)."""
+    hits, n_rel = np.asarray(hits, dtype=np.int64), np.asarray(n_rel, dtype=np.int64)
+    rr, dcg = np.asarray(rr, dtype=np.float64), np.asarray(dcg, dtype=np.float64)
+    total = int(n_rel.sum())
+    out = {"hr": int(hits.sum()) / total,
+           "arhr": float(np.sum(rr)) / total,
+           "precision": float(np.mean(hits / n)),
+           "recall": float(np.mean(hits / n_rel)),
+           "ndcg": float(np.mean(dcg / idcg[np.minimum(n_rel, n)]))}
+    if verbose:
+        for key, label in _TOP_N_LABELS.items():
+            print("{0}@{1}:  {2:1.4f}".format(label, n, out[key]))
+    return out
+
+
+def _top_n_measure(name):
+    """(key, N) for a measure name key@N with key in hr, arhr, precision, recall, ndcg (any case) and N an int >= 1;
+    None for any other name.  A top-N key with a malformed N raises ValueError."""
+    key, at, num = name.lower().partition("@")
+    if not at or key not in _TOP_N_LABELS:
+        return None
+    if not re.fullmatch("[0-9]+", num) or int(num) < 1:
+        raise ValueError("%s: N in %s@N must be an int >= 1" % (name, key))
+    return key, int(num)
 
 
 # -- device route ----------------------------------------------------------------------------------------------------

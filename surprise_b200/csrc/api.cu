@@ -95,6 +95,9 @@ int fcp_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const doubl
                    int64_t* counts, cudaStream_t st);
 int precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_ptr, const double* r, const double* est,
                               const int64_t* k_eff, double threshold, int64_t* counts, cudaStream_t st);
+int top_n_hits_dev(int64_t n_rows, const int32_t* items, int64_t ld, const int32_t* count, int w,
+                   const int64_t* rel_ptr, const int32_t* rel_idx, int64_t rel_len, const double* inv,
+                   const double* disc, int32_t* hits, double* rr, double* dcg, cudaStream_t st);
 int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32_t* u, const int32_t* i,
                         const double* r, const sb2_sgd_params* prm, int with_yj, const int64_t* u_ptr,
                         const int32_t* ui_idx, int rank, int world, cudaStream_t st, sb2_svd_plan** out);
@@ -817,6 +820,14 @@ int sb2_precision_at_k_counts_dev(int64_t n_seg, int64_t n, const int64_t* seg_p
                                   void* stream) {
     SB2_TRY(ensure_device());
     return precision_at_k_counts_dev(n_seg, n, seg_ptr, r, est, k_eff, threshold, counts, (cudaStream_t)stream);
+}
+
+int sb2_top_n_hits_dev(int64_t n_rows, const int32_t* items, int64_t ld, const int32_t* count, int w,
+                       const int64_t* rel_ptr, const int32_t* rel_idx, int64_t rel_len, const double* inv,
+                       const double* disc, int32_t* hits, double* rr, double* dcg, void* stream) {
+    SB2_TRY(ensure_device());
+    return top_n_hits_dev(n_rows, items, ld, count, w, rel_ptr, rel_idx, rel_len, inv, disc, hits, rr, dcg,
+                          (cudaStream_t)stream);
 }
 
 int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,

@@ -12,6 +12,28 @@ from .reader import Reader
 from .trainset import Trainset
 
 
+def first_appearance(a):
+    """(code, uniq): each entry's rank among the distinct values of a in first-appearance order (int32), and those
+    values in that order."""
+    n = len(a)
+    if n and np.issubdtype(a.dtype, np.integer) and int(a.max()) - int(a.min()) <= max(4 * n, 10_000_000):
+        # integer raw ids in a modest range: O(N) table instead of a sort of all the ratings
+        lo = int(a.min())
+        shifted = (a - lo).astype(np.int64)
+        first = np.full(int(shifted.max()) + 1, n, dtype=np.int64)
+        first[shifted[::-1]] = np.arange(n - 1, -1, -1, dtype=np.int64)   # repeated index: last write wins
+        present = np.nonzero(first < n)[0]
+        order = np.argsort(first[present], kind="stable")
+        rank = np.empty(len(first), dtype=np.int32)
+        rank[present[order]] = np.arange(len(present), dtype=np.int32)
+        return rank[shifted], (present[order] + lo).astype(a.dtype)
+    uniq, first, inv = np.unique(a, return_index=True, return_inverse=True)
+    order = np.argsort(first, kind="stable")          # uniq[order] is in first-appearance order
+    rank = np.empty(len(uniq), dtype=np.int64)
+    rank[order] = np.arange(len(uniq))
+    return rank[inv].astype(np.int32), uniq[order]
+
+
 class Dataset(object):
     def __init__(self, reader):
         self.reader = reader
@@ -56,24 +78,6 @@ class Dataset(object):
         return ts
 
     def _trainset_from_arrays(self, uids, iids, ratings):
-        def first_appearance(a):
-            n = len(a)
-            if n and np.issubdtype(a.dtype, np.integer) and int(a.max()) - int(a.min()) <= max(4 * n, 10_000_000):
-                # integer raw ids in a modest range: O(N) table instead of a sort of all the ratings
-                lo = int(a.min())
-                shifted = (a - lo).astype(np.int64)
-                first = np.full(int(shifted.max()) + 1, n, dtype=np.int64)
-                first[shifted[::-1]] = np.arange(n - 1, -1, -1, dtype=np.int64)   # repeated index: last write wins
-                present = np.nonzero(first < n)[0]
-                order = np.argsort(first[present], kind="stable")
-                rank = np.empty(len(first), dtype=np.int32)
-                rank[present[order]] = np.arange(len(present), dtype=np.int32)
-                return rank[shifted], (present[order] + lo).astype(a.dtype)
-            uniq, first, inv = np.unique(a, return_index=True, return_inverse=True)
-            order = np.argsort(first, kind="stable")          # uniq[order] is in first-appearance order
-            rank = np.empty(len(uniq), dtype=np.int64)
-            rank[order] = np.arange(len(uniq))
-            return rank[inv].astype(np.int32), uniq[order]
         u, raw_u = first_appearance(np.asarray(uids))
         i, raw_i = first_appearance(np.asarray(iids))
         r = np.asarray(ratings, dtype=np.float64) + self.reader.offset

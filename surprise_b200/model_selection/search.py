@@ -12,6 +12,7 @@ from itertools import product
 
 import numpy as np
 
+from .. import accuracy
 from ..dataset import DatasetUserFolds
 from ..utils import get_rng
 from .split import get_cv
@@ -83,7 +84,7 @@ class BaseSearchCV(object):
             if m in ("mae", "rmse", "mse"):
                 rank[indices] = np.arange(len(indices)) + 1
                 best_index[m] = mean_test_measures.argmin()
-            elif m in ("fcp",):
+            elif m == "fcp" or accuracy._top_n_measure(m):
                 rank[indices] = np.arange(len(indices), 0, -1)
                 best_index[m] = mean_test_measures.argmax()
             best_params[m] = self.param_combinations[best_index[m]]

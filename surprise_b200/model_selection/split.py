@@ -1,6 +1,7 @@
 """Cross-validation iterators (reference: model_selection/split.py): KFold (:57-122), RepeatedKFold (:365-415),
-ShuffleSplit (:418-540), train_test_split (:543-583), PredefinedKFold (:654-685).  Same index arithmetic and the
-same RNG calls as the reference, so a given random_state yields the same trainset / testset rows.
+ShuffleSplit (:418-540), train_test_split (:543-583), PredefinedKFold (:654-685), and upstream Surprise 1.1's
+LeaveOneOut.  Same index arithmetic and the same RNG calls as the reference, so a given random_state yields the same
+trainset / testset rows.
 
 All of them work on index arrays and hand them to ``Dataset._take``: a list-backed dataset yields the reference's
 raw-rating lists, an array-backed one (Dataset.load_from_arrays) slices its three arrays, so that 10^7..10^8
@@ -10,6 +11,7 @@ from math import ceil, floor
 
 import numpy as np
 
+from ..dataset import first_appearance
 from ..utils import get_rng
 
 
@@ -105,6 +107,51 @@ class ShuffleSplit(object):
             train = data._take(perm[:n_train])
             test = data._take(perm[n_train:n_train + n_test])
             yield data.construct_trainset(train), data.construct_testset(test)
+
+    def get_n_folds(self):
+        return self.n_splits
+
+
+class LeaveOneOut(object):
+    """Each split holds out one rating per user: upstream Surprise 1.1's LeaveOneOut, restated here.
+
+    The reference groups ``data.raw_ratings`` by uid into a ``defaultdict(list)`` (users in first-appearance order,
+    equal uids merged, each user's ratings in file order) and draws ``rng = get_rng(random_state)`` once for the whole
+    iterator.  Then, for each of the ``n_splits`` splits and each user with ``len(ratings) > min_n_ratings``, in group
+    order, it draws ``k = rng.randint(0, len(ratings))``, appends ``ratings[k]`` to the testset and the user's other
+    ratings, in order, to the trainset.  Users at or below ``min_n_ratings`` are in neither set.  An empty trainset
+    raises ``ValueError('Could not build any trainset. Maybe min_n_ratings is too high?')``.
+
+    The trainset is therefore in user-grouped order, not file order, and its inner item ids differ from the ones KFold
+    assigns.  Here the groups are index arrays (a stable sort of the first-appearance user codes), and the per-user
+    draws of one split are one ``rng.randint(0, lengths)`` call, which consumes the RandomState's stream exactly as
+    the scalar draws in user order do.  An array-backed dataset is split without creating tuples."""
+
+    def __init__(self, n_splits=5, random_state=None, min_n_ratings=0):
+        self.n_splits, self.random_state, self.min_n_ratings = n_splits, random_state, min_n_ratings
+
+    def split(self, data):
+        if data._arrays is not None:
+            code, uniq = first_appearance(data._arrays[0])
+            n_users = len(uniq)
+        else:
+            users = {}
+            setd = users.setdefault
+            code = np.array([setd(row[0], len(users)) for row in data.raw_ratings], dtype=np.int64)
+            n_users = len(users)
+        order = np.argsort(code, kind="stable")         # row indices grouped by user, file order within a user
+        length = np.bincount(code, minlength=n_users)
+        start = np.cumsum(length) - length
+        kept = np.flatnonzero(length > self.min_n_ratings)
+        in_kept = np.repeat(length > self.min_n_ratings, length)     # per entry of order
+        rng = get_rng(self.random_state)
+        for _ in range(self.n_splits):
+            test = start[kept] + rng.randint(0, length[kept]) if len(kept) else kept
+            train = in_kept.copy()
+            train[test] = False
+            if not train.any():
+                raise ValueError("Could not build any trainset. Maybe min_n_ratings is too high?")
+            yield data.construct_trainset(data._take(order[train])), data.construct_testset(data._take(order[test]))
 
     def get_n_folds(self):
         return self.n_splits

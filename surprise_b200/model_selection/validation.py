@@ -5,7 +5,8 @@ only multiply CUDA contexts.
 fit_and_score scores a device-batched algorithm from arrays: the fold's pairs are mapped to inner ids once
 (``Fold``), the estimates come from the algorithm's device estimate and the measures from
 ``accuracy._of_arrays``, which gives the bits ``accuracy.<m>(algo.test(testset))`` gives without building a
-Prediction per pair.  Any other algorithm or measure takes the tuple route.
+Prediction per pair.  Any other algorithm or rating measure takes the tuple route.  The top-N measures hr@N,
+arhr@N, precision@N, recall@N and ndcg@N (threshold None) come from one ``algo._top_n_measures`` pass per fold.
 """
 import time
 
@@ -18,9 +19,9 @@ from .split import get_cv
 class _Pairs(object):
     """Prediction pairs as arrays: inner ids (-1 unknown), r_ui minus the offset, and the users fcp groups by."""
 
-    def __init__(self, iu, ii, r_ui, uids=None, users=None):
+    def __init__(self, iu, ii, r_ui, uids=None, users=None, iids=None):
         self.iu, self.ii, self.r_ui = iu, ii, r_ui
-        self._uids, self._users, self._dev = uids, users, None
+        self._uids, self._users, self._dev, self._iids = uids, users, None, iids
 
     def device_ids(self):
         if self._dev is None:
@@ -37,6 +38,45 @@ class _Pairs(object):
             self._users = code, len(codes)
         return self._users
 
+    def relevant(self, threshold, n_items):
+        """The held-out relevant items of accuracy.top_n_measures: (iu, n_rel, rel_ptr, rel_idx).  iu (int32) is the
+        inner uid (-1 unknown) of each evaluated user -- a user with at least one row whose r_ui (minus the offset) is
+        >= threshold, or with any row for threshold None -- in first-appearance order among those rows, equal raw uids
+        merged; n_rel (int64) their |R_u|, distinct raw iids counted, unknown items included.  rel_ptr (int64) /
+        rel_idx (int32) is the CSR, over the evaluated users the trainset knows, in that order, of their distinct
+        known relevant inner iids, ascending.  No evaluated user raises ValueError."""
+        n = len(self.r_ui)
+        if threshold is None:
+            rows = np.arange(n)
+        else:
+            rows = np.flatnonzero(np.fromiter((x >= threshold for x in self.r_ui.tolist()), dtype=bool, count=n))
+        if not len(rows):
+            raise ValueError("top-N measures need at least one relevant rating in the testset")
+        code = self.users()[0][rows]
+        _, first, inv = np.unique(code, return_index=True, return_inverse=True)
+        rank = np.empty(len(first), dtype=np.int64)
+        rank[np.argsort(first, kind="stable")] = np.arange(len(first))
+        star = rank[inv.reshape(-1)]                   # evaluated user of each relevant row
+        n_star = len(first)
+        iu = np.empty(n_star, dtype=np.int32)
+        iu[star] = self.iu[rows]                      # equal raw uids have one inner id
+        item = self.ii[rows].astype(np.int64)
+        unknown = np.flatnonzero(item < 0)
+        if len(unknown):                              # unknown items: numbered past n_items by raw iid
+            codes = {}
+            setd = codes.setdefault
+            item[unknown] = n_items + np.fromiter((setd(self._iids[k], len(codes)) for k in rows[unknown].tolist()),
+                                                  dtype=np.int64, count=len(unknown))
+        base = int(item.max()) + 1
+        k_user, k_item = np.divmod(np.unique(star * base + item), base)     # distinct (user, item), by user then item
+        n_rel = np.bincount(k_user, minlength=n_star)
+        known = iu >= 0
+        keep = known[k_user] & (k_item < n_items)
+        slot = np.cumsum(known) - 1                   # position of a known user among the known ones
+        rel_ptr = np.zeros(int(known.sum()) + 1, dtype=np.int64)
+        np.cumsum(np.bincount(slot[k_user[keep]], minlength=len(rel_ptr) - 1), out=rel_ptr[1:])
+        return iu, n_rel, rel_ptr, k_item[keep].astype(np.int32)
+
 
 class Fold(object):
     """One (trainset, testset) split, with the arrays its predictions are scored from built on first use and kept
@@ -51,9 +91,10 @@ class Fold(object):
             ts = self.trainset
             rows = self.testset.tolist() if isinstance(self.testset, np.ndarray) else list(self.testset)
             uids = [row[0] for row in rows]
-            iu, ii = ts.to_inner_uids(uids), ts.to_inner_iids([row[1] for row in rows])
+            iids = [row[1] for row in rows]
+            iu, ii = ts.to_inner_uids(uids), ts.to_inner_iids(iids)
             r_ui = np.fromiter((row[2] for row in rows), dtype=np.float64, count=len(rows)) - ts.offset
-            self._test = _Pairs(iu, ii, r_ui, uids=uids)
+            self._test = _Pairs(iu, ii, r_ui, uids=uids, iids=iids)
         return self._test
 
     def train_pairs(self):
@@ -81,9 +122,27 @@ def fit_and_score(algo, trainset, testset, measures, return_train_measures=False
 
 
 def _fit_and_score(algo, fold, measures, return_train_measures):
+    top_n = {m: accuracy._top_n_measure(m) for m in measures}
+    top_n = {m: v for m, v in top_n.items() if v is not None}
+    if top_n and return_train_measures:
+        raise ValueError("return_train_measures cannot be used with top-N measures (%s): trainset items are never "
+                         "recommended, so they would be 0" % ", ".join(top_n))
     t0 = time.time()
     algo.fit(fold.trainset)
     fit_time = time.time() - t0
+    rating = [m for m in measures if m not in top_n]
+    test_m, train_m, test_time = _score_ratings(algo, fold, rating, return_train_measures) if rating else ({}, {}, 0.0)
+    if top_n:
+        t0 = time.time()
+        ns = sorted(set(n for _, n in top_n.values()))
+        by_n = dict(zip(ns, algo._top_n_measures(fold, ns, None)))
+        test_time += time.time() - t0
+        test_m.update((m, by_n[n][key]) for m, (key, n) in top_n.items())
+        test_m = {m: test_m[m] for m in measures}
+    return test_m, train_m, fit_time, test_time
+
+
+def _score_ratings(algo, fold, measures, return_train_measures):
     if algo._batched() and all(m.lower() in accuracy.ARRAY_MEASURES for m in measures):
         t0 = time.time()
         test = fold.test_pairs()
@@ -95,7 +154,7 @@ def _fit_and_score(algo, fold, measures, return_train_measures):
             train = fold.train_pairs()
             est = _estimates(algo, train)
             train_m = {m: accuracy._of_arrays(m.lower(), train.r_ui, est, train.users) for m in measures}
-        return test_m, train_m, fit_time, test_time
+        return test_m, train_m, test_time
     t0 = time.time()
     predictions = algo.test(fold.testset)
     test_time = time.time() - t0
@@ -106,7 +165,7 @@ def _fit_and_score(algo, fold, measures, return_train_measures):
         test_m[m] = f(predictions, verbose=0)
         if return_train_measures:
             train_m[m] = f(train_predictions, verbose=0)
-    return test_m, train_m, fit_time, test_time
+    return test_m, train_m, test_time
 
 
 def cross_validate(algo, data, measures=["rmse", "mae"], cv=None, return_train_measures=False, n_jobs=1,

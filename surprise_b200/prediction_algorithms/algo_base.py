@@ -214,8 +214,17 @@ class AlgoBase(object):
         width = min(n, ts.n_items)
         if not self._batched():
             return self._top_n_by_test(width, users)
+        items, est, count = self._top_n_dev(width, users, _block_rows, _events)
+        n_u = len(users)
+        return items.cpu().numpy()[:n_u], est.cpu().numpy()[:n_u], count.cpu().numpy()[:n_u]
+
+    def _top_n_dev(self, width, users, _block_rows=None, _events=None, on_block=None):
+        """top_n_inner's device block loop: (items, est, count) as device arrays of max(len(users), 1) rows.
+        ``on_block(b0, nr, items, count)``, if given, is called after each block's selection, when rows b0 .. b0 + nr
+        of the device arrays are final."""
         from .. import _native as nat
         torch = nat.torch_cuda()
+        ts = self.trainset
         n_u, n_i = len(users), ts.n_items
         items = nat.empty_dev((max(n_u, 1), width), np.int32)
         est = nat.empty_dev((max(n_u, 1), width), np.float64)
@@ -258,7 +267,59 @@ class AlgoBase(object):
                                                nat.ptr(items[b0:]), nat.ptr(est[b0:]), nat.ptr(count[b0:]), stream))
             if ev:
                 ev[2].record()
-        return items.cpu().numpy()[:n_u], est.cpu().numpy()[:n_u], count.cpu().numpy()[:n_u]
+            if on_block is not None:
+                on_block(b0, nr, items, count)
+        return items, est, count
+
+    # -- top-N measures against held-out ratings -------------------------------------------------------
+    def top_n_measures(self, testset, n=10, threshold=None):
+        """Hit rate, ARHR, precision@n, recall@n and nDCG@n of this algorithm's top-n lists against the held-out rows
+        ``(raw uid, raw iid, r_ui)`` of ``testset``: bit for bit ``accuracy.top_n_measures(self.get_top_n(n), testset,
+        n, threshold, offset=self.trainset.offset, verbose=False)``, without building get_top_n's dict or any
+        Prediction.  Only the evaluated users the trainset knows are ranked; a device-batched algorithm scores their
+        lists against the relevant items on the device (sb2_top_n_hits_dev), any other one through get_top_n."""
+        from ..model_selection.validation import Fold
+        return self._top_n_measures(Fold(self.trainset, testset), [n], threshold)[0]
+
+    def _top_n_measures(self, fold, ns, threshold, _block_rows=None):
+        """top_n_measures for each cutoff of ``ns`` on the testset of ``fold`` (a validation.Fold of this trainset): the
+        lists are ranked once at the largest cutoff, whose first N entries are the top-N lists (the ranking is a total
+        order), and the hits are counted once per cutoff."""
+        from .. import accuracy
+        ns = [_check_top_n(n) for n in ns]
+        ts = self.trainset
+        iu, n_rel, rel_ptr, rel_idx = fold.test_pairs().relevant(threshold, ts.n_items)
+        known = iu >= 0
+        top = max(ns)
+        if not self._batched():
+            lists = self.get_top_n(top, uids=[ts.to_raw_uid(u) for u in iu[known].tolist()])
+            return [accuracy.top_n_measures({u: l_u[:n] for u, l_u in lists.items()}, fold.testset, n, threshold,
+                                            ts.offset, verbose=False) for n in ns]
+        from .. import _native as nat
+        width = min(top, ts.n_items)
+        inv, disc, idcg = accuracy._rank_tables(min(top, max(width, int(n_rel.max()))))
+        d_inv, d_disc = nat.to_dev(inv, np.float64), nat.to_dev(disc, np.float64)
+        d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
+        n_k = int(known.sum())
+        outs = [tuple(nat.empty_dev((max(n_k, 1),), t) for t in (np.int32, np.float64, np.float64)) for _ in ns]
+        lib, stream = nat.lib(), nat.stream()
+
+        def count_hits(b0, nr, items, count):
+            for n, (hits, rr, dcg) in zip(ns, outs):
+                nat.check(lib.sb2_top_n_hits_dev(nr, nat.ptr(items[b0:]), width, nat.ptr(count[b0:]), min(n, width),
+                                                 nat.ptr(d_ptr[b0:]), nat.ptr(d_idx), len(rel_idx), nat.ptr(d_inv),
+                                                 nat.ptr(d_disc), nat.ptr(hits[b0:]), nat.ptr(rr[b0:]),
+                                                 nat.ptr(dcg[b0:]), stream))
+
+        if n_k:
+            self._top_n_dev(width, iu[known], _block_rows, on_block=count_hits)
+        res = []
+        for n, out in zip(ns, outs):
+            hits, rr, dcg = np.zeros(len(iu), dtype=np.int64), np.zeros(len(iu)), np.zeros(len(iu))
+            for host, dev in zip((hits, rr, dcg), out):
+                host[known] = dev.cpu().numpy()[:n_k]
+            res.append(accuracy._top_n_of_counts(hits, rr, dcg, n_rel, n, idcg, False))
+        return res
 
     def _top_n_scorer(self):
         """Device arrays for sb2_mf_score_block_dev (dict: f, biased, pu, qi, bu, bi[, yj, up, ui]), or None when
