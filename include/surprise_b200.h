@@ -293,6 +293,13 @@ int sb2_knn_predict(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t
                     const double* sim, const int64_t* y_ptr, const int32_t* x_idx, const double* r, int k,
                     int min_k, int mode, double global_mean, const double* bx, const double* by, double* est,
                     int32_t* actual_k, uint8_t* impossible);
+/* The same estimates from a block of similarity rows: pair k reads sim[x[k], .] at sim + sim_row[k] * sim_ld
+ * (for known pairs).  bx, by, the neighbour ids and every other array stay indexed by the global x / y.
+ * sb2_knn_predict_dev is this call with sim_row = x. */
+int sb2_knn_predict_rows_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t n_x, const double* sim,
+                             int64_t sim_ld, const int32_t* sim_row, const int64_t* y_ptr, const int32_t* x_idx,
+                             const double* r, int k, int min_k, int mode, double global_mean, const double* bx,
+                             const double* by, double* est, int32_t* actual_k, uint8_t* impossible, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * SlopeOne ("next" row 4 of the hot-path table).  sb2_slope_one_fit replaces the two loops of
@@ -441,6 +448,22 @@ int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y
  * sb2_sim_build applies); *denom_out (HOST int) = 0 when the ratings lie on none of these grids.
  * ------------------------------------------------------------------------------------------------ */
 int sb2_rating_denominator_dev(const double* r, int64_t nnz, int* denom_out, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Listed rows of the similarity matrix, for k-NN models whose n_x x n_x matrix is not kept: out[b * ld + j] =
+ * sim[rows[b]][j] for b < n_rows and every j < n_x, bit for bit the same rows of sb2_sim_build_dev(0, n_x) --
+ * entries left of the diagonal included, evaluated as the pair (min, max) the way the reference mirrors them
+ * (similarities.pyx:95).  Same arguments and statuses as sb2_sim_build_dev (SB2_ERR_ZERO_DIVISION for msd, duplicated
+ * pairs on the general path); rows (DEVICE int32) may come in any order and repeat; a row outside [0, n_x) is
+ * SB2_ERR_INVALID; ld >= n_x.  The tensor path packs the A side from the listed rows and contracts them against all
+ * n_x rows (2 G n_rows n_x n_y operations, no symmetry); the general path runs the listed rows' co-ratings.  The path
+ * is chosen by the cost model for n_rows where both paths give the same bits (cosine / msd / pearson on a power-of-two
+ * rating grid), otherwise as the full build chooses it.  Synchronises `stream`.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_sim_build_rows_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,
+                           const double* r, int64_t nnz, int rating_denom, int min_support, double global_mean,
+                           const double* x_biases, const double* y_biases, double shrinkage, const int32_t* rows,
+                           int64_t n_rows, double* out, int64_t ld, void* stream);
 
 #ifdef __cplusplus
 }

@@ -90,9 +90,13 @@ SIGNATURES = {
                                    _vp, _vp, _vp, _vp]),
     "sb2_knn_predict": (_int, [_i64, _vp, _vp, _i64, _i64, _vp, _vp, _vp, _vp, _int, _int, _int, _dbl, _vp, _vp, _vp,
                                _vp, _vp]),
+    "sb2_knn_predict_rows_dev": (_int, [_i64, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _int, _int, _int, _dbl,
+                                        _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb2_slope_one_fit_dev": (_int, [_i64, _i64, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "sb2_slope_one_fit": (_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "sb2_rating_denominator_dev": (_int, [_vp, _i64, _vp, _vp]),
+    "sb2_sim_build_rows_dev": (_int, [_int, _i64, _i64, _vp, _vp, _vp, _i64, _int, _int, _dbl, _vp, _vp, _dbl, _vp,
+                                      _i64, _vp, _i64, _vp]),
     "sb2_get_neighbors_dev": (_int, [_i64, _vp, _i64, _i64, _vp, _int, _vp, _vp]),
     "sb2_slope_one_predict_dev": (_int, [_i64, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb2_coclustering_fit_dev": (_int, [_i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _dbl, _int, _int,

@@ -44,6 +44,10 @@ int sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr
                         int64_t nnz, int rating_denom, int min_support, double global_mean, const double* x_biases,
                         const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end, double* sim_out,
                         cudaStream_t st);
+int sim_build_rows_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
+                       int64_t nnz, int rating_denom, int min_support, double global_mean, const double* x_biases,
+                       const double* y_biases, double shrinkage, const int32_t* rows, int64_t n_rows, double* out,
+                       int64_t ld, cudaStream_t st);
 int rating_denominator_dev(const double* r, int64_t nnz, int* denom_out, cudaStream_t st);
 int baseline_als_dev(int64_t n_users, int64_t n_items, const int64_t* u_ptr, const int32_t* ui_idx, const double* u_r,
                      const int64_t* i_ptr, const int32_t* iu_idx, const double* i_r, double mu, int n_epochs,
@@ -65,9 +69,9 @@ int mf_predict_dev(int64_t n_pairs, const int32_t* u, const int32_t* i, int f, i
                    const double* qi, const double* bu, const double* bi, const double* yj, const int64_t* u_ptr,
                    const int32_t* ui_idx, double* est, uint8_t* impossible, cudaStream_t st);
 int knn_predict_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t n_x, const double* sim,
-                    int64_t sim_ld, const int64_t* y_ptr, const int32_t* x_idx, const double* r, int k, int min_k,
-                    int mode, double mu, const double* bx, const double* by, double* est, int32_t* actual_k,
-                    uint8_t* impossible, cudaStream_t st);
+                    int64_t sim_ld, const int32_t* sim_row, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
+                    int k, int min_k, int mode, double mu, const double* bx, const double* by, double* est,
+                    int32_t* actual_k, uint8_t* impossible, cudaStream_t st);
 int get_neighbors_dev(int64_t n_x, const double* sim, int64_t sim_ld, int64_t n_rows, const int32_t* rows, int k,
                       int32_t* out, cudaStream_t st);
 int slope_one_fit_dev(int64_t n_items, int64_t n_users, const int64_t* u_ptr, const int32_t* i_idx, const double* r,
@@ -651,8 +655,21 @@ int sb2_knn_predict_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int
                         int mode, double global_mean, const double* bx, const double* by, double* est,
                         int32_t* actual_k, uint8_t* impossible, void* stream) {
     SB2_TRY(ensure_device());
-    return knn_predict_dev(n_pairs, x, y, n_x, sim, sim_ld, y_ptr, x_idx, r, k, min_k, mode, global_mean, bx, by, est,
+    return knn_predict_dev(n_pairs, x, y, n_x, sim, sim_ld, x, y_ptr, x_idx, r, k, min_k, mode, global_mean, bx, by, est,
                            actual_k, impossible, (cudaStream_t)stream);
+}
+
+int sb2_knn_predict_rows_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t n_x, const double* sim,
+                             int64_t sim_ld, const int32_t* sim_row, const int64_t* y_ptr, const int32_t* x_idx,
+                             const double* r, int k, int min_k, int mode, double global_mean, const double* bx,
+                             const double* by, double* est, int32_t* actual_k, uint8_t* impossible, void* stream) {
+    SB2_TRY(ensure_device());
+    if (n_pairs > 0 && !sim_row) {
+        set_error("knn_predict_rows: null sim_row");
+        return SB2_ERR_INVALID;
+    }
+    return knn_predict_dev(n_pairs, x, y, n_x, sim, sim_ld, sim_row, y_ptr, x_idx, r, k, min_k, mode, global_mean, bx,
+                           by, est, actual_k, impossible, (cudaStream_t)stream);
 }
 
 int sb2_knn_predict(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t n_x, int64_t n_y, const double* sim,
@@ -681,7 +698,7 @@ int sb2_knn_predict(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t
     SB2_TRY(d_ak.alloc((size_t)std::max<int64_t>(n_pairs, 1) * 4, st));
     SB2_TRY(d_imp.alloc((size_t)std::max<int64_t>(n_pairs, 1), st));
     SB2_TRY(knn_predict_dev(n_pairs, d_x.as<int32_t>(), d_y.as<int32_t>(), n_x, d_sim.as<double>(), n_x,
-                            d_ptr.as<int64_t>(), d_idx.as<int32_t>(), d_r.as<double>(), k, min_k, mode, global_mean,
+                            d_x.as<int32_t>(), d_ptr.as<int64_t>(), d_idx.as<int32_t>(), d_r.as<double>(), k, min_k, mode, global_mean,
                             mode ? d_bx.as<double>() : nullptr, (mode && by) ? d_by.as<double>() : nullptr, d_est.as<double>(),
                             d_ak.as<int32_t>(), d_imp.as<uint8_t>(), st));
     SB2_TRY(download(est, d_est.p, (size_t)n_pairs, st));
@@ -837,6 +854,15 @@ int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y
     SB2_TRY(ensure_device());
     return sim_build_upper_dev(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases,
                                y_biases, shrinkage, row_begin, row_end, sim_out, (cudaStream_t)stream);
+}
+
+int sb2_sim_build_rows_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,
+                           const double* r, int64_t nnz, int rating_denom, int min_support, double global_mean,
+                           const double* x_biases, const double* y_biases, double shrinkage, const int32_t* rows,
+                           int64_t n_rows, double* out, int64_t ld, void* stream) {
+    SB2_TRY(ensure_device());
+    return sim_build_rows_dev(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases,
+                              y_biases, shrinkage, rows, n_rows, out, ld, (cudaStream_t)stream);
 }
 
 int sb2_rating_denominator_dev(const double* r, int64_t nnz, int* denom_out, void* stream) {

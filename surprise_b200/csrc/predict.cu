@@ -443,7 +443,8 @@ __device__ __noinline__ KnnSums knn_select_long(const double* __restrict__ srow,
 #endif
 __global__ void __launch_bounds__(KNN_WARPS * 32, SB2_KNN_MIN_BLOCKS)
 knn_predict_kernel(int64_t n_pairs, const int32_t* __restrict__ x, const int32_t* __restrict__ y, int64_t n_x,
-                   const double* __restrict__ sim, int64_t sim_ld, const int64_t* __restrict__ y_ptr,
+                   const double* __restrict__ sim, int64_t sim_ld, const int32_t* __restrict__ sim_row,
+                   const int64_t* __restrict__ y_ptr,
                    const int32_t* __restrict__ x_idx, const double* __restrict__ r, int k, int min_k, int mode,
                    double mu, const double* __restrict__ bx, const double* __restrict__ by, double* __restrict__ est,
                    int32_t* __restrict__ actual_k, uint8_t* __restrict__ impossible) {
@@ -473,7 +474,7 @@ knn_predict_kernel(int64_t n_pairs, const int32_t* __restrict__ x, const int32_t
         } else {
             if (mode >= 3) e = bx[xx];  // means[x] (knns.py:187, :382)
             const int64_t b = y_ptr[yy], len = y_ptr[yy + 1] - b;
-            const double* srow = sim + (size_t)xx * (size_t)sim_ld;
+            const double* srow = sim + (size_t)sim_row[p] * (size_t)sim_ld;  // row x of the matrix
             const int32_t* idx = x_idx + b;
             // per-neighbour term of the weighted sum (knns.py:113 / :195 / :296-297 / :389)
             auto term_of = [&](double bs, int pos) -> double {
@@ -514,10 +515,11 @@ knn_predict_kernel(int64_t n_pairs, const int32_t* __restrict__ x, const int32_t
     }
 }
 
+// pair p reads its similarities from sim + sim_row[p] * sim_ld (sim_row = x for the whole matrix)
 int knn_predict_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t n_x, const double* sim,
-                    int64_t sim_ld, const int64_t* y_ptr, const int32_t* x_idx, const double* r, int k, int min_k,
-                    int mode, double mu, const double* bx, const double* by, double* est, int32_t* actual_k,
-                    uint8_t* impossible, cudaStream_t st) {
+                    int64_t sim_ld, const int32_t* sim_row, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
+                    int k, int min_k, int mode, double mu, const double* bx, const double* by, double* est,
+                    int32_t* actual_k, uint8_t* impossible, cudaStream_t st) {
     if (n_pairs <= 0) return SB2_OK;
     if (mode < 0 || mode > 4 || (mode != 0 && !bx) || ((mode == 1 || mode == 2 || mode == 4) && !by)) {
         set_error("knn_predict: invalid mode / missing baselines");
@@ -526,8 +528,9 @@ int knn_predict_dev(int64_t n_pairs, const int32_t* x, const int32_t* y, int64_t
     int64_t blocks = ceil_div(n_pairs, KNN_WARPS);
     const int64_t cap = (int64_t)sm_count() * 8;
     if (blocks > cap) blocks = cap;
-    knn_predict_kernel<<<(unsigned)blocks, KNN_WARPS * 32, 0, st>>>(n_pairs, x, y, n_x, sim, sim_ld, y_ptr, x_idx, r, k,
-                                                                    min_k, mode, mu, bx, by, est, actual_k, impossible);
+    knn_predict_kernel<<<(unsigned)blocks, KNN_WARPS * 32, 0, st>>>(n_pairs, x, y, n_x, sim, sim_ld, sim_row, y_ptr, x_idx,
+                                                                    r, k, min_k, mode, mu, bx, by, est, actual_k,
+                                                                    impossible);
     SB2_LAUNCH_CHECK();
     return SB2_OK;
 }

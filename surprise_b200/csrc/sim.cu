@@ -23,7 +23,7 @@
 namespace sb2 {
 
 // status words written by the kernels (device int[8])
-enum { ST_BAD_RATING = 0, ST_MAX_Q = 1, ST_DUP = 2, ST_ZERODIV = 3, ST_NWORDS = 8 };
+enum { ST_BAD_RATING = 0, ST_MAX_Q = 1, ST_DUP = 2, ST_ZERODIV = 3, ST_BAD_ROW = 4, ST_NWORDS = 8 };
 
 __device__ __forceinline__ int64_t find_segment(const int64_t* __restrict__ ptr, int64_t n_seg, int64_t a) {
     int64_t lo = 0, hi = n_seg;  // largest s with ptr[s] <= a
@@ -143,7 +143,9 @@ struct FinArgs {
     double inv_d, inv_d2;  // 1/denom, 1/denom^2
     int min_support;
     double shrinkage;
-    double* sim;  // (row_end-row_begin) x n_x
+    double* sim;  // (row_end-row_begin) x n_x; rows kernel: output row b at sim + (b - row_begin) * out_ld
+    int64_t out_ld;
+    const int32_t* rows;  // row list of sb2_sim_build_rows_dev: output (and plane) row b is matrix row rows[b]
     int* status;
 };
 
@@ -226,15 +228,37 @@ __global__ void sim_finalize_sym_kernel(const FinArgs f) {
     }
 }
 
-// row-shard build: every (i, j) of the shard rows, accumulators valid at (i, j) itself
+// row-shard or row-list build: every (i, j) of the output rows, accumulators valid at (i, j) itself.  sim_value reads
+// the accumulators of (i, j) with the roles swapped below the diagonal, which gives the bits the symmetric build
+// mirrors from (j, i): every plane holds exact integer sums (or, for pearson_baseline, the same digit products in the
+// same order on either side).
 __global__ void sim_finalize_rows_kernel(const FinArgs f) {
     const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    const int64_t i = f.band_begin + blockIdx.y;
-    if (j >= f.n_x || i >= f.band_end) return;
+    const int64_t b = f.band_begin + blockIdx.y;
+    if (j >= f.n_x || b >= f.band_end) return;
+    const int64_t i = f.rows ? f.rows[b] : b;
     double s;
     if (i == j) s = 1.0;
-    else s = sim_value(f, (size_t)(i - f.plane_row0) * f.ld + j, i, j, i > j);
-    f.sim[(size_t)(i - f.row_begin) * f.n_x + j] = s;
+    else s = sim_value(f, (size_t)(b - f.plane_row0) * f.ld + j, i, j, i > j);
+    f.sim[(size_t)(b - f.row_begin) * f.out_ld + j] = s;
+}
+
+// A-side panels of a row-list build: slot b of every panel is a copy of panel row rows[b]
+__global__ void sim_gather_rows_kernel(const uint8_t* __restrict__ src, size_t src_panel_bytes, uint8_t* __restrict__ dst,
+                                       size_t dst_panel_bytes, int n_panels, const int32_t* __restrict__ rows,
+                                       int64_t n_rows, int64_t k_pad) {
+    const int64_t per_row = k_pad / 16, per_panel = n_rows * per_row;
+    for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < per_panel * n_panels;
+         t += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t q = t / per_panel, rem = t - q * per_panel, b = rem / per_row, c = rem - b * per_row;
+        const uint4* s = reinterpret_cast<const uint4*>(src + q * src_panel_bytes + (size_t)rows[b] * k_pad);
+        reinterpret_cast<uint4*>(dst + q * dst_panel_bytes + (size_t)b * k_pad)[c] = s[c];
+    }
+}
+
+__global__ void sim_check_rows_kernel(const int32_t* __restrict__ rows, int64_t n_rows, int64_t n_x, int* status) {
+    const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (b < n_rows && (rows[b] < 0 || rows[b] >= n_x)) atomicExch(&status[ST_BAD_ROW], 1);
 }
 
 // SlopeOne (slope_one.pyx:59-70): freq[i][j] = |U_ij| (int64, symmetric, diagonal = raters of i);
@@ -282,13 +306,18 @@ static int n_digits(unsigned long long v) {
 
 constexpr int KIND_SLOPE_ONE = 4;  // internal: freq + dev of SlopeOne from the FREQ / SI / SJ planes
 
+// rows == nullptr: the matrix rows [row_begin, row_end).  Otherwise a row-list build: row_begin = 0, output row b
+// (b < row_end) is matrix row rows[b] (checked to lie in [0, n_x)), written at sim_out + b * out_ld.  Its A-side panels
+// hold the listed rows only (gathered from the full panels, which stay the B side), and the row blocks of the GEMM and
+// the finalize walk the list's slots: 2 G n_rows n_x n_y operations, no symmetry.
 static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
                     int64_t nnz, int rating_denom, int min_support, double global_mean, const double* x_biases,
-                    const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end, double* sim_out,
-                    int64_t* freq_out, bool upper, cudaStream_t st) {
+                    const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end,
+                    const int32_t* rows, double* sim_out, int64_t out_ld, int64_t* freq_out, bool upper,
+                    cudaStream_t st) {
     const bool slope = (kind == KIND_SLOPE_ONE);
     if (kind < 0 || kind > 4 || n_x <= 0 || n_y < 0 || nnz < 0 || rating_denom <= 0 || row_begin < 0 ||
-        row_end > n_x || row_begin >= row_end) {
+        (!rows && row_end > n_x) || (rows && (row_begin != 0 || upper || slope)) || row_begin >= row_end) {
         set_error("sim_build: invalid argument");
         return SB2_ERR_INVALID;
     }
@@ -298,7 +327,7 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
         return SB2_ERR_INVALID;
     }
     if (pb && min_support < 2) min_support = 2;  // similarities.pyx:334
-    const bool full = (row_begin == 0 && row_end == n_x);
+    const bool full = (!rows && row_begin == 0 && row_end == n_x);
     const int TR = gemm_tile_rows();  // 256 (CTA-pair kernel) or 128
     if (!full && row_begin % TR) {
         set_error("sim_build: row_begin of a shard must be a multiple of %d", TR);
@@ -306,7 +335,7 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
     }
     const int64_t n_pad = round_up(n_x, TR);
     const int64_t k_pad = round_up(std::max<int64_t>(n_y, 1), GEMM_BK);  // 128
-    const int64_t rows_pad = round_up(row_end, TR) - row_begin;  // plane rows (shard)
+    const int64_t rows_pad = round_up(row_end, TR) - row_begin;  // plane rows (shard, or slots of a row list)
     const int64_t ld = n_pad;
 
     // ---- pass 1: analyse ratings --------------------------------------------------------------
@@ -399,6 +428,16 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
     pa.status = status_d.as<int>();
     if (nnz > 0) {
         sim_pack_kernel<<<(unsigned)ceil_div(nnz, 256), 256, 0, st>>>(pa);
+        SB2_LAUNCH_CHECK();
+    }
+    DevBuf a_panels_d;
+    const size_t a_panel_bytes = (size_t)rows_pad * (size_t)k_pad;
+    if (rows) {
+        SB2_TRY(a_panels_d.alloc(a_panel_bytes * n_panels, st));
+        SB2_CUDA(cudaMemsetAsync(a_panels_d.p, 0, a_panel_bytes * n_panels, st));
+        const int64_t n16 = row_end * (k_pad / 16) * n_panels;
+        sim_gather_rows_kernel<<<(unsigned)std::min<int64_t>(ceil_div(n16, 256), 65536), 256, 0, st>>>(
+            base, panel_bytes, a_panels_d.as<uint8_t>(), a_panel_bytes, n_panels, rows, row_end, k_pad);
         SB2_LAUNCH_CHECK();
     }
 
@@ -499,6 +538,9 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
         }
         jobs.swap(ordered);
     }
+    if (rows)  // the A side of every job reads the same panel's gathered rows
+        for (GemmJob& jb : jobs)
+            jb.a = a_panels_d.as<uint8_t>() + (size_t)(jb.a - base) / panel_bytes * a_panel_bytes;
     const bool timing = getenv("SB2_SIM_TIMING") != nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     if (timing) {
@@ -538,19 +580,25 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
     f.inv_d = 1.0 / (double)rating_denom;
     f.inv_d2 = 1.0 / ((double)rating_denom * (double)rating_denom);
     f.min_support = min_support; f.shrinkage = shrinkage; f.sim = sim_out; f.status = status_d.as<int>();
+    f.out_ld = rows ? out_ld : n_x; f.rows = rows;
     const unsigned nt = (unsigned)ceil_div(n_x, 32);
     for (size_t bi = 0; bi + 1 < band_off.size(); ++bi) {
         const int64_t band_begin = ((int64_t)rb0 + (int64_t)bi * band_rb) * TR;
         const int64_t band_end = std::min<int64_t>(row_end, band_begin + (int64_t)band_rb * TR);
         const size_t t0 = band_off[bi], nt_band = band_off[bi + 1] - t0;
         if (nt_band)
-            SB2_TRY(gemm_u8_tc_run(jobs.data(), (int)jobs.size(), n_pad, k_pad, tiles_d.as<int2>() + t0, (int)nt_band, ld,
-                                   band_begin, st));
+            SB2_TRY(gemm_u8_tc_run2(jobs.data(), (int)jobs.size(), rows ? rows_pad : n_pad, n_pad, k_pad,
+                                    tiles_d.as<int2>() + t0, (int)nt_band, ld, band_begin, st));
         f.band_begin = band_begin; f.band_end = band_end; f.plane_row0 = band_begin;
         const unsigned rows32 = (unsigned)ceil_div(band_end - band_begin, 32);
         if (slope) slope_finalize_kernel<<<dim3(nt, rows32), dim3(32, 8), 0, st>>>(f, freq_out, sim_out);
         else if (full || upper) sim_finalize_sym_kernel<<<dim3(nt, rows32), dim3(32, 8), 0, st>>>(f);
-        else sim_finalize_rows_kernel<<<dim3((unsigned)ceil_div(n_x, 256), (unsigned)(band_end - band_begin)), 256, 0, st>>>(f);
+        else
+            for (int64_t c0 = band_begin; c0 < band_end; c0 += 65535) {  // gridDim.y <= 65535
+                f.band_begin = c0;
+                f.band_end = std::min<int64_t>(band_end, c0 + 65535);
+                sim_finalize_rows_kernel<<<dim3((unsigned)ceil_div(n_x, 256), (unsigned)(f.band_end - c0)), 256, 0, st>>>(f);
+            }
         SB2_LAUNCH_CHECK();
     }
     if (timing) {
@@ -585,7 +633,8 @@ static int sim_core(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
 
 int sim_general_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
                     int64_t nnz, int min_support, double global_mean, const double* x_biases, const double* y_biases,
-                    double shrinkage, int64_t row_begin, int64_t row_end, bool upper, double* sim_out, cudaStream_t st);
+                    double shrinkage, int64_t row_begin, int64_t row_end, const int32_t* rows, bool upper,
+                    double* sim_out, int64_t out_ld, cudaStream_t st);
 
 __global__ void sim_visits_kernel(int64_t n_y, const int64_t* __restrict__ y_ptr, double* __restrict__ out) {
     const int64_t y = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -609,13 +658,32 @@ __global__ void sim_visits_kernel(int64_t n_y, const int64_t* __restrict__ y_ptr
 // general path: everything the reference accepts is computed, nothing is rejected.  Otherwise the cheaper one by the
 // cost model below runs; pearson_baseline prefers the general path unless the digit path is clearly (1.5x) faster,
 // because only the general path reproduces the reference's bits there.  SB2_SIM_PATH=digit|general overrides.
+// A row-list build (rows != nullptr, slots [0, row_end)) is costed for its own rows, without symmetry, where both paths
+// give the same bits (cosine / msd / pearson on a power-of-two grid: every sum is exact on both).  Elsewhere
+// (pearson_baseline, grids like 1/10) it takes the path the full build takes, so that its rows are the full build's
+// rows bit for bit.
 static int sim_dispatch(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
                         int64_t nnz, int rating_denom, int min_support, double global_mean, const double* x_biases,
-                        const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end, double* sim_out,
-                        bool upper, cudaStream_t st) {
-    if (kind < 0 || kind > 3 || n_x <= 0 || n_y < 0 || row_begin < 0 || row_end > n_x || row_begin >= row_end) {
+                        const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end,
+                        const int32_t* row_list, double* sim_out, int64_t out_ld, bool upper, cudaStream_t st) {
+    if (kind < 0 || kind > 3 || n_x <= 0 || n_y < 0 || row_begin < 0 || (!row_list && row_end > n_x) ||
+        (row_list && (row_begin != 0 || upper)) || row_begin >= row_end) {
         set_error("sim_build: invalid argument");
         return SB2_ERR_INVALID;
+    }
+    if (row_list) {
+        DevBuf bad_d;
+        SB2_TRY(bad_d.alloc(ST_NWORDS * sizeof(int), st));
+        SB2_CUDA(cudaMemsetAsync(bad_d.p, 0, ST_NWORDS * sizeof(int), st));
+        sim_check_rows_kernel<<<(unsigned)ceil_div(row_end, 256), 256, 0, st>>>(row_list, row_end, n_x, bad_d.as<int>());
+        SB2_LAUNCH_CHECK();
+        int bad[ST_NWORDS];
+        SB2_CUDA(cudaMemcpyAsync(bad, bad_d.p, sizeof(bad), cudaMemcpyDeviceToHost, st));
+        SB2_CUDA(cudaStreamSynchronize(st));
+        if (bad[ST_BAD_ROW]) {
+            set_error("sim_build_rows: row id out of range for n_x=%lld", (long long)n_x);
+            return SB2_ERR_INVALID;
+        }
     }
     bool use_digit = rating_denom > 0;
     const char* force = getenv("SB2_SIM_PATH");
@@ -629,14 +697,16 @@ static int sim_dispatch(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr
         double visits = 0.0;
         SB2_CUDA(cudaMemcpyAsync(&visits, v_d.p, sizeof(double), cudaMemcpyDeviceToHost, st));
         SB2_CUDA(cudaStreamSynchronize(st));
-        const double rows = (double)(row_end - row_begin), frac = rows / (double)n_x;
+        const bool same_bits = kind != SB2_SIM_PEARSON_BASELINE && (rating_denom & (rating_denom - 1)) == 0;
+        const bool as_full = row_list && !same_bits;
+        const double rows = (double)(as_full ? n_x : row_end - row_begin), frac = rows / (double)n_x;
         // general: co-ratings of the shard's rows + zeroing / reading the 32-byte column records of every row
         const double keep = upper ? 1.0 - ((double)row_begin + 0.5 * rows) / (double)n_x : 1.0;  // columns >= row_begin
         const double t_general = frac * keep * visits / 2.0e10 + rows * (double)n_x * 64.0 / 3.0e12 + 2e-4;
         // digit: accumulators x tiles x k at the measured 3.6 POP/s issued, + packing the dense panels
         const int n_acc = kind == SB2_SIM_PEARSON_BASELINE ? 30 : kind == SB2_SIM_PEARSON ? 6 : 4;
         const double n_pad = (double)round_up(n_x, 256), k_pad = (double)round_up(std::max<int64_t>(n_y, 1), 128);
-        const bool tri = (row_begin == 0 && row_end == n_x) || upper;
+        const bool tri = as_full || (!row_list && row_begin == 0 && row_end == n_x) || upper;
         const double cols = tri ? (n_pad - (double)row_begin - 0.5 * rows) : n_pad;
         const double t_digit = 2.0 * n_acc * rows * cols * k_pad / 3.6e15 + (n_acc / 2 + 3) * n_pad * k_pad / 4.0e12 + 3e-4;
         const double bias = kind == SB2_SIM_PEARSON_BASELINE ? 1.5 : 1.0;
@@ -645,10 +715,10 @@ static int sim_dispatch(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr
     int rc = SB2_ERR_DUPLICATE;
     if (use_digit)
         rc = sim_core(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases, y_biases,
-                      shrinkage, row_begin, row_end, sim_out, nullptr, upper, st);
+                      shrinkage, row_begin, row_end, row_list, sim_out, out_ld, nullptr, upper, st);
     if (rc != SB2_ERR_DUPLICATE) return rc;
     return sim_general_dev(kind, n_x, n_y, y_ptr, x_idx, r, nnz, min_support, global_mean, x_biases, y_biases, shrinkage,
-                           row_begin, row_end, upper, sim_out, st);
+                           row_begin, row_end, row_list, upper, sim_out, out_ld, st);
 }
 
 int sim_build_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
@@ -656,7 +726,22 @@ int sim_build_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, cons
                   const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end, double* sim_out,
                   cudaStream_t st) {
     return sim_dispatch(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases, y_biases,
-                        shrinkage, row_begin, row_end, sim_out, false, st);
+                        shrinkage, row_begin, row_end, nullptr, sim_out, n_x, false, st);
+}
+
+// rows[0 .. n_rows) of the matrix, in the given order (repeats allowed): out[b * ld + j] = sim[rows[b]][j], the bits of
+// the same rows of the full build
+int sim_build_rows_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
+                       int64_t nnz, int rating_denom, int min_support, double global_mean, const double* x_biases,
+                       const double* y_biases, double shrinkage, const int32_t* rows, int64_t n_rows, double* out,
+                       int64_t ld, cudaStream_t st) {
+    if (n_rows == 0) return SB2_OK;
+    if (!rows || !out || n_rows < 0 || ld < n_x) {
+        set_error("sim_build_rows: invalid argument");
+        return SB2_ERR_INVALID;
+    }
+    return sim_dispatch(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases, y_biases,
+                        shrinkage, 0, n_rows, rows, out, ld, false, st);
 }
 
 // row shard of a symmetric multi-rank build: only sim[i][j] with j >= row_begin is computed (tiles at or above the
@@ -667,7 +752,7 @@ int sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr
                         const double* y_biases, double shrinkage, int64_t row_begin, int64_t row_end, double* sim_out,
                         cudaStream_t st) {
     return sim_dispatch(kind, n_x, n_y, y_ptr, x_idx, r, nnz, rating_denom, min_support, global_mean, x_biases, y_biases,
-                        shrinkage, row_begin, row_end, sim_out, true, st);
+                        shrinkage, row_begin, row_end, nullptr, sim_out, n_x, true, st);
 }
 
 // SlopeOne.fit (slope_one.pyx:44-80): u_ptr / i_idx / r is the ur CSR (items rated by each user)
@@ -678,7 +763,7 @@ int slope_one_fit_dev(int64_t n_items, int64_t n_users, const int64_t* u_ptr, co
         return SB2_ERR_INVALID;
     }
     return sim_core(KIND_SLOPE_ONE, n_items, n_users, u_ptr, i_idx, r, nnz, 1, 0, 0.0, nullptr, nullptr, 0.0, 0, n_items,
-                    dev_out, freq_out, false, st);
+                    nullptr, dev_out, n_items, freq_out, false, st);
 }
 
 // Smallest supported denominator d such that every rating is an integer multiple of 1/d in [0, 65535/d]

@@ -395,11 +395,6 @@ int gemm_u8_tc_run2(const GemmJob* jobs, int n_jobs, int64_t a_rows, int64_t b_r
     return SB2_OK;
 }
 
-int gemm_u8_tc_run(const GemmJob* jobs, int n_jobs, int64_t n_pad_rows, int64_t k_pad, const int2* tiles_dev,
-                   int n_tiles, int64_t ld, int64_t plane_row0, cudaStream_t st) {
-    return gemm_u8_tc_run2(jobs, n_jobs, n_pad_rows, n_pad_rows, k_pad, tiles_dev, n_tiles, ld, plane_row0, st);
-}
-
 // ----------------------------------------------------------------------------------------------
 // test hooks
 // ----------------------------------------------------------------------------------------------

@@ -48,8 +48,9 @@ struct GemmJob {
 
 // Builds tensor maps, batches jobs (<= 2 accumulators, <= 4 operand tiles per stage per launch) and
 // launches the tcgen05 kernel once per batch over `tiles` (int2 {row_blk, col_blk}, device array).
-int gemm_u8_tc_run(const GemmJob* jobs, int n_jobs, int64_t n_pad_rows, int64_t k_pad, const int2* tiles_dev,
-                   int n_tiles, int64_t ld, int64_t plane_row0, cudaStream_t st);
+// A-side panels have a_rows rows, B-side panels b_rows.
+int gemm_u8_tc_run2(const GemmJob* jobs, int n_jobs, int64_t a_rows, int64_t b_rows, int64_t k_pad,
+                    const int2* tiles_dev, int n_tiles, int64_t ld, int64_t plane_row0, cudaStream_t st);
 
 // rows (= columns) of an output tile: 256, computed by a CTA pair
 int gemm_tile_rows();

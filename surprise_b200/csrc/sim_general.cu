@@ -13,7 +13,8 @@
 // of round-to-nearest products and sums (no FMA contraction), and the per-row finalize applies the reference's
 // formula with the reference's operation order: the result is bit-identical to the reference for any input, which
 // the tests check against the oracle (and, through it, against the compiled reference's goldens).
-// Rows are independent, so a row range [row_begin, row_end) is a shard of a multi-rank build as it stands.
+// Rows are independent, so a row range [row_begin, row_end) is a shard of a multi-rank build as it stands, and a list
+// of rows in any order (sb2_sim_build_rows_dev) is the same rows built by CTAs that look their row up.
 //
 // Cost: sum_y |yr[y]|^2 pair visits of ~6 L2-resident read-modify-writes each (accumulators: 44 B per column per
 // CTA), i.e. HBM/L2-latency work, not tensor work: ~10^2..10^3 x slower than the digit path per build and still
@@ -49,10 +50,12 @@ struct GenArgs {
     double mu, shrinkage;
     const double* bx;
     const double* by;
-    int64_t row_begin, row_end;
+    int64_t row_begin, n_rows;  // output row b is matrix row rows[b], or row_begin + b when rows is null
+    const int32_t* rows;
     int64_t col_begin;      // columns below it are neither accumulated nor written (shard of a symmetric build: the
                             // transposes of the blocks owned by the shards before this one, filled in by the exchange)
-    double* sim;            // (row_end - row_begin) x n_x
+    double* sim;            // n_rows x out_ld
+    int64_t out_ld;
     double* scratch;        // per CTA: one record per column, [prods | sqi | sqj | freq] (32 B: one sector per
                             // co-rating) or [prods | sqi | sqj | si | sj | freq] for pearson
     int64_t scratch_stride; // doubles per CTA
@@ -108,7 +111,8 @@ __global__ void __launch_bounds__(256) sim_rows_kernel(const GenArgs a) {
     constexpr int I_SQI = 1, I_SQJ = 2, I_SI = 3, I_SJ = 4, I_FQ = NREC - 1;  // [0] = prods (msd: sq_diff)
     int min_sprt = a.min_support;
     if (KIND == 3 && min_sprt < 2) min_sprt = 2;  // similarities.pyx:334
-    for (int64_t row = a.row_begin + blockIdx.x; row < a.row_end; row += gridDim.x) {
+    for (int64_t ob = blockIdx.x; ob < a.n_rows; ob += gridDim.x) {
+        const int64_t row = a.rows ? a.rows[ob] : a.row_begin + ob;
         for (int64_t x = tid; x < n_x * NREC; x += nthr) REC[x] = 0.0;   // freq is kept as a double (exact below 2^53)
         __syncthreads();
         const double bxi = KIND == 3 ? a.bx[row] : 0.0;
@@ -197,7 +201,7 @@ __global__ void __launch_bounds__(256) sim_rows_kernel(const GenArgs a) {
         // etc., same terms in the same order) evaluating [row, xj] with the roles swapped for xj < row gives the
         // same bits (with duplicated pairs too: the accumulation above keeps the reference's loop nesting for the
         // columns below the diagonal), so every row is finished by its own CTA.
-        double* out = a.sim + (size_t)(row - a.row_begin) * n_x;
+        double* out = a.sim + (size_t)ob * (size_t)a.out_ld;
         for (int64_t xj = a.col_begin + tid; xj < n_x; xj += nthr) {
             double s = 0.0;
             const double* R = REC + (size_t)xj * NREC;
@@ -291,7 +295,8 @@ __global__ void __launch_bounds__(256, 4) sim_rows_fast_kernel(const GenArgs a) 
     if (KIND == 3 && min_sprt < 2) min_sprt = 2;  // similarities.pyx:334
     double* REC = a.scratch + (size_t)blockIdx.x * a.scratch_stride;   // this CTA's row of column records
     const int c0 = (int)a.col_begin, c1 = (int)n_x;
-    for (int64_t row = a.row_begin + blockIdx.x; row < a.row_end; row += gridDim.x) {
+    for (int64_t ob = blockIdx.x; ob < a.n_rows; ob += gridDim.x) {
+        const int64_t row = a.rows ? a.rows[ob] : a.row_begin + ob;
         for (int64_t x = tid; x < (int64_t)(c1 - c0) * NREC / 2; x += nthr)
             reinterpret_cast<double2*>(REC)[x] = make_double2(0.0, 0.0);
         // ri / rj: ratings -- or, for pearson_baseline, the precomputed deviations
@@ -365,7 +370,7 @@ __global__ void __launch_bounds__(256, 4) sim_rows_fast_kernel(const GenArgs a) 
         __syncthreads();
         // finalize (similarities.pyx:86-95 / :155-164 / :240-256 / :347-359); see sim_rows_kernel for why every row
         // can evaluate both triangles itself
-        double* out = a.sim + (size_t)(row - a.row_begin) * n_x;
+        double* out = a.sim + (size_t)ob * (size_t)a.out_ld;
         for (int xj = c0 + tid; xj < c1; xj += nthr) {
             double s = 0.0;
             const double* R = REC + (size_t)(xj - c0) * NREC;
@@ -401,11 +406,14 @@ __global__ void __launch_bounds__(256, 4) sim_rows_fast_kernel(const GenArgs a) 
     }
 }
 
+// rows == nullptr: output rows are the matrix rows [row_begin, row_end).  Otherwise row_begin = 0 and output row b is
+// matrix row rows[b] (b < row_end, the rows already checked to lie in [0, n_x)).  Output row b starts at sim_out + b * out_ld.
 int sim_general_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx, const double* r,
                     int64_t nnz, int min_support, double global_mean, const double* x_biases, const double* y_biases,
-                    double shrinkage, int64_t row_begin, int64_t row_end, bool upper, double* sim_out, cudaStream_t st) {
-    if (kind < 0 || kind > 3 || n_x <= 0 || n_y < 0 || nnz < 0 || nnz > 0x7FFFFFF0ll || row_begin < 0 || row_end > n_x ||
-        row_begin >= row_end) {
+                    double shrinkage, int64_t row_begin, int64_t row_end, const int32_t* rows, bool upper,
+                    double* sim_out, int64_t out_ld, cudaStream_t st) {
+    if (kind < 0 || kind > 3 || n_x <= 0 || n_y < 0 || nnz < 0 || nnz > 0x7FFFFFF0ll || row_begin < 0 ||
+        (!rows && row_end > n_x) || (rows && (row_begin != 0 || upper)) || row_begin >= row_end || out_ld < n_x) {
         set_error("sim_build (general path): invalid argument");
         return SB2_ERR_INVALID;
     }
@@ -460,10 +468,10 @@ int sim_general_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
         set_error("sim_build: more than 255 copies of one (x, y) pair");
         return SB2_ERR_UNSUPPORTED;
     }
-    const int64_t rows = row_end - row_begin;
+    const int64_t rows_n = row_end - row_begin;
     int per_sm = 4;
     if (const char* e = getenv("SB2_SIM_GENERAL_CTAS")) per_sm = std::max(1, std::min(8, atoi(e)));
-    const int grid = (int)std::min<int64_t>(rows, (int64_t)sm_count() * per_sm);
+    const int grid = (int)std::min<int64_t>(rows_n, (int64_t)sm_count() * per_sm);
     const int64_t stride = (6 * n_x + 7) & ~(int64_t)3;  // records of 4 doubles (6 for pearson) per column, 32 B aligned
     SB2_TRY(scratch_d.alloc((size_t)grid * (size_t)stride * sizeof(double), st));
     GenArgs a;
@@ -471,7 +479,8 @@ int sim_general_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, co
     a.n_x = n_x; a.n_y = n_y; a.nnz = nnz; a.y_ptr = y_ptr; a.x_idx = x_idx; a.r = r;
     a.x_ptr = xptr_d.as<int64_t>(); a.x_ent = ent2_d.as<int>(); a.y_of = y_of_d.as<int>(); a.occ = occ_d.as<uint8_t>();
     a.max_occ = status_h[G_ST_MAXOCC]; a.min_support = min_support; a.mu = global_mean; a.shrinkage = shrinkage;
-    a.bx = x_biases; a.by = y_biases; a.row_begin = row_begin; a.row_end = row_end; a.sim = sim_out;
+    a.bx = x_biases; a.by = y_biases; a.row_begin = row_begin; a.n_rows = rows_n; a.rows = rows; a.sim = sim_out;
+    a.out_ld = out_ld;
     a.col_begin = upper ? row_begin : 0;
     a.scratch = scratch_d.as<double>(); a.scratch_stride = stride; a.status = status_d.as<int>();
     DevBuf xmb_d, xml_d, xmr_d, xmp_d;

@@ -98,6 +98,24 @@ def build_device(kind, n_x, yr, min_support, global_mean=0.0, x_biases=None, y_b
     return out
 
 
+def build_rows_device(kind, inputs, rows, out, min_support, global_mean=0.0, shrinkage=100):
+    """Rows ``rows`` (CUDA int32 tensor, any order, repeats allowed) of the similarity matrix of ``inputs`` (the
+    result of upload_inputs()) into the first len(rows) rows of ``out`` (CUDA float64, n_x columns, contiguous): the
+    bits of the same rows of build_device()."""
+    n_x = inputs["n_x"]
+    rows = nat.to_dev(rows, np.int32)
+    if (str(out.dtype) != "torch.float64" or out.dim() != 2 or out.shape[1] != n_x or out.shape[0] < len(rows)
+            or not out.is_contiguous()):
+        raise ValueError("out must be a contiguous (>= %d) x %d float64 tensor" % (len(rows), n_x))
+    rc = nat.lib().sb2_sim_build_rows_dev(nat.SIM_KINDS[kind], n_x, inputs["n_y"], nat.ptr(inputs["ptr"]),
+                                          nat.ptr(inputs["idx"]), nat.ptr(inputs["val"]), inputs["nnz"],
+                                          inputs["denom"], int(min_support), float(global_mean),
+                                          nat.ptr(inputs["bx"]), nat.ptr(inputs["by"]), float(shrinkage),
+                                          nat.ptr(rows), len(rows), nat.ptr(out), n_x, nat.stream())
+    nat.check(rc)
+    return out
+
+
 def _host(t):
     return t.cpu().numpy()
 
