@@ -179,6 +179,33 @@ def svdpp_sgd(u, i, r, u_ptr, ui_idx, pu, qi, yj, n_epochs, global_mean, lr_bu, 
     return pu, qi, yj, bu, bi
 
 
+# variant bits of svdpp_relaxed_sgd: deliberate deviations from the relaxation, for the mutation tests
+PP_Y_FROZEN, PP_NO_DECAY, PP_ISQ_INV_N, PP_Z_FROZEN, PP_C_RATERS, PP_G_KEPT = 1, 2, 4, 8, 16, 32
+
+
+def svdpp_relaxed_sgd(u, i, r, u_ptr, ui_idx, stratum, order, bounds, pu, qi, yj, n_epochs, global_mean, lr_bu,
+                      lr_bi, lr_pu, lr_qi, lr_yj, reg_bu, reg_bi, reg_pu, reg_qi, reg_yj, variant=0):
+    """NOT the reference: the stratified kernel's SVD++ relaxation in fp64 (see orc_svdpp_relaxed_sgd).
+    stratum: per rating (indexed like u); order: the ratings in the sequence they are applied; bounds: the chunks'
+    strata, chunk c = [bounds[c], bounds[c + 1]).  Returns (pu, qi, yj, bu, bi)."""
+    u, i, r = _i32(u), _i32(i), _f64(r)
+    u_ptr, ui_idx, stratum, order, bounds = _i64(u_ptr), _i32(ui_idx), _i32(stratum), _i64(order), _i32(bounds)
+    assert len(u_ptr) == len(pu) + 1 and len(stratum) == len(u) and len(bounds) >= 2
+    pu, qi, yj = (np.array(a, dtype=np.float64, order="C") for a in (pu, qi, yj))
+    bu, bi = np.zeros(pu.shape[0]), np.zeros(qi.shape[0])
+    d = C.c_double
+    rc = lib().orc_svdpp_relaxed_sgd(C.c_int64(pu.shape[0]), C.c_int64(qi.shape[0]), C.c_int64(len(u)),
+                                     C.c_int(pu.shape[1]), _p(u, C.c_int32), _p(i, C.c_int32), _p(r, C.c_double),
+                                     _p(u_ptr, C.c_int64), _p(ui_idx, C.c_int32), _p(stratum, C.c_int32),
+                                     C.c_int64(len(order)), _p(order, C.c_int64), C.c_int(len(bounds) - 1),
+                                     _p(bounds, C.c_int32), C.c_int(n_epochs), d(global_mean), d(lr_bu), d(lr_bi),
+                                     d(lr_pu), d(lr_qi), d(lr_yj), d(reg_bu), d(reg_bi), d(reg_pu), d(reg_qi),
+                                     d(reg_yj), C.c_int(variant), _p(pu, C.c_double), _p(qi, C.c_double),
+                                     _p(yj, C.c_double), _p(bu, C.c_double), _p(bi, C.c_double))
+    _check(rc)
+    return pu, qi, yj, bu, bi
+
+
 def nmf_sgd(n_users, n_items, u, i, r, n_ur, n_ir, pu, qi, n_epochs, biased, global_mean, reg_pu, reg_qi,
             reg_bu, reg_bi, lr_bu, lr_bi):
     u, i, r = _i32(u), _i32(i), _f64(r)

@@ -320,6 +320,127 @@ int orc_svdpp_sgd(int64_t n, int f, const int32_t *u, const int32_t *i, const do
     return ORC_OK;
 }
 
+/* ------------------------------------------------------------------------------------------
+ * NOT the reference: the SVD++ relaxation of the stratified SGD kernel (surprise_b200/csrc/sgd.cu,
+ * DESIGN.md section 6), restated in fp64 as an element-wise schedule oracle for
+ * tests/test_gpu_sgd_schedule.py.  The reference updates every y_j, j in I_u, with each rating of u;
+ * the kernel keeps z_u = sum_{j in I_u} y_j / sqrt|I_u| and a gradient accumulator g_u per user and
+ * applies the accumulated gradients to y_j once per chunk of strata:
+ *
+ *   for each epoch, for each chunk c (strata [bounds[c], bounds[c+1])):
+ *     z_u = isq_u sum_{j in I_u} y_j;  g_u = 0;  cnt_u = 0           (svdpp_user_refresh_kernel)
+ *     for k in order whose stratum lies in the chunk:
+ *       err = r - (mu + bu + bi + q.(p + z))
+ *       bu += lr_bu (err - reg_bu bu);  bi += lr_bi (err - reg_bi bi)
+ *       p' = p + lr_pu (err q - reg_pu p);  q' = q + lr_qi (err (p + z) - reg_qi q)
+ *       z' = z + lr_yj (err q - reg_yj z);  g += err isq_u q;  cnt_u += 1      (old p, q, z)
+ *     for every item j with c_j = sum_{u in U_j} cnt_u > 0:              (svdpp_item_apply_kernel)
+ *       y_j = y_j d^c_j + lr_yj (1 - d^c_j) / (c_j (1 - d)) sum_{u in U_j} g_u,  d = 1 - lr_yj reg_yj
+ *       (reg_yj = 0: y_j + lr_yj sum g_u)
+ *
+ * isq_u = 1/sqrt|I_u| (0 without ratings); I_u from the ur CSR (u_ptr, ui_idx), U_j = the raters of j
+ * among all n ratings (u, i), whether or not `order` holds them.  stratum[k] is rating k's stratum,
+ * order[0 .. n_order) the sequence in which the ratings are applied (every rating of a chunk in the
+ * order they appear there).  `variant` = 0 is the relaxation above; its bits each restate one way a
+ * kernel could deviate from it, for the mutation tests (tests/test_sgd_schedule_cpu.py):
+ * ------------------------------------------------------------------------------------------ */
+enum {
+    ORC_PP_Y_FROZEN = 1,      /* the y_j application never runs */
+    ORC_PP_NO_DECAY = 2,      /* y_j d^c_j + lr_yj sum g_u: the decay of the c_j updates not integrated */
+    ORC_PP_ISQ_INV_N = 4,     /* 1/|I_u| instead of 1/sqrt|I_u| */
+    ORC_PP_Z_FROZEN = 8,      /* z_u not advanced by the user's own updates */
+    ORC_PP_C_RATERS = 16,     /* c_j = raters of j with cnt_u > 0 instead of their ratings */
+    ORC_PP_G_KEPT = 32,       /* g_u not reset between chunks */
+};
+
+int orc_svdpp_relaxed_sgd(int64_t n_users, int64_t n_items, int64_t n, int f, const int32_t *u,
+                          const int32_t *i, const double *r, const int64_t *u_ptr, const int32_t *ui_idx,
+                          const int32_t *stratum, int64_t n_order, const int64_t *order, int n_chunks,
+                          const int32_t *bounds, int n_epochs, double global_mean, double lr_bu, double lr_bi,
+                          double lr_pu, double lr_qi, double lr_yj, double reg_bu, double reg_bi, double reg_pu,
+                          double reg_qi, double reg_yj, int variant, double *pu, double *qi, double *yj,
+                          double *bu, double *bi)
+{
+    const size_t su = (size_t)n_users * f;
+    double *z = malloc(su * sizeof(double)), *g = calloc(su, sizeof(double));
+    double *isq = malloc((size_t)n_users * sizeof(double)), *cnt = calloc((size_t)n_users, sizeof(double));
+    double *acc = malloc((size_t)n_items * f * sizeof(double)), *cj = malloc((size_t)n_items * sizeof(double));
+    int64_t *seen = malloc((size_t)n_users * sizeof(int64_t));
+    int rc = ORC_OK;
+    if (!z || !g || !isq || !cnt || !acc || !cj || !seen) { rc = ORC_NOMEM; goto done; }
+    for (int64_t x = 0; x < n_users; ++x) {
+        const double len = (double)(u_ptr[x + 1] - u_ptr[x]);
+        isq[x] = len > 0 ? ((variant & ORC_PP_ISQ_INV_N) ? 1.0 / len : 1.0 / sqrt(len)) : 0.0;
+        seen[x] = -1;
+    }
+    memset(bu, 0, (size_t)n_users * sizeof(double));
+    memset(bi, 0, (size_t)n_items * sizeof(double));
+    const double x1 = lr_yj * reg_yj, l1 = log1p(-x1);
+    int64_t pass = 0;
+    for (int ep = 0; ep < n_epochs; ++ep)
+        for (int c = 0; c < n_chunks; ++c, ++pass) {
+            const int32_t lo = bounds[c], hi = bounds[c + 1];
+            if (lo >= hi) continue;
+            for (int64_t x = 0; x < n_users; ++x) cnt[x] = 0.0;
+            if (!(variant & ORC_PP_G_KEPT)) memset(g, 0, su * sizeof(double));
+            for (int64_t a = 0; a < n_order; ++a) {
+                const int64_t k = order[a];
+                if (stratum[k] < lo || stratum[k] >= hi) continue;
+                const int32_t uu = u[k], ii = i[k];
+                double *p = pu + (size_t)uu * f, *q = qi + (size_t)ii * f;
+                double *zu = z + (size_t)uu * f, *gu = g + (size_t)uu * f;
+                if (seen[uu] != pass) { /* z_u as of the chunk's start: y_j does not change inside a chunk */
+                    seen[uu] = pass;
+                    for (int j = 0; j < f; ++j) {
+                        double s = 0.0;
+                        for (int64_t b = u_ptr[uu]; b < u_ptr[uu + 1]; ++b) s += yj[(size_t)ui_idx[b] * f + j];
+                        zu[j] = isq[uu] * s;
+                    }
+                }
+                double dot = 0.0;
+                for (int j = 0; j < f; ++j) dot += q[j] * (p[j] + zu[j]);
+                const double err = r[k] - (global_mean + bu[uu] + bi[ii] + dot);
+                bu[uu] += lr_bu * (err - reg_bu * bu[uu]);
+                bi[ii] += lr_bi * (err - reg_bi * bi[ii]);
+                const double eg = err * isq[uu];
+                for (int j = 0; j < f; ++j) {
+                    const double puf = p[j], qif = q[j], zuf = zu[j];
+                    p[j] = puf + lr_pu * (err * qif - reg_pu * puf);
+                    q[j] = qif + lr_qi * (err * (puf + zuf) - reg_qi * qif);
+                    if (!(variant & ORC_PP_Z_FROZEN)) zu[j] = zuf + lr_yj * (err * qif - reg_yj * zuf);
+                    gu[j] += eg * qif;
+                }
+                cnt[uu] += 1.0;
+            }
+            if (variant & ORC_PP_Y_FROZEN) continue;
+            /* sum_{u in U_j} g_u and c_j, scattered over all n ratings */
+            memset(acc, 0, (size_t)n_items * f * sizeof(double));
+            memset(cj, 0, (size_t)n_items * sizeof(double));
+            for (int64_t k = 0; k < n; ++k) {
+                const int32_t uu = u[k], ii = i[k];
+                if (cnt[uu] > 0) cj[ii] += (variant & ORC_PP_C_RATERS) ? 1.0 : cnt[uu];
+                else if (!(variant & ORC_PP_G_KEPT)) continue; /* g_u = 0 */
+                const double *gu = g + (size_t)uu * f;
+                double *aj = acc + (size_t)ii * f;
+                for (int j = 0; j < f; ++j) aj[j] += gu[j];
+            }
+            for (int64_t ii = 0; ii < n_items; ++ii) {
+                if (cj[ii] == 0) continue;
+                double decay = 1.0, gain = lr_yj;
+                if (x1 > 0) {
+                    decay = exp(cj[ii] * l1);
+                    if (!(variant & ORC_PP_NO_DECAY)) gain = lr_yj * -expm1(cj[ii] * l1) / (cj[ii] * x1);
+                }
+                double *y = yj + (size_t)ii * f;
+                const double *aj = acc + (size_t)ii * f;
+                for (int j = 0; j < f; ++j) y[j] = y[j] * decay + gain * aj[j];
+            }
+        }
+done:
+    free(z); free(g); free(isq); free(cnt); free(acc); free(cj); free(seen);
+    return rc;
+}
+
 /* prediction_algorithms/matrix_factorization.pyx:684-730 (NMF.sgd epochs).
  * n_ur[u] = len(ur[u]), n_ir[i] = len(ir[i]).  global_mean already 0 when unbiased (:681-682). */
 int orc_nmf_sgd(int64_t n_users, int64_t n_items, int64_t n, int f, const int32_t *u, const int32_t *i,

@@ -18,6 +18,14 @@ hand-offs of item blocks are correct.  ``oracle.svd_sgd(u[o], i[o], r[o], ...)``
 element-wise reference for the kernel's factors.  DEP mode (``SB2_DSGD_DEP=1``) applies the same order: its
 dependency counts follow the colour-sorted records.
 
+SVD++ runs the same kernel and order, but not the reference's per-rating ``y_j`` updates: the user row carries
+``z_u = sum y_j / sqrt|I_u|`` and a gradient accumulator ``g_u``, and the accumulated gradients reach ``y_j`` once per
+chunk of strata (DESIGN.md section 6).  ``oracle_fit(..., yj0=...)`` restates that relaxation in fp64
+(``oracle.svdpp_relaxed_sgd``): the same order, each rating's stratum, and the chunks' strata (``chunk_bounds``: the
+whole epoch by default and on a ring, ``SB2_SVDPP_CHUNKS`` of them on one GPU).  Its link to the reference is pinned
+on the CPU (tests/test_sgd_schedule_cpu.py): on a conflict-free input, and with ``lr_yj = 0``, it equals
+``oracle.svdpp_sgd`` to fp64 rounding.
+
 ``plan_smem`` restates the planner's shared-memory arithmetic (``svd_plan_create_dev``) for the layout tests.
 """
 import numpy as np
@@ -29,8 +37,8 @@ SMEM_BUDGET = 200 * 1024
 # Hyper-parameters of the schedule-exact comparisons.  Learning rates this large make the update order a first-order
 # effect, so that a lost, duplicated or reordered update moves the factors far beyond fp32 rounding.
 LR, REG, INIT_STD, EPOCHS = 0.03, 0.02, 0.1, 2
-# Largest element-wise |kernel - oracle| allowed on pu, qi, bu, bi.  Every mutant schedule of
-# tests/test_sgd_schedule_cpu.py must move the oracle's factors by at least MARGIN times this.
+# Largest element-wise |kernel - oracle| allowed on pu, qi, bu, bi (and yj of SVD++, against the relaxation).  Every
+# mutant schedule of tests/test_sgd_schedule_cpu.py must move the oracle's factors by at least MARGIN times this.
 ATOL = 2e-5
 MARGIN = 20
 
@@ -40,12 +48,40 @@ def f32(x):
     return float(np.float32(x))
 
 
-def oracle_fit(u, i, r, order, pu0, qi0, epochs=EPOCHS, biased=True, lr=LR, reg=REG):
-    """The fp64 sequential oracle on the ratings in `order`, with the kernel's fp32 scalars."""
+def ur_csr(u, i, n_users):
+    """(u_ptr, ui_idx) of the ratings grouped by user, input order inside a user (Trainset.user_csr's layout)."""
+    u = np.asarray(u, dtype=np.int64)
+    o = np.argsort(u, kind="stable")
+    return np.r_[0, np.cumsum(np.bincount(u, minlength=n_users))].astype(np.int64), np.asarray(i)[o].astype(np.int32)
+
+
+def chunk_bounds(n_strata, chunks=1):
+    """Strata of the y_j applications of one epoch: chunk c = [bounds[c], bounds[c + 1]) (svd_plan_run)."""
+    return [n_strata * c // chunks for c in range(chunks + 1)]
+
+
+def oracle_fit(u, i, r, order, pu0, qi0, epochs=EPOCHS, biased=True, lr=LR, reg=REG, yj0=None, stratum=None,
+               bounds=None, mu=None, variant=0):
+    """The fp64 oracle on the ratings in `order`, with the kernel's fp32 scalars.  lr / reg: one value for all, or
+    (bu, bi, pu, qi[, yj]); mu: the global mean (default: the mean of r).
+
+    SVD (yj0 None): the sequential reference; returns (pu, qi, bu, bi).
+    SVD++ (yj0 given): the kernel's relaxation (oracle.svdpp_relaxed_sgd), always biased; `stratum` per rating
+    (indexed like u), `bounds` the chunks' strata (chunk_bounds), `variant` a mutation of it; returns
+    (pu, qi, bu, bi, yj)."""
     import oracle
-    mu = f32(np.mean(r)) if biased else 0.0
-    return oracle.svd_sgd(u[order], i[order], r[order], pu0, qi0, epochs, biased, mu, *([f32(lr)] * 4),
-                          *([f32(reg)] * 4))
+    pp = yj0 is not None
+    k = 5 if pp else 4
+    lr = [f32(x) for x in (lr if np.ndim(lr) else [lr] * k)]
+    reg = [f32(x) for x in (reg if np.ndim(reg) else [reg] * k)]
+    assert len(lr) == len(reg) == k
+    mu = f32(np.mean(r) if mu is None else mu) if biased or pp else 0.0
+    if not pp:
+        return oracle.svd_sgd(u[order], i[order], r[order], pu0, qi0, epochs, biased, mu, *lr, *reg)
+    ptr, idx = ur_csr(u, i, len(pu0))
+    pu, qi, yj, bu, bi = oracle.svdpp_relaxed_sgd(u, i, r, ptr, idx, stratum, order, bounds, pu0, qi0, yj0, epochs,
+                                                  mu, *lr, *reg, variant=variant)
+    return pu, qi, bu, bi, yj
 
 
 def max_dist(a, b):

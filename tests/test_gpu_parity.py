@@ -745,6 +745,15 @@ def test_svd_conflict_free_input_matches_oracle():
         pu, qi, bu, bi = oracle.svd_sgd(u, i, r, pu0, qi0, 3, biased, float(ts.global_mean), *([.005] * 4), *([.02] * 4))
         assert np.allclose(algo.pu, pu, rtol=0, atol=2e-6) and np.allclose(algo.qi, qi, rtol=0, atol=2e-6)
         assert np.allclose(algo.bu, bu, rtol=0, atol=2e-6) and np.allclose(algo.bi, bi, rtol=0, atol=2e-6)
+    # SVD++: each y_j has one rater, who rates nothing else, so its relaxation is exact here as well
+    algo = sb.SVDpp(n_factors=12, n_epochs=3, random_state=4).fit(ts)
+    rs = np.random.RandomState(4)
+    pu0, qi0, yj0 = (rs.normal(0, .1, (n, 12)) for _ in range(3))
+    ptr, idx, _ = ts.user_csr()
+    want = oracle.svdpp_sgd(u, i, r, ptr, idx, pu0, qi0, yj0, 3, float(ts.global_mean), *([.007] * 5), *([.02] * 5))
+    for name, w in zip(("pu", "qi", "yj", "bu", "bi"), want):
+        assert np.allclose(getattr(algo, name), w, rtol=0, atol=2e-6), name
+    assert np.abs(algo.yj - yj0).max() > 1e-4
 
 
 def test_svd_split_launches_bit_identical(monkeypatch):

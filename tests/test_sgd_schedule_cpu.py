@@ -6,7 +6,11 @@
 * A literal per-rating transcription of dsgd_key_kernel and dsgd_color_kernel gives the same order.
 * Discrimination: schedules that a subtly wrong kernel would apply (strata swapped, colour order ignored, tail
   reversed, a rating lost, the wrong cluster size in the key) move the oracle's factors by at least MARGIN x ATOL,
-  the tolerance of the element-wise GPU comparison (tests/test_gpu_sgd_schedule.py).
+  the tolerance of the element-wise GPU comparison (tests/test_gpu_sgd_schedule.py).  For SVD++ the same order
+  mutants and the y_j-side ones (y_j frozen, the decay not integrated, 1/|I_u|, z_u not advanced, c_j counting
+  raters, a chunk count off by one, g_u kept across chunks) move the relaxation by at least MARGIN x ATOL.
+* The SVD++ relaxation (oracle.svdpp_relaxed_sgd) equals its pseudo-code transcribed in numpy, and the reference
+  (oracle.svdpp_sgd) where the two must agree: on a conflict-free input, and with lr_yj = 0 in the same order.
 * The planner's shared-memory arithmetic: the item counts at which capping B at the co-resident clusters used to
   leave a clustered plan without item buffers.
 """
@@ -167,12 +171,30 @@ DISCRIMINATION = {
 }
 
 
+def _pp_mutants():
+    """SVD++ relaxations a subtly wrong kernel or host would apply: name -> (chunks of the exact schedule, chunks of
+    the mutant, variant bits of oracle.svdpp_relaxed_sgd)."""
+    return {
+        "y_j frozen": (1, 1, oracle.PP_Y_FROZEN),
+        "decay not integrated": (1, 1, oracle.PP_NO_DECAY),
+        "1/|I_u|": (1, 1, oracle.PP_ISQ_INV_N),
+        "z not advanced": (1, 1, oracle.PP_Z_FROZEN),
+        "c_j from raters": (1, 1, oracle.PP_C_RATERS),
+        "chunks 2 instead of 1": (1, 2, 0),
+        "chunks 2 instead of 3": (3, 2, 0),
+        "g_u not reset between chunks": (3, 3, oracle.PP_G_KEPT),
+    }
+
+
 @pytest.mark.parametrize("case", sorted(DISCRIMINATION))
 def test_mutant_schedules_move_the_factors(case):
+    """SVD, then SVD++ (the relaxation of tests/sgd_schedule.oracle_fit): the order mutants, and for SVD++ the
+    mutants of the y_j side."""
     shape, B, C, f = DISCRIMINATION[case]
     u, i, r, nu, ni = S.draw(**shape)
     rng = np.random.RandomState(0)
     pu0, qi0 = rng.normal(0, S.INIT_STD, (nu, f)), rng.normal(0, S.INIT_STD, (ni, f))
+    yj0 = rng.normal(0, S.INIT_STD, (ni, f))
     o, mutants = _mutants(u, i, B, C, 1)
     want = S.oracle_fit(u, i, r, o, pu0, qi0)
     if case == "dense":
@@ -184,6 +206,25 @@ def test_mutant_schedules_move_the_factors(case):
         report.append("%s: %.3g = %.0f x ATOL" % (name, d, d / S.ATOL))
         assert d >= S.MARGIN * S.ATOL, (case, name, d)
     print("\n%s (B=%d, C=%d, f=%d): %s" % (case, B, C, f, "; ".join(report)))
+
+    stratum = S.schedule(u, i, B, C)["stratum"]
+
+    def pp(order, chunks, variant=0):
+        return S.oracle_fit(u, i, r, order, pu0, qi0, yj0=yj0, stratum=stratum, bounds=S.chunk_bounds(B, chunks),
+                            variant=variant)
+    exact = {1: pp(o, 1)}
+    runs = [(name, exact[1], pp(m, 1)) for name, m in mutants.items()]
+    for name, (base, chunks, variant) in _pp_mutants().items():
+        if base not in exact:
+            exact[base] = pp(o, base)
+        runs.append((name, exact[base], pp(o, chunks, variant)))
+    report, dists = [], []
+    for name, a, b in runs:
+        d = S.max_dist(a, b)
+        dists.append(d / S.ATOL)
+        report.append("%s: %.3g = %.0f x ATOL" % (name, d, d / S.ATOL))
+        assert d >= S.MARGIN * S.ATOL, (case, "svdpp", name, d)
+    print("%s SVD++: smallest %.0f x ATOL; %s" % (case, min(dists), "; ".join(report)))
 
 
 def test_oracle_is_order_sensitive_only_through_the_order():
@@ -197,6 +238,125 @@ def test_oracle_is_order_sensitive_only_through_the_order():
     w = oracle.svd_sgd(u[o], i[o], r[o], pu0, qi0, S.EPOCHS, True, S.f32(np.mean(r)), *([S.f32(S.LR)] * 4),
                        *([S.f32(S.REG)] * 4))
     assert all(np.array_equal(x, y) for x, y in zip(a, w))
+
+
+# --------------------------------------------------------------------------------------------------------------
+# the SVD++ relaxation (oracle.svdpp_relaxed_sgd) and its link to the reference (oracle.svdpp_sgd)
+LRS = (0.011, 0.013, 0.017, 0.019, 0.023)        # bu, bi, pu, qi, yj: a swapped pair moves the result
+REGS = (0.029, 0.031, 0.037, 0.041, 0.043)
+
+
+def _relaxed_py(u, i, r, order, stratum, bounds, pu0, qi0, yj0, epochs, mu, lr, reg):
+    """The relaxation of DESIGN.md section 6, literally and slowly (small inputs only)."""
+    (lbu, lbi, lpu, lqi, lyj), (rbu, rbi, rpu, rqi, ryj) = lr, reg
+    nu, ni = len(pu0), len(qi0)
+    pu, qi, yj, bu, bi = pu0.copy(), qi0.copy(), yj0.copy(), np.zeros(nu), np.zeros(ni)
+    items = [i[u == x] for x in range(nu)]
+    raters = [u[i == j] for j in range(ni)]
+    isq = np.array([1 / np.sqrt(len(s)) if len(s) else 0. for s in items])
+    d = 1 - lyj * ryj
+    for _ in range(epochs):
+        for lo, hi in zip(bounds[:-1], bounds[1:]):
+            z = np.stack([isq[x] * yj[items[x]].sum(0) for x in range(nu)])
+            g, cnt = np.zeros_like(pu), np.zeros(nu)
+            for k in order:
+                if not lo <= stratum[k] < hi:
+                    continue
+                x, j = u[k], i[k]
+                p, q, zz = pu[x].copy(), qi[j].copy(), z[x].copy()
+                err = r[k] - (mu + bu[x] + bi[j] + q @ (p + zz))
+                bu[x] += lbu * (err - rbu * bu[x])
+                bi[j] += lbi * (err - rbi * bi[j])
+                pu[x] = p + lpu * (err * q - rpu * p)
+                qi[j] = q + lqi * (err * (p + zz) - rqi * q)
+                z[x] = zz + lyj * (err * q - ryj * zz)
+                g[x] += err * isq[x] * q
+                cnt[x] += 1
+            for j in range(ni):
+                c = cnt[raters[j]].sum()
+                if c == 0:
+                    continue
+                gain = lyj if d == 1 else lyj * (1 - d ** c) / (c * (1 - d))
+                yj[j] = yj[j] * d ** c + gain * g[raters[j]].sum(0)
+    return pu, qi, bu, bi, yj
+
+
+@pytest.mark.parametrize("reg_yj", (REGS[4], 0.0))
+@pytest.mark.parametrize("chunks", (1, 3))
+def test_relaxed_oracle_literal_transcription(chunks, reg_yj):
+    """The C relaxation equals its pseudo-code, transcribed in numpy, to fp64 rounding; reg_yj = 0 takes the plain
+    sum (no 0 / 0)."""
+    u, i, r, nu, ni = S.draw(40, 30, 500, seed=8)
+    B, C = 4, 2
+    sc = S.schedule(u, i, B, C)
+    rng = np.random.RandomState(5)
+    pu0, qi0, yj0 = (rng.normal(0, S.INIT_STD, (m, 6)) for m in (nu, ni, ni))
+    reg = REGS[:4] + (reg_yj,)
+    got = S.oracle_fit(u, i, r, sc["order"], pu0, qi0, 2, lr=LRS, reg=reg, yj0=yj0, stratum=sc["stratum"],
+                       bounds=S.chunk_bounds(B, chunks))
+    want = _relaxed_py(u, i, r, sc["order"], sc["stratum"], S.chunk_bounds(B, chunks), pu0, qi0, yj0, 2,
+                       S.f32(np.mean(r)), [S.f32(x) for x in LRS], [S.f32(x) for x in reg])
+    assert all(np.isfinite(x).all() for x in got)
+    assert S.max_dist(got, want) <= 1e-12, [float(np.abs(a - b).max()) for a, b in zip(got, want)]
+    assert S.max_dist(got[4:], (yj0,)) > 1e-3                    # y_j moved
+
+
+def _pp_reference(u, i, r, order, pu0, qi0, yj0, epochs, lr, reg):
+    """oracle.svdpp_sgd on the ratings in `order`, as (pu, qi, bu, bi, yj)."""
+    ptr, idx = S.ur_csr(u, i, len(pu0))
+    pu, qi, yj, bu, bi = oracle.svdpp_sgd(u[order], i[order], r[order], ptr, idx, pu0, qi0, yj0, epochs,
+                                          S.f32(np.mean(r)), *[S.f32(x) for x in lr], *[S.f32(x) for x in reg])
+    return pu, qi, bu, bi, yj
+
+
+@pytest.mark.parametrize("B,C,chunks", [(1, 1, 1), (4, 2, 1), (8, 2, 3)])
+def test_relaxed_oracle_is_the_reference_on_a_conflict_free_input(B, C, chunks):
+    """A permutation matrix of ratings: each y_j has one rater, who rates nothing else, so applying its gradient
+    after the chunk is the reference's per-rating update."""
+    n, f = 400, 12
+    rng = np.random.RandomState(9)
+    u = np.arange(n, dtype=np.int32)
+    i = rng.permutation(n).astype(np.int32)
+    r = rng.randint(1, 6, n).astype(np.float64)
+    pu0, qi0, yj0 = (rng.normal(0, S.INIT_STD, (n, f)) for _ in range(3))
+    sc = S.schedule(u, i, B, C)
+    got = S.oracle_fit(u, i, r, sc["order"], pu0, qi0, 3, lr=LRS, reg=REGS, yj0=yj0, stratum=sc["stratum"],
+                       bounds=S.chunk_bounds(B, chunks))
+    want = _pp_reference(u, i, r, sc["order"], pu0, qi0, yj0, 3, LRS, REGS)
+    assert S.max_dist(got, want) <= 1e-12, [float(np.abs(a - b).max()) for a, b in zip(got, want)]
+    assert S.max_dist(got[4:], (yj0,)) > 1e-3
+
+
+@pytest.mark.parametrize("chunks", (1, 3))
+def test_relaxed_oracle_without_lr_yj_is_the_reference_in_the_same_order(chunks):
+    """lr_yj = 0: y_j and z_u never move, and the relaxation is the reference applied in the kernel's order."""
+    u, i, r, nu, ni = S.draw(600, 400, 30_000, seed=1)
+    B, C, f = 8, 2, 20
+    sc = S.schedule(u, i, B, C)
+    rng = np.random.RandomState(0)
+    pu0, qi0, yj0 = (rng.normal(0, S.INIT_STD, (m, f)) for m in (nu, ni, ni))
+    lr = LRS[:4] + (0.0,)
+    got = S.oracle_fit(u, i, r, sc["order"], pu0, qi0, lr=lr, reg=REGS, yj0=yj0, stratum=sc["stratum"],
+                       bounds=S.chunk_bounds(B, chunks))
+    want = _pp_reference(u, i, r, sc["order"], pu0, qi0, yj0, S.EPOCHS, lr, REGS)
+    assert S.max_dist(got, want) <= 1e-12, [float(np.abs(a - b).max()) for a, b in zip(got, want)]
+    assert np.array_equal(got[4], yj0)
+
+
+def test_relaxed_oracle_reg_yj_zero_is_the_limit():
+    """reg_yj = 0 (the plain sum lr_yj sum g_u) is the limit of the integrated decay as reg_yj -> 0."""
+    u, i, r, nu, ni = S.draw(300, 200, 8000, seed=4)
+    sc = S.schedule(u, i, 8, 2)
+    rng = np.random.RandomState(1)
+    pu0, qi0, yj0 = (rng.normal(0, S.INIT_STD, (m, 8)) for m in (nu, ni, ni))
+
+    def fit(reg_yj, variant=0):
+        return S.oracle_fit(u, i, r, sc["order"], pu0, qi0, yj0=yj0, stratum=sc["stratum"],
+                            bounds=S.chunk_bounds(8), reg=(S.REG,) * 4 + (reg_yj,), variant=variant)
+    plain = fit(0.0)
+    assert S.max_dist(plain, fit(1e-9)) <= 1e-6
+    assert S.max_dist(plain, fit(0.0, oracle.PP_NO_DECAY)) == 0.0
+    assert S.max_dist(plain, fit(S.REG)) >= S.MARGIN * S.ATOL
 
 
 # --------------------------------------------------------------------------------------------------------------
