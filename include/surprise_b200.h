@@ -430,6 +430,26 @@ int sb2_top_n_hits_dev(int64_t n_rows, const int32_t* items, int64_t ld, const i
                        const double* disc, int32_t* hits, double* rr, double* dcg, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Coverage, novelty and intra-list similarity of top-N lists (AlgoBase.top_n_list_measures; the definition is
+ * accuracy.top_n_list_measures, DESIGN.md section 3.11).  All arrays are DEVICE arrays.  items (int32, row b at
+ * items + b * ld), est (fp64, same layout) and count (int32 per row) are a block of sb2_top_n_select_dev's output;
+ * w <= ld is the cutoff.  With c_b = min(count[b], w) and L_b = items[b * ld + 0 .. c_b):
+ *   covered[b] = 1 when some p < c_b has est[b * ld + p] >= threshold (when has_threshold is 0: when c_b > 0), else 0;
+ *   nov[b] = the sum of info[L_b[p]] over p ascending;
+ *   ils[b] = the sum of sim[L_b[p] * n_items + L_b[q]] over p < q, p ascending and q ascending inside it (only when
+ *   sim is not null; sim is the n_items x n_items row-major item-item similarity);
+ *   seen[L_b[p]] = 1 for every p (a byte per item; the call never clears it, so one zeroed array can collect several
+ *   calls).
+ * Each sum is taken from +0.0 with one fp64 add per term (no FMA).  info (fp64, n_items entries) is the host's
+ * self-information table, so no logarithm is evaluated on the device.  est may be null when has_threshold is 0.
+ * SB2_ERR_INVALID for a null pointer, w < 0, ld < w, or a listed item outside [0, n_items) (checked inside the kernel;
+ * such an item is read nowhere).  One launch per call; the call synchronises `stream` to read that check.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_top_n_lists_dev(int64_t n_rows, const int32_t* items, int64_t ld, const double* est, const int32_t* count,
+                        int w, int has_threshold, double threshold, int64_t n_items, const double* info,
+                        const double* sim, int32_t* covered, double* nov, double* ils, uint8_t* seen, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Row shard of a SYMMETRIC multi-rank similarity build (SURVEY.md 8e "cyclic upper-triangular tile sharding").
  * Same arguments as sb2_sim_build_dev, but only sim[i][j] with row_begin <= i < row_end and j >= row_begin is
  * computed (tiles at or above the block diagonal; the shard's own diagonal square is mirrored like the

@@ -1,6 +1,6 @@
 """rmse / mse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), the FAQ's
-precision_recall_at_k, and top_n_measures: hit rate, ARHR, precision@N, recall@N and nDCG@N of get_top_n output against
-held-out ratings.
+precision_recall_at_k, top_n_measures: hit rate, ARHR, precision@N, recall@N and nDCG@N of get_top_n output against
+held-out ratings, and top_n_list_measures: user and catalog coverage, novelty and diversity of the lists themselves.
 
 fcp and precision_recall_at_k reduce to integer counts per user.  Where a CUDA device is usable and every r_ui and est
 is a real number that float64 holds exactly, the counts come from the device (csrc/rank_metrics.cu, DESIGN.md section
@@ -13,7 +13,7 @@ from operator import index, itemgetter
 
 import numpy as np
 
-__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k", "top_n_measures"]
+__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k", "top_n_measures", "top_n_list_measures"]
 
 
 def _need(predictions):
@@ -205,6 +205,111 @@ def _top_n_measure(name):
     None for any other name.  A top-N key with a malformed N raises ValueError."""
     key, at, num = name.lower().partition("@")
     if not at or key not in _TOP_N_LABELS:
+        return None
+    if not re.fullmatch("[0-9]+", num) or int(num) < 1:
+        raise ValueError("%s: N in %s@N must be an int >= 1" % (name, key))
+    return key, int(num)
+
+
+def top_n_list_measures(top_n, trainset, n, uids=None, threshold=None, sim=None, verbose=True):
+    """Coverage, novelty and diversity of ``top_n`` (get_top_n output, ``{raw uid: [(raw iid, est), ...]}``) over the
+    users ``uids`` of ``trainset``, as a dict of floats with keys user_coverage, catalog_coverage and novelty, plus
+    diversity when ``sim`` is given.
+
+    This plain-Python function is what the measures mean: AlgoBase.top_n_list_measures computes them on the device and
+    the tests compare it against this function.
+
+    * U is the distinct raw uids of ``uids`` in first-appearance order (equal uids merged as dict keys merge them), or
+      every trainset user in inner-id order when ``uids`` is None.  An empty U raises ValueError.  L_u is the first n
+      entries of ``top_n.get(u, [])`` and c_u = |L_u|: a uid absent from ``top_n`` (unknown to the trainset, or who
+      rated every item) has c_u = 0.  ``n`` must be an int >= 1.
+    * user_coverage = |{u in U : some entry of L_u has est >= threshold}| / |U|, a Python compare (a NaN est never
+      counts); with threshold None, a user counts when c_u > 0.
+    * catalog_coverage = |union over U of the iids of L_u| / trainset.n_items.
+    * novelty is the mean self-information of the recommended entries.  With the host table
+      ``info = np.log2(trainset.n_users / cnt)``, cnt the int64 np.diff of the item CSR's ptr (len(ir[i]); duplicate
+      ratings count), nov_u is the left-to-right sum from 0.0 of info[inner(iid)] over L_u, and
+      novelty = float(np.sum(nov)) over U in order, divided by sum(c_u); nan when sum(c_u) = 0.
+    * diversity = 1 - intra-list similarity, only when ``sim`` is given: a float64 (n_items, n_items) array indexed
+      by this trainset's inner item ids (any other shape raises ValueError).  ils_u is the sum from 0.0 of
+      float(sim[inner(L_u[p]), inner(L_u[q])]) over p < q, p ascending and q ascending inside it, and
+      diversity = 1.0 - float(np.sum(ils)) / sum(c_u (c_u - 1) / 2); nan when there are no pairs.
+
+    With ``verbose``, one line per key is printed."""
+    from .prediction_algorithms.algo_base import _check_top_n
+    n = _check_top_n(n)
+    if uids is None:
+        users = [trainset.to_raw_uid(u) for u in range(trainset.n_users)]
+    else:
+        users = list(dict.fromkeys(uids))
+    if not users:
+        raise ValueError("top-N list measures need at least one user")
+    if sim is not None:
+        sim = _check_list_sim(sim, trainset.n_items)
+    info = _novelty_table(trainset).tolist()
+    covered, nov, ils, count, seen = [], [], [], [], set()
+    for u in users:
+        l_u = top_n.get(u, [])[:n]
+        inner = [trainset.to_inner_iid(iid) for iid, _ in l_u]
+        covered.append(len(l_u) > 0 if threshold is None else any(est >= threshold for _, est in l_u))
+        count.append(len(l_u))
+        seen.update(inner)
+        s = 0.0
+        for i in inner:
+            s += info[i]
+        nov.append(s)
+        if sim is not None:
+            t = 0.0
+            for p in range(len(inner)):
+                for q in range(p + 1, len(inner)):
+                    t += float(sim[inner[p], inner[q]])
+            ils.append(t)
+    return _top_n_lists_of_counts(covered, nov, ils if sim is not None else None, count, len(seen), trainset.n_items,
+                                  n, verbose)
+
+
+def _check_list_sim(sim, n_items):
+    sim = np.asarray(sim, dtype=np.float64)
+    if sim.shape != (n_items, n_items):
+        raise ValueError("sim must be an (n_items, n_items) = (%d, %d) array indexed by inner item ids (got shape %s)"
+                         % (n_items, n_items, sim.shape))
+    return sim
+
+
+def _novelty_table(trainset):
+    """info[i] = np.log2(n_users / cnt[i]) (float64), cnt the number of ratings of inner item i (duplicates count)."""
+    cnt = np.diff(trainset.item_csr()[0]).astype(np.int64)
+    with np.errstate(divide="ignore"):
+        return np.log2(trainset.n_users / cnt)
+
+
+_LIST_LABELS = {"user_coverage": "User coverage", "catalog_coverage": "Catalog coverage", "novelty": "Novelty",
+                "diversity": "Diversity"}
+
+
+def _top_n_lists_of_counts(covered, nov, ils, count, n_seen, n_items, n, verbose):
+    """top_n_list_measures' result from the per-user covered flags, nov, ils (None without sim) and c_u in U order and
+    the number of distinct recommended items (both routes end here)."""
+    count = np.asarray(count, dtype=np.int64)
+    total = int(count.sum())
+    pairs = int((count * (count - 1) // 2).sum())
+    out = {"user_coverage": int(np.count_nonzero(covered)) / len(count),
+           "catalog_coverage": n_seen / n_items,
+           "novelty": float(np.sum(np.asarray(nov, dtype=np.float64))) / total if total else float("nan")}
+    if ils is not None:
+        ils_sum = float(np.sum(np.asarray(ils, dtype=np.float64)))
+        out["diversity"] = 1.0 - ils_sum / pairs if pairs else float("nan")
+    if verbose:
+        for key in out:
+            print("{0}@{1}:  {2:1.4f}".format(_LIST_LABELS[key], n, out[key]))
+    return out
+
+
+def _top_n_list_measure(name):
+    """(key, N) for a measure name key@N with key in user_coverage, catalog_coverage, novelty, diversity (any case)
+    and N an int >= 1; None for any other name.  A list-measure key with a malformed N raises ValueError."""
+    key, at, num = name.lower().partition("@")
+    if not at or key not in _LIST_LABELS:
         return None
     if not re.fullmatch("[0-9]+", num) or int(num) < 1:
         raise ValueError("%s: N in %s@N must be an int >= 1" % (name, key))

@@ -84,7 +84,7 @@ class BaseSearchCV(object):
             if m in ("mae", "rmse", "mse"):
                 rank[indices] = np.arange(len(indices)) + 1
                 best_index[m] = mean_test_measures.argmin()
-            elif m == "fcp" or accuracy._top_n_measure(m):
+            elif m == "fcp" or accuracy._top_n_measure(m) or accuracy._top_n_list_measure(m):
                 rank[indices] = np.arange(len(indices), 0, -1)
                 best_index[m] = mean_test_measures.argmax()
             best_params[m] = self.param_combinations[best_index[m]]

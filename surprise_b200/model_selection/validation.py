@@ -6,7 +6,8 @@ fit_and_score scores a device-batched algorithm from arrays: the fold's pairs ar
 (``Fold``), the estimates come from the algorithm's device estimate and the measures from
 ``accuracy._of_arrays``, which gives the bits ``accuracy.<m>(algo.test(testset))`` gives without building a
 Prediction per pair.  Any other algorithm or rating measure takes the tuple route.  The top-N measures hr@N,
-arhr@N, precision@N, recall@N and ndcg@N (threshold None) come from one ``algo._top_n_measures`` pass per fold.
+arhr@N, precision@N, recall@N and ndcg@N (threshold None) and the list measures user_coverage@N, catalog_coverage@N,
+novelty@N and diversity@N (over the same evaluated users) come from one ``algo._top_n_fold`` pass per fold.
 """
 import time
 
@@ -84,7 +85,20 @@ class Fold(object):
 
     def __init__(self, trainset, testset):
         self.trainset, self.testset = trainset, testset
-        self._test = self._train = None
+        self._test = self._train = self._cosine = None
+
+    def item_cosine(self):
+        """The item-item cosine similarity of the trainset (min_support 1), a CUDA float64 tensor: diversity@N's
+        similarity, built on first use.  ValueError when its 8 n_items^2 bytes exceed half the device's memory."""
+        if self._cosine is None:
+            from .. import similarities as sims
+            from ..prediction_algorithms.knns import _device_bytes, streams_similarities
+            ts = self.trainset
+            if streams_similarities(ts.n_items, _device_bytes()):
+                raise ValueError("diversity@N needs the %d x %d item-item cosine matrix, which takes more than half "
+                                 "the device's memory" % (ts.n_items, ts.n_items))
+            self._cosine = sims.build_device("cosine", ts.n_items, ts.user_csr(), min_support=1)
+        return self._cosine
 
     def test_pairs(self):
         if self._test is None:
@@ -124,20 +138,26 @@ def fit_and_score(algo, trainset, testset, measures, return_train_measures=False
 def _fit_and_score(algo, fold, measures, return_train_measures):
     top_n = {m: accuracy._top_n_measure(m) for m in measures}
     top_n = {m: v for m, v in top_n.items() if v is not None}
-    if top_n and return_train_measures:
+    lists = {m: accuracy._top_n_list_measure(m) for m in measures}
+    lists = {m: v for m, v in lists.items() if v is not None}
+    if (top_n or lists) and return_train_measures:
         raise ValueError("return_train_measures cannot be used with top-N measures (%s): trainset items are never "
-                         "recommended, so they would be 0" % ", ".join(top_n))
+                         "recommended, so they would be 0" % ", ".join(list(top_n) + list(lists)))
     t0 = time.time()
     algo.fit(fold.trainset)
     fit_time = time.time() - t0
-    rating = [m for m in measures if m not in top_n]
+    rating = [m for m in measures if m not in top_n and m not in lists]
     test_m, train_m, test_time = _score_ratings(algo, fold, rating, return_train_measures) if rating else ({}, {}, 0.0)
-    if top_n:
+    if top_n or lists:
         t0 = time.time()
-        ns = sorted(set(n for _, n in top_n.values()))
-        by_n = dict(zip(ns, algo._top_n_measures(fold, ns, None)))
+        hit_ns = sorted(set(n for _, n in top_n.values()))
+        list_ns = sorted(set(n for _, n in lists.values()))
+        sim = fold.item_cosine() if any(key == "diversity" for key, _ in lists.values()) else None
+        hit_res, list_res = algo._top_n_fold(fold, hit_ns, list_ns, sim)
         test_time += time.time() - t0
+        by_n, by_list_n = dict(zip(hit_ns, hit_res)), dict(zip(list_ns, list_res))
         test_m.update((m, by_n[n][key]) for m, (key, n) in top_n.items())
+        test_m.update((m, by_list_n[n][key]) for m, (key, n) in lists.items())
         test_m = {m: test_m[m] for m in measures}
     return test_m, train_m, fit_time, test_time
 

@@ -220,8 +220,8 @@ class AlgoBase(object):
 
     def _top_n_dev(self, width, users, _block_rows=None, _events=None, on_block=None):
         """top_n_inner's device block loop: (items, est, count) as device arrays of max(len(users), 1) rows.
-        ``on_block(b0, nr, items, count)``, if given, is called after each block's selection, when rows b0 .. b0 + nr
-        of the device arrays are final."""
+        ``on_block(b0, nr, items, est, count)``, if given, is called after each block's selection, when rows
+        b0 .. b0 + nr of the device arrays are final."""
         from .. import _native as nat
         torch = nat.torch_cuda()
         ts = self.trainset
@@ -268,7 +268,7 @@ class AlgoBase(object):
             if ev:
                 ev[2].record()
             if on_block is not None:
-                on_block(b0, nr, items, count)
+                on_block(b0, nr, items, est, count)
         return items, est, count
 
     # -- top-N measures against held-out ratings -------------------------------------------------------
@@ -285,41 +285,156 @@ class AlgoBase(object):
         """top_n_measures for each cutoff of ``ns`` on the testset of ``fold`` (a validation.Fold of this trainset): the
         lists are ranked once at the largest cutoff, whose first N entries are the top-N lists (the ranking is a total
         order), and the hits are counted once per cutoff."""
+        return self._top_n_fold(fold, ns, [], None, threshold, _block_rows)[0]
+
+    def _top_n_fold(self, fold, hit_ns, list_ns, sim, threshold=None, _block_rows=None):
+        """(top_n_measures at each cutoff of ``hit_ns``, top_n_list_measures at each cutoff of ``list_ns``) on the
+        testset of ``fold``, from one selection pass at the largest cutoff.  The list measures are taken over the
+        evaluated users U* of ``threshold`` (users unknown to the trainset have no list) with no est threshold;
+        ``sim`` (a CUDA float64 item-item matrix, or None) gives diversity."""
         from .. import accuracy
-        ns = [_check_top_n(n) for n in ns]
+        hit_ns = [_check_top_n(n) for n in hit_ns]
+        list_ns = [_check_top_n(n) for n in list_ns]
         ts = self.trainset
-        iu, n_rel, rel_ptr, rel_idx = fold.test_pairs().relevant(threshold, ts.n_items)
+        pairs = fold.test_pairs()
+        iu, n_rel, rel_ptr, rel_idx = pairs.relevant(threshold, ts.n_items)
         known = iu >= 0
-        top = max(ns)
+        top = max(hit_ns + list_ns)
         if not self._batched():
             lists = self.get_top_n(top, uids=[ts.to_raw_uid(u) for u in iu[known].tolist()])
-            return [accuracy.top_n_measures({u: l_u[:n] for u, l_u in lists.items()}, fold.testset, n, threshold,
-                                            ts.offset, verbose=False) for n in ns]
+            hits = [accuracy.top_n_measures({u: l_u[:n] for u, l_u in lists.items()}, fold.testset, n, threshold,
+                                            ts.offset, verbose=False) for n in hit_ns]
+            star = list(dict.fromkeys(u for u, r in zip(pairs._uids, pairs.r_ui.tolist())
+                                      if threshold is None or r >= threshold))
+            sim_h = None if sim is None else sim.cpu().numpy()
+            return hits, [accuracy.top_n_list_measures(lists, ts, n, star, None, sim_h, verbose=False)
+                          for n in list_ns]
         from .. import _native as nat
         width = min(top, ts.n_items)
-        inv, disc, idcg = accuracy._rank_tables(min(top, max(width, int(n_rel.max()))))
-        d_inv, d_disc = nat.to_dev(inv, np.float64), nat.to_dev(disc, np.float64)
-        d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
         n_k = int(known.sum())
-        outs = [tuple(nat.empty_dev((max(n_k, 1),), t) for t in (np.int32, np.float64, np.float64)) for _ in ns]
         lib, stream = nat.lib(), nat.stream()
+        hooks, outs = [], []
+        if hit_ns:
+            inv, disc, idcg = accuracy._rank_tables(min(max(hit_ns), max(width, int(n_rel.max()))))
+            d_inv, d_disc = nat.to_dev(inv, np.float64), nat.to_dev(disc, np.float64)
+            d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
+            outs = [tuple(nat.empty_dev((max(n_k, 1),), t) for t in (np.int32, np.float64, np.float64))
+                    for _ in hit_ns]
 
-        def count_hits(b0, nr, items, count):
-            for n, (hits, rr, dcg) in zip(ns, outs):
-                nat.check(lib.sb2_top_n_hits_dev(nr, nat.ptr(items[b0:]), width, nat.ptr(count[b0:]), min(n, width),
-                                                 nat.ptr(d_ptr[b0:]), nat.ptr(d_idx), len(rel_idx), nat.ptr(d_inv),
-                                                 nat.ptr(d_disc), nat.ptr(hits[b0:]), nat.ptr(rr[b0:]),
-                                                 nat.ptr(dcg[b0:]), stream))
+            def count_hits(b0, nr, items, est, count):
+                for n, (hits, rr, dcg) in zip(hit_ns, outs):
+                    nat.check(lib.sb2_top_n_hits_dev(nr, nat.ptr(items[b0:]), width, nat.ptr(count[b0:]),
+                                                     min(n, width), nat.ptr(d_ptr[b0:]), nat.ptr(d_idx), len(rel_idx),
+                                                     nat.ptr(d_inv), nat.ptr(d_disc), nat.ptr(hits[b0:]),
+                                                     nat.ptr(rr[b0:]), nat.ptr(dcg[b0:]), stream))
+            hooks.append(count_hits)
+        if list_ns:
+            count_lists, finish_lists = self._list_counter(list_ns, width, n_k, None, sim)
+            hooks.append(count_lists)
 
-        if n_k:
-            self._top_n_dev(width, iu[known], _block_rows, on_block=count_hits)
+        def on_block(*blk):
+            for hook in hooks:
+                hook(*blk)
+
+        count = self._top_n_dev(width, iu[known], _block_rows, on_block=on_block)[2] if n_k else None
         res = []
-        for n, out in zip(ns, outs):
+        for n, out in zip(hit_ns, outs):
             hits, rr, dcg = np.zeros(len(iu), dtype=np.int64), np.zeros(len(iu)), np.zeros(len(iu))
             for host, dev in zip((hits, rr, dcg), out):
                 host[known] = dev.cpu().numpy()[:n_k]
             res.append(accuracy._top_n_of_counts(hits, rr, dcg, n_rel, n, idcg, False))
-        return res
+        return res, (finish_lists(known, count) if list_ns else [])
+
+    # -- coverage, novelty and diversity of the top-N lists --------------------------------------------
+    def top_n_list_measures(self, n=10, uids=None, threshold=None, sim=None, _block_rows=None):
+        """User coverage, catalog coverage, novelty and (with ``sim``) diversity of this algorithm's top-n lists for the
+        users ``uids`` (raw ids; default every user): bit for bit ``accuracy.top_n_list_measures(self.get_top_n(n,
+        uids), self.trainset, n, uids, threshold, sim_array, verbose=False)``, without building get_top_n's dict.
+
+        An unknown uid raises ValueError, as get_top_n does.  ``sim`` is an (n_items, n_items) array indexed by this
+        trainset's inner item ids, uploaded once, or a fitted item-based k-NN model whose trainset is this one, whose
+        device matrix is read in place; a streamed or user-based model, or one fitted on another trainset, raises
+        ValueError.  A device-batched algorithm counts the lists on the device (sb2_top_n_lists_dev) when ``threshold``
+        is None or a real number float64 holds exactly; otherwise the definition runs over get_top_n."""
+        from .. import accuracy
+        n = _check_top_n(n)
+        ts = self.trainset
+        if uids is None:
+            raw_u, users = None, np.arange(ts.n_users, dtype=np.int32)
+        else:
+            raw_u = list(dict.fromkeys(uids))
+            users = np.array([ts.to_inner_uid(x) for x in raw_u], dtype=np.int32)
+        if not len(users):
+            raise ValueError("top-N list measures need at least one user")
+        model = self._list_sim_model(sim)
+        if not self._batched() or not (threshold is None or accuracy._exact_reals([threshold])):
+            arr = model.sim if model is not None else sim
+            return accuracy.top_n_list_measures(self.get_top_n(n, raw_u), ts, n, raw_u, threshold, arr, verbose=False)
+        from .. import _native as nat
+        if model is not None:
+            d_sim = model._sim_device()
+        else:
+            d_sim = None if sim is None else nat.to_dev(accuracy._check_list_sim(sim, ts.n_items), np.float64)
+        width = min(n, ts.n_items)
+        count_lists, finish_lists = self._list_counter([n], width, len(users), threshold, d_sim)
+        count = self._top_n_dev(width, users, _block_rows, on_block=count_lists)[2]
+        return finish_lists(np.ones(len(users), dtype=bool), count)[0]
+
+    def _list_sim_model(self, sim):
+        """``sim`` when it is a k-NN model top_n_list_measures can read the matrix of; None for an array or None."""
+        from .knns import SymmetricAlgo
+        if not isinstance(sim, SymmetricAlgo):
+            return None
+        if sim.sim_options["user_based"]:
+            raise ValueError("sim must be an item-based k-NN model (user_based=False)")
+        if getattr(sim, "trainset", None) is not self.trainset:
+            raise ValueError("sim must be a k-NN model fitted on this algorithm's trainset")
+        if sim._streamed:
+            raise ValueError("sim is a streamed k-NN model, which keeps no similarity matrix; pass the matrix instead")
+        return sim
+
+    def _list_counter(self, ns, width, n_rows, threshold, sim):
+        """(on_block, finish) computing top_n_list_measures at each cutoff of ``ns`` over the rows of one _top_n_dev
+        pass of n_rows users at ``width``: on_block is the pass's block hook (sb2_top_n_lists_dev once per cutoff);
+        finish(known, count) returns the results for the users U, where ``known`` (bool per user of U) marks the users
+        that had a row, in order, and ``count`` is the pass's count array (the others have no list)."""
+        from .. import _native as nat
+        from .. import accuracy
+        torch = nat.torch_cuda()
+        ts = self.trainset
+        d_info = nat.to_dev(accuracy._novelty_table(ts), np.float64)
+        rows = max(n_rows, 1)
+        outs = [(nat.empty_dev((rows,), np.int32), nat.empty_dev((rows,), np.float64),
+                 nat.empty_dev((rows,), np.float64) if sim is not None else None,
+                 torch.zeros(ts.n_items, dtype=torch.uint8, device=nat.device())) for _ in ns]
+        has_t = threshold is not None
+        lib, stream = nat.lib(), nat.stream()
+
+        def count_lists(b0, nr, items, est, count):
+            for n, (cov, nov, ils, seen) in zip(ns, outs):
+                nat.check(lib.sb2_top_n_lists_dev(nr, nat.ptr(items[b0:]), width, nat.ptr(est[b0:]),
+                                                  nat.ptr(count[b0:]), min(n, width), int(has_t),
+                                                  float(threshold) if has_t else 0.0, ts.n_items, nat.ptr(d_info),
+                                                  nat.ptr(sim), nat.ptr(cov[b0:]), nat.ptr(nov[b0:]),
+                                                  None if ils is None else nat.ptr(ils[b0:]), nat.ptr(seen), stream))
+
+        def finish(known, count):
+            c_u = np.zeros(len(known), dtype=np.int64)
+            if n_rows:
+                c_u[known] = count.cpu().numpy()[:n_rows]
+            res = []
+            for n, (cov, nov, ils, seen) in zip(ns, outs):
+                h_cov, h_nov, h_ils = np.zeros(len(known), dtype=bool), np.zeros(len(known)), np.zeros(len(known))
+                if n_rows:
+                    h_cov[known] = cov.cpu().numpy()[:n_rows] != 0
+                    h_nov[known] = nov.cpu().numpy()[:n_rows]
+                    if ils is not None:
+                        h_ils[known] = ils.cpu().numpy()[:n_rows]
+                res.append(accuracy._top_n_lists_of_counts(h_cov, h_nov, None if ils is None else h_ils,
+                                                           np.minimum(c_u, n), int(seen.sum()), ts.n_items, n, False))
+            return res
+
+        return count_lists, finish
 
     def _top_n_scorer(self):
         """Device arrays for sb2_mf_score_block_dev (dict: f, biased, pu, qi, bu, bi[, yj, up, ui]), or None when
