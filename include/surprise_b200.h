@@ -450,6 +450,28 @@ int sb2_top_n_lists_dev(int64_t n_rows, const int32_t* items, int64_t ld, const 
                         const double* sim, int32_t* covered, double* nov, double* ils, uint8_t* seen, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Where held-out items land in each user's full ranking (AlgoBase.rank_measures: AUC, MRR, MPR; the definition is
+ * accuracy.rank_measures, DESIGN.md section 3.12).  All arrays are DEVICE arrays.  rows, scores / ld, impossible,
+ * default_est, offset, low, high and the ur CSR u_ptr / ui_idx are exactly sb2_top_n_select_dev's: the candidates
+ * of row b are the items rows[b] did not rate, ranked in that function's order.  rel_idx[rel_ptr[b] ..
+ * rel_ptr[b + 1]) (int64 offsets into rel_idx, rel_len entries) are row b's relevant inner item ids, strictly
+ * ascending; a relevant item the user rated is no candidate.  With the position of a candidate = the number of
+ * candidates ranked before it, for every row b:
+ *   c[b] = the number of candidates, k[b] = the number of relevant candidates, s[b] (int64) = the sum of their
+ *   positions, f[b] = the smallest of them, or -1 when k[b] == 0.
+ * SB2_ERR_INVALID for a null pointer, ld < n_items, or a row whose offsets leave [0, rel_len], decrease, or whose
+ * list is not strictly ascending inside [0, n_items) (checked inside the kernel; such a row's outputs are not
+ * written); SB2_ERR_ZERO_DIVISION where a candidate has impossible == 2, as sb2_top_n_select_dev;
+ * SB2_ERR_UNSUPPORTED when the rated-item bitmap does not fit in shared memory (about 1.4 M items).  One launch per
+ * call, one pass over each row's scores per 2048 relevant candidates (at least one); the call synchronises `stream`
+ * to read its checks.
+ * ------------------------------------------------------------------------------------------------ */
+int sb2_top_n_ranks_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                        const uint8_t* impossible, double default_est, double offset, double low, double high,
+                        const int64_t* u_ptr, const int32_t* ui_idx, const int64_t* rel_ptr, const int32_t* rel_idx,
+                        int64_t rel_len, int32_t* c, int32_t* k, int64_t* s, int32_t* f, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Row shard of a SYMMETRIC multi-rank similarity build (SURVEY.md 8e "cyclic upper-triangular tile sharding").
  * Same arguments as sb2_sim_build_dev, but only sim[i][j] with row_begin <= i < row_end and j >= row_begin is
  * computed (tiles at or above the block diagonal; the shard's own diagonal square is mirrored like the

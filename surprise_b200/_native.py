@@ -112,6 +112,8 @@ SIGNATURES = {
     "sb2_top_n_hits_dev": (_int, [_i64, _vp, _i64, _vp, _int, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sb2_top_n_lists_dev": (_int, [_i64, _vp, _i64, _vp, _vp, _int, _int, _dbl, _i64, _vp, _vp, _vp, _vp, _vp, _vp,
                                    _vp]),
+    "sb2_top_n_ranks_dev": (_int, [_i64, _vp, _i64, _vp, _i64, _vp, _dbl, _dbl, _dbl, _dbl, _vp, _vp, _vp, _vp, _i64,
+                                   _vp, _vp, _vp, _vp, _vp]),
     "sb2_fcp_counts_dev": (_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "sb2_precision_at_k_counts_dev": (_int, [_i64, _i64, _vp, _vp, _vp, _vp, _dbl, _vp, _vp]),
 }

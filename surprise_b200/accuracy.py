@@ -1,6 +1,7 @@
 """rmse / mse / mae / fcp over a list of Prediction tuples (reference: surprise/accuracy.py:22-143), the FAQ's
 precision_recall_at_k, top_n_measures: hit rate, ARHR, precision@N, recall@N and nDCG@N of get_top_n output against
-held-out ratings, and top_n_list_measures: user and catalog coverage, novelty and diversity of the lists themselves.
+held-out ratings, top_n_list_measures: user and catalog coverage, novelty and diversity of the lists themselves, and
+rank_measures: AUC, MRR and mean percentile rank of held-out items over each user's full candidate ranking.
 
 fcp and precision_recall_at_k reduce to integer counts per user.  Where a CUDA device is usable and every r_ui and est
 is a real number that float64 holds exactly, the counts come from the device (csrc/rank_metrics.cu, DESIGN.md section
@@ -13,7 +14,8 @@ from operator import index, itemgetter
 
 import numpy as np
 
-__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k", "top_n_measures", "top_n_list_measures"]
+__all__ = ["rmse", "mse", "mae", "fcp", "precision_recall_at_k", "top_n_measures", "top_n_list_measures",
+           "rank_measures"]
 
 
 def _need(predictions):
@@ -314,6 +316,89 @@ def _top_n_list_measure(name):
     if not re.fullmatch("[0-9]+", num) or int(num) < 1:
         raise ValueError("%s: N in %s@N must be an int >= 1" % (name, key))
     return key, int(num)
+
+
+def rank_measures(top_n, testset, trainset, threshold=None, verbose=True):
+    """AUC, MRR and mean percentile rank (MPR) of the held-out rows ``(raw uid, raw iid, r_ui)`` of ``testset`` over
+    each user's full ranking ``top_n`` (get_top_n output at n = trainset.n_items), as a dict of floats with keys auc,
+    mrr and mpr.  Higher AUC and MRR are better; lower MPR is better.
+
+    This plain-Python function is what the measures mean: AlgoBase.rank_measures computes them on the device and the
+    tests compare it against this function.
+
+    * Users and relevance are those of top_n_measures: a row is relevant when ``threshold`` is None or
+      ``float(r_ui) - trainset.offset >= threshold``; U* is the uids with a relevant row, in first-appearance order,
+      equal uids merged as dict keys merge them; R_u is u's set of relevant raw iids (unknown items count) and
+      n_rel_u = |R_u|.  No relevant row raises ValueError.
+    * F_u = ``top_n.get(u, [])`` must be u's complete ranking: every item u did not rate in ``trainset``, in get_top_n
+      order, so len(F_u) = n_items - |distinct items of ur[u]| for a user the trainset knows and 0 for any other;
+      otherwise ValueError (pass ``get_top_n(n=trainset.n_items)``).
+    * c_u = len(F_u); K_u is the ascending list of 0-based positions p with F_u[p][0] in R_u, k_u = len(K_u),
+      s_u = sum(K_u) and f_u = K_u[0] when k_u > 0.  A relevant item not in F_u (unknown to the trainset, or rated by
+      u in it) is unranked.
+    * Per user, in integers until the divisions (each a float64 division): rr_u = 1.0 / (f_u + 1) if k_u else 0.0.
+      With neg_u = c_u - k_u negatives, when neg_u > 0, correct_u = k_u (c_u - 1) - s_u - k_u (k_u - 1) // 2 is the
+      number of (relevant, negative) pairs ordered correctly (an unranked relevant item makes none) and
+      auc_u = correct_u / (n_rel_u neg_u); a user with neg_u = 0 (an unknown user, or every candidate relevant) has no
+      AUC.  mpr_u = (s_u / (c_u - 1) if c_u > 1 else 0.0) + (n_rel_u - k_u): an unranked relevant item counts as
+      percentile 1.0, the bottom.
+    * mrr = float(np.mean(rr)) over U*; auc = float(np.mean(auc_u)) over the users that have one, nan when none does;
+      mpr = float(np.sum(mpr_u)) over U* divided by sum(n_rel_u).
+
+    The AUC is taken per user and then averaged over users (what some libraries call GAUC), never pooled over the
+    pairs of all users: the estimates of different users are not on a common scale.  With ``verbose``, one line per
+    measure is printed."""
+    relevant = {}
+    for uid, iid, r_ui in testset:
+        if threshold is None or float(r_ui) - trainset.offset >= threshold:
+            relevant.setdefault(uid, set()).add(iid)
+    if not relevant:
+        raise ValueError("rank measures need at least one relevant rating in the testset")
+    users = list(relevant)
+    inner = trainset.to_inner_uids(users)
+    ptr, idx, _ = trainset.user_csr()
+    c, k, s, f = [], [], [], []
+    for u, iu, r_u in zip(users, inner.tolist(), relevant.values()):
+        f_u = top_n.get(u, [])
+        want = trainset.n_items - len(np.unique(idx[ptr[iu]:ptr[iu + 1]])) if iu >= 0 else 0
+        if len(f_u) != want:
+            raise ValueError("rank measures need each user's complete ranking, %d items for user %r (got %d): pass "
+                             "get_top_n(n=trainset.n_items)" % (want, u, len(f_u)))
+        k_u = [p for p, (iid, _) in enumerate(f_u) if iid in r_u]
+        c.append(len(f_u))
+        k.append(len(k_u))
+        s.append(sum(k_u))
+        f.append(k_u[0] if k_u else -1)
+    return _rank_of_counts(c, k, s, f, [len(r_u) for r_u in relevant.values()], verbose)
+
+
+_RANK_LABELS = {"auc": "AUC", "mrr": "MRR", "mpr": "MPR"}
+
+
+def _rank_of_counts(c, k, s, f, n_rel, verbose):
+    """rank_measures' result from the per-user c_u, k_u, s_u, f_u (-1 when k_u = 0) and n_rel_u in U* order (both
+    routes end here)."""
+    c, k, s, f, n_rel = (np.asarray(x, dtype=np.int64) for x in (c, k, s, f, n_rel))
+    neg = c - k
+    has = neg > 0
+    correct = k * (c - 1) - s - k * (k - 1) // 2
+    auc_u = correct[has] / (n_rel[has] * neg[has])
+    with np.errstate(divide="ignore", invalid="ignore"):    # the branches np.where drops
+        rr = np.where(k > 0, 1.0 / (f + 1), 0.0)
+        pct = np.where(c > 1, s / (c - 1), 0.0)
+    out = {"auc": float(np.mean(auc_u)) if len(auc_u) else float("nan"),
+           "mrr": float(np.mean(rr)),
+           "mpr": float(np.sum(pct + (n_rel - k))) / int(n_rel.sum())}
+    if verbose:
+        for key, label in _RANK_LABELS.items():
+            print("{0}:  {1:1.4f}".format(label, out[key]))
+    return out
+
+
+def _rank_measure(name):
+    """The key of a rank measure name (auc, mrr or mpr, any case), or None for any other name."""
+    key = name.lower()
+    return key if key in _RANK_LABELS else None
 
 
 # -- device route ----------------------------------------------------------------------------------------------------

@@ -105,6 +105,10 @@ int top_n_hits_dev(int64_t n_rows, const int32_t* items, int64_t ld, const int32
 int top_n_lists_dev(int64_t n_rows, const int32_t* items, int64_t ld, const double* est, const int32_t* count, int w,
                     int has_threshold, double threshold, int64_t n_items, const double* info, const double* sim,
                     int32_t* covered, double* nov, double* ils, uint8_t* seen, cudaStream_t st);
+int top_n_ranks_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                    const uint8_t* impossible, double default_est, double offset, double low, double high,
+                    const int64_t* u_ptr, const int32_t* ui_idx, const int64_t* rel_ptr, const int32_t* rel_idx,
+                    int64_t rel_len, int32_t* c, int32_t* k, int64_t* s, int32_t* f, cudaStream_t st);
 int svd_plan_create_dev(int64_t n_users, int64_t n_items, int64_t n, const int32_t* u, const int32_t* i,
                         const double* r, const sb2_sgd_params* prm, int with_yj, const int64_t* u_ptr,
                         const int32_t* ui_idx, int rank, int world, cudaStream_t st, sb2_svd_plan** out);
@@ -856,6 +860,15 @@ int sb2_top_n_lists_dev(int64_t n_rows, const int32_t* items, int64_t ld, const 
     SB2_TRY(ensure_device());
     return top_n_lists_dev(n_rows, items, ld, est, count, w, has_threshold, threshold, n_items, info, sim, covered,
                            nov, ils, seen, (cudaStream_t)stream);
+}
+
+int sb2_top_n_ranks_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, const double* scores, int64_t ld,
+                        const uint8_t* impossible, double default_est, double offset, double low, double high,
+                        const int64_t* u_ptr, const int32_t* ui_idx, const int64_t* rel_ptr, const int32_t* rel_idx,
+                        int64_t rel_len, int32_t* c, int32_t* k, int64_t* s, int32_t* f, void* stream) {
+    SB2_TRY(ensure_device());
+    return top_n_ranks_dev(n_rows, rows, n_items, scores, ld, impossible, default_est, offset, low, high, u_ptr, ui_idx,
+                           rel_ptr, rel_idx, rel_len, c, k, s, f, (cudaStream_t)stream);
 }
 
 int sb2_sim_build_upper_dev(int kind, int64_t n_x, int64_t n_y, const int64_t* y_ptr, const int32_t* x_idx,

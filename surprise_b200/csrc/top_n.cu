@@ -4,7 +4,7 @@
 //   - a per-row selection shared by every algorithm: default_prediction for impossible pairs, offset, clipping,
 //     the user's trainset items masked out, and the first n in (score desc, item asc) order -- the order Python's
 //     stable sort(reverse=True) leaves the anti-testset (ascending inner item id per user) in.
-#include "common.cuh"
+#include "top_n.cuh"
 
 namespace sb2 {
 
@@ -175,51 +175,9 @@ int mf_score_block_dev(int64_t n_rows, const int32_t* rows, int64_t n_items, int
 // becomes the threshold.  A final sort emits them.  n > SEL_KMAX runs further passes, each taking the next K
 // strictly after the last emitted entry.
 // ------------------------------------------------------------------------------------------------
-constexpr int SEL_THREADS = 256;
 constexpr int SEL_PER = 4;                          // candidates per thread per tile
 constexpr int SEL_TILE = SEL_THREADS * SEL_PER;
 constexpr int SEL_KMAX = 2048;                      // entries kept per pass
-
-__device__ __forceinline__ double top_n_value(double s, int code, double def, double offset, double low,
-                                              double high) {
-    if (code == 1) s = def;
-    s = __dsub_rn(s, offset);
-    s = high < s ? high : s;   // np.minimum(high, est): est itself on ties (signed zeros) and NaN
-    s = low > s ? low : s;     // np.maximum(low, est)
-    return s;
-}
-
-__device__ __forceinline__ unsigned long long top_n_key(double v) {
-    if (v != v) return 0ull;   // NaN: after every number
-    const unsigned long long b = (unsigned long long)__double_as_longlong(__dadd_rn(v, 0.0));   // -0.0 -> +0.0
-    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-
-// (key desc, item asc)
-__device__ __forceinline__ bool top_n_better(unsigned long long ka, int ia, unsigned long long kb, int ib) {
-    return ka > kb || (ka == kb && ia < ib);
-}
-
-// sorts key/item[0, c) best-first; c is block-uniform
-__device__ void top_n_sort(unsigned long long* key, int* item, int c) {
-    int P = 1;
-    while (P < c) P <<= 1;
-    for (int j = c + threadIdx.x; j < P; j += SEL_THREADS) { key[j] = 0ull; item[j] = 0x7FFFFFFF; }
-    __syncthreads();
-    for (int k = 2; k <= P; k <<= 1)
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int x = threadIdx.x; x < P; x += SEL_THREADS) {
-                const int y = x ^ j;
-                if (y > x) {
-                    const unsigned long long kx = key[x], ky = key[y];
-                    const int ix = item[x], iy = item[y];
-                    const bool swap = (x & k) == 0 ? top_n_better(ky, iy, kx, ix) : top_n_better(kx, ix, ky, iy);
-                    if (swap) { key[x] = ky; key[y] = kx; item[x] = iy; item[y] = ix; }
-                }
-            }
-            __syncthreads();
-        }
-}
 
 __global__ void __launch_bounds__(SEL_THREADS)
 top_n_select_kernel(int64_t n_items, const int32_t* __restrict__ rows, const double* __restrict__ scores, int64_t ld,

@@ -81,10 +81,10 @@ class BaseSearchCV(object):
             indices = mean_test_measures.argsort()
             rank = np.empty_like(indices)
             cv_results["rank_test_{}".format(m)] = rank
-            if m in ("mae", "rmse", "mse"):
+            if m in ("mae", "rmse", "mse", "mpr"):
                 rank[indices] = np.arange(len(indices)) + 1
                 best_index[m] = mean_test_measures.argmin()
-            elif m == "fcp" or accuracy._top_n_measure(m) or accuracy._top_n_list_measure(m):
+            elif m in ("fcp", "auc", "mrr") or accuracy._top_n_measure(m) or accuracy._top_n_list_measure(m):
                 rank[indices] = np.arange(len(indices), 0, -1)
                 best_index[m] = mean_test_measures.argmax()
             best_params[m] = self.param_combinations[best_index[m]]

@@ -7,7 +7,8 @@ fit_and_score scores a device-batched algorithm from arrays: the fold's pairs ar
 ``accuracy._of_arrays``, which gives the bits ``accuracy.<m>(algo.test(testset))`` gives without building a
 Prediction per pair.  Any other algorithm or rating measure takes the tuple route.  The top-N measures hr@N,
 arhr@N, precision@N, recall@N and ndcg@N (threshold None) and the list measures user_coverage@N, catalog_coverage@N,
-novelty@N and diversity@N (over the same evaluated users) come from one ``algo._top_n_fold`` pass per fold.
+novelty@N and diversity@N (over the same evaluated users) and the rank measures auc, mrr and mpr over the full ranking
+come from one ``algo._top_n_fold`` pass per fold.
 """
 import time
 
@@ -140,24 +141,27 @@ def _fit_and_score(algo, fold, measures, return_train_measures):
     top_n = {m: v for m, v in top_n.items() if v is not None}
     lists = {m: accuracy._top_n_list_measure(m) for m in measures}
     lists = {m: v for m, v in lists.items() if v is not None}
-    if (top_n or lists) and return_train_measures:
+    ranks = {m: accuracy._rank_measure(m) for m in measures}
+    ranks = {m: v for m, v in ranks.items() if v is not None}
+    if (top_n or lists or ranks) and return_train_measures:
         raise ValueError("return_train_measures cannot be used with top-N measures (%s): trainset items are never "
-                         "recommended, so they would be 0" % ", ".join(list(top_n) + list(lists)))
+                         "recommended, so they would be 0" % ", ".join(list(top_n) + list(lists) + list(ranks)))
     t0 = time.time()
     algo.fit(fold.trainset)
     fit_time = time.time() - t0
-    rating = [m for m in measures if m not in top_n and m not in lists]
+    rating = [m for m in measures if m not in top_n and m not in lists and m not in ranks]
     test_m, train_m, test_time = _score_ratings(algo, fold, rating, return_train_measures) if rating else ({}, {}, 0.0)
-    if top_n or lists:
+    if top_n or lists or ranks:
         t0 = time.time()
         hit_ns = sorted(set(n for _, n in top_n.values()))
         list_ns = sorted(set(n for _, n in lists.values()))
         sim = fold.item_cosine() if any(key == "diversity" for key, _ in lists.values()) else None
-        hit_res, list_res = algo._top_n_fold(fold, hit_ns, list_ns, sim)
+        hit_res, list_res, rank_res = algo._top_n_fold(fold, hit_ns, list_ns, sim, rank=bool(ranks))
         test_time += time.time() - t0
         by_n, by_list_n = dict(zip(hit_ns, hit_res)), dict(zip(list_ns, list_res))
         test_m.update((m, by_n[n][key]) for m, (key, n) in top_n.items())
         test_m.update((m, by_list_n[n][key]) for m, (key, n) in lists.items())
+        test_m.update((m, rank_res[key]) for m, key in ranks.items())
         test_m = {m: test_m[m] for m in measures}
     return test_m, train_m, fit_time, test_time
 

@@ -218,19 +218,24 @@ class AlgoBase(object):
         n_u = len(users)
         return items.cpu().numpy()[:n_u], est.cpu().numpy()[:n_u], count.cpu().numpy()[:n_u]
 
-    def _top_n_dev(self, width, users, _block_rows=None, _events=None, on_block=None):
+    def _top_n_dev(self, width, users, _block_rows=None, _events=None, on_block=None, on_scores=None, select=True,
+                   d_csr=None):
         """top_n_inner's device block loop: (items, est, count) as device arrays of max(len(users), 1) rows.
+        ``on_scores(b0, nr, d_rows, scores, impossible)``, if given, is called with each block's scores (row k of the
+        block at scores + k * n_items) and impossible codes (None when there are none) before its selection.
         ``on_block(b0, nr, items, est, count)``, if given, is called after each block's selection, when rows
-        b0 .. b0 + nr of the device arrays are final."""
+        b0 .. b0 + nr of the device arrays are final.  With ``select`` False nothing is selected and (None, None, None)
+        is returned.  ``d_csr`` is the trainset's user CSR (ptr, idx) on the device, uploaded here when None."""
         from .. import _native as nat
         torch = nat.torch_cuda()
         ts = self.trainset
         n_u, n_i = len(users), ts.n_items
-        items = nat.empty_dev((max(n_u, 1), width), np.int32)
-        est = nat.empty_dev((max(n_u, 1), width), np.float64)
-        count = nat.empty_dev((max(n_u, 1),), np.int32)
-        ptr, idx, _ = ts.user_csr()
-        d_up, d_ui = nat.to_dev(ptr, np.int64), nat.to_dev(idx, np.int32)
+        items = est = count = None
+        if select:
+            items = nat.empty_dev((max(n_u, 1), width), np.int32)
+            est = nat.empty_dev((max(n_u, 1), width), np.float64)
+            count = nat.empty_dev((max(n_u, 1),), np.int32)
+        d_up, d_ui = self._user_csr_dev() if d_csr is None else d_csr
         d_users = nat.to_dev(users, np.int32)
         scorer = self._top_n_scorer()
         rows = int(_block_rows) if _block_rows else max(1, _TOP_N_BLOCK_BYTES // (8 * n_i))
@@ -261,15 +266,24 @@ class AlgoBase(object):
                 sc, imp = self._estimate_dev(d_u, d_i)
             if ev:
                 ev[1].record()
-            nat.check(lib.sb2_top_n_select_dev(nr, nat.ptr(d_rows), n_i, nat.ptr(sc), n_i, nat.ptr(imp),
-                                               float(self.default_prediction()), float(ts.offset), float(low),
-                                               float(high), nat.ptr(d_up), nat.ptr(d_ui), width,
-                                               nat.ptr(items[b0:]), nat.ptr(est[b0:]), nat.ptr(count[b0:]), stream))
+            if on_scores is not None:
+                on_scores(b0, nr, d_rows, sc, imp)
+            if select:
+                nat.check(lib.sb2_top_n_select_dev(nr, nat.ptr(d_rows), n_i, nat.ptr(sc), n_i, nat.ptr(imp),
+                                                   float(self.default_prediction()), float(ts.offset), float(low),
+                                                   float(high), nat.ptr(d_up), nat.ptr(d_ui), width,
+                                                   nat.ptr(items[b0:]), nat.ptr(est[b0:]), nat.ptr(count[b0:]),
+                                                   stream))
             if ev:
                 ev[2].record()
-            if on_block is not None:
+            if select and on_block is not None:
                 on_block(b0, nr, items, est, count)
         return items, est, count
+
+    def _user_csr_dev(self):
+        from .. import _native as nat
+        ptr, idx, _ = self.trainset.user_csr()
+        return nat.to_dev(ptr, np.int64), nat.to_dev(idx, np.int32)
 
     # -- top-N measures against held-out ratings -------------------------------------------------------
     def top_n_measures(self, testset, n=10, threshold=None):
@@ -281,17 +295,30 @@ class AlgoBase(object):
         from ..model_selection.validation import Fold
         return self._top_n_measures(Fold(self.trainset, testset), [n], threshold)[0]
 
+    # -- where held-out items land in the full ranking ---------------------------------------------------
+    def rank_measures(self, testset, threshold=None, _block_rows=None):
+        """AUC, MRR and mean percentile rank of the held-out rows ``(raw uid, raw iid, r_ui)`` of ``testset`` over each
+        user's full ranking of the items they did not rate: bit for bit ``accuracy.rank_measures(self.get_top_n(
+        self.trainset.n_items), testset, self.trainset, threshold, verbose=False)``, without building get_top_n's dict.
+        A device-batched algorithm scores the evaluated users the trainset knows one block at a time and counts where
+        their relevant items rank in each block's scores on the device (sb2_top_n_ranks_dev); nothing is selected.
+        Any other algorithm goes through the definition over get_top_n for those users.  ``_block_rows`` overrides the
+        number of users scored per device block (the result does not depend on it)."""
+        from ..model_selection.validation import Fold
+        return self._top_n_fold(Fold(self.trainset, testset), [], [], None, threshold, _block_rows, rank=True)[2]
+
     def _top_n_measures(self, fold, ns, threshold, _block_rows=None):
         """top_n_measures for each cutoff of ``ns`` on the testset of ``fold`` (a validation.Fold of this trainset): the
         lists are ranked once at the largest cutoff, whose first N entries are the top-N lists (the ranking is a total
         order), and the hits are counted once per cutoff."""
         return self._top_n_fold(fold, ns, [], None, threshold, _block_rows)[0]
 
-    def _top_n_fold(self, fold, hit_ns, list_ns, sim, threshold=None, _block_rows=None):
-        """(top_n_measures at each cutoff of ``hit_ns``, top_n_list_measures at each cutoff of ``list_ns``) on the
-        testset of ``fold``, from one selection pass at the largest cutoff.  The list measures are taken over the
-        evaluated users U* of ``threshold`` (users unknown to the trainset have no list) with no est threshold;
-        ``sim`` (a CUDA float64 item-item matrix, or None) gives diversity."""
+    def _top_n_fold(self, fold, hit_ns, list_ns, sim, threshold=None, _block_rows=None, rank=False):
+        """(top_n_measures at each cutoff of ``hit_ns``, top_n_list_measures at each cutoff of ``list_ns``,
+        rank_measures when ``rank`` else None) on the testset of ``fold``, from one scoring pass, with a selection at
+        the largest cutoff when there is one.  The list measures are taken over the evaluated users U* of
+        ``threshold`` (users unknown to the trainset have no list) with no est threshold; ``sim`` (a CUDA float64
+        item-item matrix, or None) gives diversity."""
         from .. import accuracy
         hit_ns = [_check_top_n(n) for n in hit_ns]
         list_ns = [_check_top_n(n) for n in list_ns]
@@ -299,7 +326,7 @@ class AlgoBase(object):
         pairs = fold.test_pairs()
         iu, n_rel, rel_ptr, rel_idx = pairs.relevant(threshold, ts.n_items)
         known = iu >= 0
-        top = max(hit_ns + list_ns)
+        top = max(hit_ns + list_ns + ([ts.n_items] if rank and not self._batched() else []), default=0)
         if not self._batched():
             lists = self.get_top_n(top, uids=[ts.to_raw_uid(u) for u in iu[known].tolist()])
             hits = [accuracy.top_n_measures({u: l_u[:n] for u, l_u in lists.items()}, fold.testset, n, threshold,
@@ -308,16 +335,17 @@ class AlgoBase(object):
                                       if threshold is None or r >= threshold))
             sim_h = None if sim is None else sim.cpu().numpy()
             return hits, [accuracy.top_n_list_measures(lists, ts, n, star, None, sim_h, verbose=False)
-                          for n in list_ns]
+                          for n in list_ns], \
+                accuracy.rank_measures(lists, fold.testset, ts, threshold, verbose=False) if rank else None
         from .. import _native as nat
         width = min(top, ts.n_items)
         n_k = int(known.sum())
         lib, stream = nat.lib(), nat.stream()
         hooks, outs = [], []
         if hit_ns:
+            d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
             inv, disc, idcg = accuracy._rank_tables(min(max(hit_ns), max(width, int(n_rel.max()))))
             d_inv, d_disc = nat.to_dev(inv, np.float64), nat.to_dev(disc, np.float64)
-            d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
             outs = [tuple(nat.empty_dev((max(n_k, 1),), t) for t in (np.int32, np.float64, np.float64))
                     for _ in hit_ns]
 
@@ -332,18 +360,55 @@ class AlgoBase(object):
             count_lists, finish_lists = self._list_counter(list_ns, width, n_k, None, sim)
             hooks.append(count_lists)
 
+        d_csr = self._user_csr_dev() if n_k else None
+        count_ranks, finish_ranks = self._rank_counter(n_k, rel_ptr, rel_idx, d_csr) if rank else (None, None)
+
         def on_block(*blk):
             for hook in hooks:
                 hook(*blk)
 
-        count = self._top_n_dev(width, iu[known], _block_rows, on_block=on_block)[2] if n_k else None
+        count = None
+        if n_k:
+            count = self._top_n_dev(width, iu[known], _block_rows, on_block=on_block, on_scores=count_ranks,
+                                    select=bool(hit_ns or list_ns), d_csr=d_csr)[2]
         res = []
         for n, out in zip(hit_ns, outs):
             hits, rr, dcg = np.zeros(len(iu), dtype=np.int64), np.zeros(len(iu)), np.zeros(len(iu))
             for host, dev in zip((hits, rr, dcg), out):
                 host[known] = dev.cpu().numpy()[:n_k]
             res.append(accuracy._top_n_of_counts(hits, rr, dcg, n_rel, n, idcg, False))
-        return res, (finish_lists(known, count) if list_ns else [])
+        rank_res = None
+        if rank:
+            c, k, s = (np.zeros(len(iu), dtype=np.int64) for _ in range(3))
+            f = np.full(len(iu), -1, dtype=np.int64)
+            if n_k:
+                for host, dev in zip((c, k, s, f), finish_ranks()):
+                    host[known] = dev
+            rank_res = accuracy._rank_of_counts(c, k, s, f, n_rel, False)
+        return res, (finish_lists(known, count) if list_ns else []), rank_res
+
+    def _rank_counter(self, n_rows, rel_ptr, rel_idx, d_csr):
+        """(on_scores, finish) counting where the relevant items rank over one _top_n_dev pass of n_rows users:
+        on_scores is the pass's score hook (sb2_top_n_ranks_dev on each block, against the relevant CSR rel_ptr /
+        rel_idx of those users, with d_csr the trainset's user CSR on the device); finish() returns the (c, k, s, f)
+        counts of the n_rows users as host int64 arrays."""
+        from .. import _native as nat
+        ts = self.trainset
+        low, high = ts.rating_scale
+        d_ptr, d_idx = nat.to_dev(rel_ptr, np.int64), nat.to_dev(rel_idx, np.int32)
+        outs = [nat.empty_dev((max(n_rows, 1),), t) for t in (np.int32, np.int32, np.int64, np.int32)]
+        lib, stream = nat.lib(), nat.stream()
+
+        def count_ranks(b0, nr, d_rows, sc, imp):
+            nat.check(lib.sb2_top_n_ranks_dev(nr, nat.ptr(d_rows), ts.n_items, nat.ptr(sc), ts.n_items, nat.ptr(imp),
+                                              float(self.default_prediction()), float(ts.offset), float(low),
+                                              float(high), nat.ptr(d_csr[0]), nat.ptr(d_csr[1]), nat.ptr(d_ptr[b0:]),
+                                              nat.ptr(d_idx), len(rel_idx), *(nat.ptr(o[b0:]) for o in outs), stream))
+
+        def finish():
+            return [o.cpu().numpy()[:n_rows].astype(np.int64) for o in outs]
+
+        return count_ranks, finish
 
     # -- coverage, novelty and diversity of the top-N lists --------------------------------------------
     def top_n_list_measures(self, n=10, uids=None, threshold=None, sim=None, _block_rows=None):
